@@ -10,6 +10,8 @@ rank owns its own 256 maps (seed 1000 + global index), no data-path collective.
   roofline : the HBM-bound stencil kernel, algorithmic bytes N + 17n per map over its measured time
   cpu_baseline : the unmodified reference (oracle/_ref, stock glibc) on a bounded sample of the same maps
 `--impl reference` times that CPU reference alone (rank 0 only), one map per host thread.
+`--dump-outputs DIR` writes rank 0's segment tables of the last timed step as .npy files (see dump_outputs) so that two
+builds can be compared output for output: the inputs depend on the arguments only.
 """
 import argparse
 import json
@@ -103,6 +105,41 @@ def cpu_reference_throughput(size, n_maps, threads, first_gidx=0):
     return dict(seconds=dt, mpix_per_s=n_maps * size * size / dt / 1e6, segments=int(sum(counts)), n_maps=n_maps)
 
 
+DUMP_LIMIT = 64 * 10**6
+
+
+def split_nonfinite(a):
+    """a 2-D array -> (a with its non-finite entries set to 0, one (row, column, code) record per such entry; code 1 = +inf,
+    -1 = -inf, 2 = NaN), both finite float64: vertical segments carry k = -inf, b = NaN (structLinesInfo)."""
+    bad = ~np.isfinite(a)
+    r, c = np.nonzero(bad)
+    code = np.where(np.isnan(a[r, c]), 2.0, np.sign(a[r, c]))
+    return np.where(bad, 0.0, a), np.stack([r, c, code], axis=1).astype(np.float64)
+
+
+def dump_outputs(out_dir, got, lines_to_array):
+    """Writes what a caller of the timed path receives, as finite float64 .npy files under out_dir: counts (segments per map),
+    maps (the indices of the maps whose tables follow), lines (structLinesInfo in oracle column order) and rects (rectangle and
+    log-NFA records), the tables of those maps concatenated in map order, with their non-finite entries in lines_nonfinite /
+    rects_nonfinite (see split_nonfinite).  Every map when the files fit in DUMP_LIMIT bytes, else a fixed seeded sample of
+    the maps."""
+    counts = np.asarray(got["counts"], np.int64)
+    tables = [(lines_to_array(got["lines"][i]), got["rects"][i]) for i in range(counts.size)]
+    map_bytes = np.array([8 * (ln.size + rc.size) + 24 * int((~np.isfinite(ln)).sum() + (~np.isfinite(rc)).sum()) for ln, rc in tables])
+    budget = DUMP_LIMIT - 2 * 8 * counts.size - 6 * 128     # counts, maps and the six .npy headers
+    order = np.arange(counts.size)
+    if map_bytes.sum() > budget:
+        order = np.random.default_rng(0).permutation(counts.size)
+    maps = np.sort(order[np.cumsum(map_bytes[order]) <= budget])
+    lines, lines_nf = split_nonfinite(np.concatenate([np.zeros((0, 10))] + [tables[i][0] for i in maps]))
+    rects, rects_nf = split_nonfinite(np.concatenate([np.zeros((0, 13))] + [tables[i][1] for i in maps]))
+    out = {"counts": counts.astype(np.float64), "maps": maps.astype(np.float64), "lines": lines, "lines_nonfinite": lines_nf,
+           "rects": rects, "rects_nonfinite": rects_nf}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def stencil_traffic(n, size):
     """dram__bytes_read.sum + dram__bytes_write.sum of ONE stencil launch (lsdb_stencil2_kernel), from this round's ncu
     capture (profiles/r2_stencil_traffic.json, written by tools/stencil_traffic.py from the .ncu-rep), scaled to this
@@ -119,7 +156,7 @@ def run_reference(args, rank, world):
         return
     cores = os.cpu_count() or 1
     threads = min(cores, args.ref_threads or cores)
-    k_run, w_run = min(args.steps, 3), min(args.warmup, 1)   # every step is >= one 4096^2 map per thread (~30 s)
+    k_run, w_run = args.steps, args.warmup   # a step is one map per host thread: ~30 s at 4096^2
     sample = f"{threads} maps of {args.size}x{args.size} per step, one per host thread (of the {args.maps_per_gpu}-map batch)"
     for s in range(w_run):
         r = cpu_reference_throughput(args.size, threads, threads)
@@ -138,7 +175,7 @@ def run_reference(args, rank, world):
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": k_run, "warmup": w_run,
         "ms_per_step": t_all / k_run * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
         "data": "synthetic", "config": {"workload": f"synthetic {args.size}x{args.size} occupancy grids (BASELINE configs[2])",
-                                        "maps_per_step": threads, "note": "steps/warmup capped at 3/1: one step is ~30 s of CPU per thread"},
+                                        "maps_per_step": threads},
         "cpu_baseline": {"value": v, "unit": UNIT, "cores": threads, "kind": "reference", "sample": sample},
         "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0}))
@@ -232,7 +269,8 @@ def run_giant(args, rank, world, local):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=int, default=8, help="timed steps of the resident loop (the headline value) and of --impl reference; "
+                    "the end-to-end leg runs a multiple of the batches in flight, at least four per batch")
     ap.add_argument("--warmup", type=int, default=4)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--maps-per-gpu", type=int, default=256)
@@ -251,7 +289,10 @@ def main():
                     help="batch: BASELINE configs[2] (the headline); giant: ONE --giant-size^2 map tiled over the ranks (configs[4])")
     ap.add_argument("--giant-size", type=int, default=16384)
     ap.add_argument("--parity-maps", type=int, default=8, help="maps of the timed batch whose segment tables are checked against the CPU oracle (rank 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's segment tables of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "batch"):
+        ap.error("--dump-outputs needs --impl b200 --workload batch")
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -345,9 +386,12 @@ def main():
     # ---------------- the bench checks what it times: segment tables of the first maps of the timed batch against the CPU
     # oracle (bit for bit), before anything else touches the batches.  A mismatch fails the bench.
     parity_k = 0
+    if rank == 0 and (args.parity_maps > 0 or args.dump_outputs):
+        got0 = batches[(args.steps - 1) % NB].download(want_rects=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, got0, lsdb.lines_to_array)
     if rank == 0 and args.parity_maps > 0:
         import oraclebind
-        got0 = batches[(args.steps - 1) % NB].download(want_rects=True)
         parity_k = min(args.parity_maps, n)
         for i in range(parity_k):
             o = oraclebind.lsd(hnp[i], want_maps=False, want_line_im=False, max_lines=4096)

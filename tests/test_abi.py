@@ -65,7 +65,7 @@ def test_dropin_library_keeps_the_reference_entry_points():
     import subprocess
     so = os.path.join(ROOT, "oracle", "_ref", "libref_dropin.so")
     if not os.path.exists(so):
-        pytest.skip("libref_dropin.so not built (needs /root/reference)")
+        pytest.skip("libref_dropin.so not built (needs LSD_REFERENCE_DIR)")
     L = C.CDLL(so)
     L.ref_variant.restype = C.c_char_p
     assert L.ref_variant() == b"dropin"

@@ -8,7 +8,8 @@ import pytest
 import datautil
 import oraclebind
 
-REF_DATA = "/root/reference/data"
+REF_ROOT = os.environ.get("LSD_REFERENCE_DIR")          # a checkout of the original LineSegmentDetector-SLAM
+REF_DATA = os.path.join(REF_ROOT, "data") if REF_ROOT else None
 
 
 def test_map_cache_file_round_trip(lsdb, tmp_path):
@@ -36,7 +37,7 @@ def test_map_value_and_param_files(lsdb, tmp_path):
     assert v.tolist() == [[255, 0, 1, 0, 255], [0, 1, 1, 0, 255], [255, 255, 0, 0, 1]]   # -1 -> 255 (`%d` into a uint8 slot)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference data not present")
+@pytest.mark.skipif(not (REF_DATA and os.path.isdir(REF_DATA)), reason="reference data not present (set LSD_REFERENCE_DIR)")
 def test_bundled_files_parse_like_the_reference(lsdb):
     gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "bundled_maps.npz"))
     p = lsdb.read_map_param(os.path.join(REF_DATA, "mapParam.txt"))

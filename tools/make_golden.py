@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Generates tests/golden/*.npz from the UNMODIFIED reference compiled into oracle/_ref (stock glibc variant).
 
-Run in the authoring container (needs /root/reference and oracle/_ref):  python tools/make_golden.py
+Needs oracle/_ref, built from the checkout LSD_REFERENCE_DIR names:  LSD_REFERENCE_DIR=... python tools/make_golden.py
   bundled_maps.npz : the six bundled occupancy grids (inputs, u8) and the reference's outputs for each:
                      segment table, usedMap, regIdx, sorted seed list, lineIm (bit-packed)
   fa_frames.npz    : the first frames of data/Lidar.txt pushed through the reference's own RDP front-end
@@ -17,7 +17,8 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import datautil  # noqa: E402
 import refbind  # noqa: E402
 
-D = "/root/reference/data/"
+REF_ROOT = os.environ["LSD_REFERENCE_DIR"]
+D = os.path.join(REF_ROOT, "data") + "/"
 MAPS = [("mapValue", "mapParam"), ("mapValue_aisle1", "mapParam_aisle1"), ("mapValue_aisle2", "mapParam_aisle2"),
         ("mapValue_aisle3", "mapParam_aisle3"), ("mapValue_map1", "mapParam_map1"), ("mapValue_map2", "mapParam_map1")]
 out = {}
@@ -65,7 +66,7 @@ np.savez_compressed(os.path.join(ROOT, "tests", "golden", "fa_frames.npz"), **fa
 # whether the stock-glibc build gives the identical result for that frame.
 import glob  # noqa: E402
 picks = [(D + "Lidar.txt", list(range(0, 96, 8)))]
-for fn in sorted(glob.glob("/root/reference/data_2019051*/data_f*key/data*/Lidar.txt")):
+for fn in sorted(glob.glob(os.path.join(REF_ROOT, "data_2019051*/data_f*key/data*/Lidar.txt"))):
     picks.append((fn, [5, 31, 35, 119]))
 ls = {}
 k = 0

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """tests/golden/extra_maps.npz: the two further distinct occupancy grids of the reference mount (data_20190513/data_f3key,
 1440x979; data_20190514/data_f4key, 1404x707 — BASELINE configs[1] "all bundled maps") through the UNMODIFIED reference
-(oracle/_ref, stock glibc): segment table, usedMap, regIdx, sorted seed list.  Run in the authoring container."""
+(oracle/_ref, stock glibc): segment table, usedMap, regIdx, sorted seed list.  Needs LSD_REFERENCE_DIR (a checkout of the original)."""
 import glob
 import os
 import sys
@@ -14,7 +14,8 @@ import datautil  # noqa: E402
 import refbind  # noqa: E402
 
 out = {}
-for name, pat in (("f3key", "/root/reference/data_20190513/data_f3key/data*/"), ("f4key", "/root/reference/data_20190514/data_f4key/data*/")):
+REF_ROOT = os.environ["LSD_REFERENCE_DIR"]
+for name, pat in (("f3key", os.path.join(REF_ROOT, "data_20190513/data_f3key/data*/")), ("f4key", os.path.join(REF_ROOT, "data_20190514/data_f4key/data*/"))):
     d = next(x for x in sorted(glob.glob(pat)) if os.path.exists(x + "mapValue.txt") and os.path.exists(x + "mapParam.txt"))
     p = datautil.load_map_param(d + "mapParam.txt")
     m = datautil.load_map_value(d + "mapValue.txt", p["cols"], p["rows"])

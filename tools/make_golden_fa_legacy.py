@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Golden vectors of the catkin snapshot's association (ROS/lsd/src/FeatureAssociation.cpp), made HERE (where /root/reference exists)
+"""Golden vectors of the catkin snapshot's association (ROS/lsd/src/FeatureAssociation.cpp), made where LSD_REFERENCE_DIR names a checkout of the original
 by the UNMODIFIED source behind oracle/ros_fa_harness.cpp (oracle/_ref/libref_rosfa.so, stock libm): tests/golden/fa_legacy.npz.
 Inputs: the bundled map of configs[0] (its LSD lines from tests/golden/bundled_maps.npz, its mapCache with unreached cells at 2.0 as
 the snapshot's three-argument createMapCache leaves them), seeded synthetic scan frames / lidar sweeps from the package's synth.py."""
