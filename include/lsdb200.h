@@ -218,6 +218,37 @@ int lsdb_fa_score_kept(lsdb_ctx* ctx, const lsdb_fa_map* m, int n_frames, const 
 int lsdb_fa_legacy(lsdb_ctx* ctx, const lsdb_fa_map* m, const lsdb_line* scan_lines, int n_scan, double map_resol, double map_ori_x,
                    double map_ori_y, const int* lidar_pos, const double* ranges, const double* angles, int n_rays, double* pose_all,
                    int max_cols, int* n_cols, double* estimate_pose, double* estimate_pose_realworld);
+/* one record per frame of lsdb_fa_legacy_frames */
+typedef struct {
+    int n_cols;                        /* T of the frame = 4 x candidate pairs */
+    int best_col;                      /* t of :117-119, frame-local column; -1 when T == 0 */
+    double best_score;                 /* poseAll(3, t); NaN when T == 0 */
+    double estimate_pose[3];           /* pixels, radians (:120-123); NaN when T == 0 */
+    double estimate_pose_realworld[3]; /* metres (:124-127); NaN when T == 0 */
+} lsdb_fa_legacy_estimate;             /* 64 bytes */
+/* lsdb_fa_legacy for n_frames sweeps against one map in one call (a log replayed, a parameter sweep).  Frames are independent in
+ * the snapshot (no pose of one frame gates the next), so every frame gets exactly what lsdb_fa_legacy returns for it alone, however
+ * the frames are grouped into calls:
+ *   scan_lines : ScanlinesInfo of every frame concatenated, scan_line_off[n_frames+1]; lidar_pos : [n_frames][2]
+ *   ranges / angles : concatenated, ray_off[n_frames+1] (Inf / NaN ranges fall outside the map)
+ * Per frame: the length filter of :61-70 with 0.3 / map_resol in the reference's (scan line, map line) order, the four pairings,
+ * RotateScanIm and the ray re-projection score.  Frame f's records are the columns [col_off[f], col_off[f+1]) of pose_all (15
+ * doubles each, as lsdb_fa_legacy); column 12 is the frame-local scan-line index, so a frame's slice equals its lsdb_fa_legacy output.
+ * est[f].best_col is the column the reference's `t = 0; for i: if (s[i] < s[t]) t = i` ends at, i.e.: 0 if s[0] is NaN, otherwise
+ * the FIRST column whose score == the minimum of the non-NaN scores (-0 ties +0; a frame of +inf scores gives 0).  A frame without
+ * rays scores NaN (0/0) everywhere and gets best_col = 0; a frame without a candidate pair gets best_col = -1 and NaNs.
+ * Sizes: est and col_off (nullable) are always filled first.  pose_all == NULL asks for the estimates only.  pose_all != NULL and a
+ * total T > max_cols: LSDB_ERR_CAPACITY with est and col_off filled and pose_all untouched (the sizing query).  A total T above
+ * 2^31-1 is LSDB_ERR_CAPACITY.  n_frames == 0 is LSDB_OK.  LSDB_ERR_ARG: offsets that do not start at 0 or decrease, null arrays
+ * with non-zero counts, est or lidar_pos NULL (n_frames > 0), max_cols < 0, map_resol <= 0.
+ * One host-to-device copy, two launches (scores, per-frame selection), one synchronise. */
+int lsdb_fa_legacy_frames(lsdb_ctx* ctx, const lsdb_fa_map* m, int n_frames,
+                          const lsdb_line* scan_lines, const int* scan_line_off,
+                          double map_resol, double map_ori_x, double map_ori_y,
+                          const int* lidar_pos,
+                          const double* ranges, const double* angles, const int* ray_off,
+                          lsdb_fa_legacy_estimate* est,
+                          double* pose_all, int max_cols, int* col_off);
 /* The per-frame reduction that follows the scoring in FeatureAssociation (LSD/myFA.cpp:65-171, everything before ukf),
  * done on the device so that only one record per frame comes back instead of every hypothesis:
  *   n_kept  : hypotheses with score < 3 (:261); 0 = "no match, start a new chain" (:70-90)
@@ -233,7 +264,8 @@ typedef struct {
 int lsdb_fa_estimate_frames(lsdb_ctx* ctx, const lsdb_fa_map* m, int n_frames, const lsdb_line* scan_lines,
                             const int* scan_line_off, const double* scan_pts, const int* scan_pt_off,
                             const double* lidar_pose, const double* last_pose, lsdb_fa_estimate* out);
-/* device time of the last lsdb_fa_score kernel (ms) */
+/* device time of the kernels of the last association call on this context (ms): lsdb_fa_score, lsdb_fa_score_kept,
+ * lsdb_fa_estimate_frames, lsdb_scan_estimate_frames (its association part), lsdb_fa_legacy, lsdb_fa_legacy_frames */
 float lsdb_fa_last_ms(const lsdb_ctx* ctx);
 
 /* ---- scan front-end: lidar frames -> scan lines + raster samples (the inputs of the association) ---- */

@@ -29,6 +29,8 @@ SCAN_INFO_DTYPE = np.dtype([("n_lines", "i4"), ("n_pts", "i4"), ("im_cols", "i4"
 RDP_DEFAULTS = dict(least_point=3, thre_line=0.08, least_dist_m=0.5)  # LSD/baseFunc.h:70-72
 HYP_DTYPE = np.dtype([("frame", "i4"), ("i_scan", "i4"), ("i_map", "i4"), ("i_pair", "i4"), ("x", "f8"), ("y", "f8"),
                       ("ang", "f8"), ("score", "f8")])
+LEGACY_EST_DTYPE = np.dtype([("n_cols", "i4"), ("best_col", "i4"), ("best_score", "f8"), ("estimate_pose", "f8", (3,)),
+                             ("estimate_pose_realworld", "f8", (3,))])   # lsdb_fa_legacy_estimate
 
 
 class LsdbError(RuntimeError):
@@ -96,6 +98,7 @@ def lib():
         L.lsdb_fa_score.argtypes = [vp, vp, ci, vp, vp, vp, vp, vp, vp, vp, ci, vp]
         L.lsdb_fa_score_kept.argtypes = [vp, vp, ci, vp, vp, vp, vp, vp, vp, cd, vp, ci, vp, vp]
         L.lsdb_fa_legacy.argtypes = [vp, vp, vp, ci, cd, cd, cd, vp, vp, vp, ci, vp, ci, vp, vp, vp]
+        L.lsdb_fa_legacy_frames.argtypes = [vp, vp, ci, vp, vp, cd, cd, cd, vp, vp, vp, vp, vp, vp, ci, vp]
         L.lsdb_fa_estimate_frames.argtypes = [vp, vp, ci, vp, vp, vp, vp, vp, vp, vp]
         L.lsdb_fa_last_ms.argtypes = [vp]; L.lsdb_fa_last_ms.restype = C.c_float
         L.lsdb_feature_scan_frames.argtypes = [vp, cd, cd, cd, C.POINTER(_RdpParams), ci, vp, vp, vp, vp, vp, ci, vp, vp, ci, vp, vp,
@@ -480,6 +483,39 @@ class FaMap:
         if n.value == 0:
             return out[:0].copy(), None, None
         return out[:n.value].copy(), est, real
+
+    @staticmethod
+    def pack_legacy(frames):
+        """frames (dicts of scan_lines, lidar_pos, ranges, angles) as the flat arrays lsdb_fa_legacy_frames takes:
+        (n_frames, scan lines, scan_line_off, lidar_pos (n,2) int32, ranges, angles, ray_off)."""
+        nf = len(frames)
+        sl = [f["scan_lines"] if getattr(f["scan_lines"], "dtype", None) == LINE_DTYPE else array_to_lines(f["scan_lines"]) for f in frames]
+        loff = np.zeros(nf + 1, np.int32); roff = np.zeros(nf + 1, np.int32)
+        loff[1:] = np.cumsum([len(x) for x in sl]); roff[1:] = np.cumsum([len(f["ranges"]) for f in frames])
+        if any(len(f["ranges"]) != len(f["angles"]) for f in frames):
+            raise ValueError("ranges and angles differ in length")
+        lines = np.ascontiguousarray(np.concatenate(sl)) if nf else np.zeros(0, LINE_DTYPE)
+        lp = np.ascontiguousarray(np.array([np.asarray(f["lidar_pos"]).reshape(2) for f in frames], np.int32).reshape(nf, 2))
+        r = np.ascontiguousarray(np.concatenate([np.asarray(f["ranges"], np.float64).ravel() for f in frames])) if nf else np.zeros(0)
+        a = np.ascontiguousarray(np.concatenate([np.asarray(f["angles"], np.float64).ravel() for f in frames])) if nf else np.zeros(0)
+        return nf, lines, loff, lp, r, a, roff
+
+    def legacy_frames(self, frames, map_resol, map_ori, want_pose_all=False, max_cols=None):
+        """lsdb_fa_legacy_frames — lsdb_fa_legacy for many frames in one call.  `frames`: a list of dicts (scan_lines, lidar_pos,
+        ranges, angles) or the tuple pack_legacy() returned.  Returns (est LEGACY_EST_DTYPE[n_frames], pose_all (T,15) or None,
+        col_off int32[n_frames+1]); frame f's records are pose_all[col_off[f]:col_off[f+1]].  max_cols bounds pose_all (default:
+        every pair the frames' scan lines could form)."""
+        nf, lines, loff, lp, r, a, roff = frames if isinstance(frames, tuple) else self.pack_legacy(frames)
+        est = np.zeros(nf, LEGACY_EST_DTYPE); coff = np.zeros(nf + 1, np.int32)
+        out = None
+        if want_pose_all:
+            if max_cols is None:
+                max_cols = min(4 * int(loff[-1]) * max(self.n_lines, 1), 2**31 - 1)
+            out = np.empty((max(int(max_cols), 1), 15))   # only the T records written are touched
+        self.ctx.check(lib().lsdb_fa_legacy_frames(self.ctx.h, self.h, nf, _p(lines), _p(loff), float(map_resol), float(map_ori[0]),
+                                                   float(map_ori[1]), _p(lp), _p(r), _p(a), _p(roff), _p(est), _p(out),
+                                                   int(max_cols or 0), _p(coff)), "lsdb_fa_legacy_frames")
+        return est, (out[:coff[-1]] if want_pose_all else None), coff
 
     def pack(self, frames):
         """the frames as the flat arrays the C ABI takes (do this once when the same frames are scored repeatedly)"""

@@ -121,9 +121,12 @@ void lsdb_launch_fa(cudaStream_t s, int nTasks, const LsdbFaTask* tasks, const L
 size_t lsdb_fa_pose_bytes(int nTasks);
 struct LsdbFaEst { int nHyp, nKept; double bx, by, bang, bscore, mx, my, mang, mscore; };  // == lsdb_fa_estimate
 void lsdb_launch_fa_reduce(cudaStream_t s, int nFrames, const LsdbFaHyp* hyp, const int* hypOff, LsdbFaEst* est);
-void lsdb_launch_fa_legacy(cudaStream_t s, int nPairs, const int2* pairs, const LsdbFaLine* scanLines, const LsdbFaLine* mapLines,
-                           int lidarX, int lidarY, const double* mapCache, int cols, int rows, double resol, const double* ranges,
-                           const double* angles, int nRays, double* out);
+struct LsdbFaLegacyEst { int nCols, bestCol; double bestScore, pose[3], real[3]; };  // == lsdb_fa_legacy_estimate
+void lsdb_launch_fa_legacy(cudaStream_t s, int nHyp, const LsdbFaTask* tasks, const LsdbFaLine* scanLines, const int* scanLineOff,
+                           const LsdbFaLine* mapLines, const int* lidarPos, const double* mapCache, int cols, int rows, double resol,
+                           const double* ranges, const double* angles, const int* rayOff, double* out);
+void lsdb_launch_fa_legacy_reduce(cudaStream_t s, int nFrames, const int* colOff, const double* rec, double resol, double oriX, double oriY,
+                                  LsdbFaLegacyEst* est);
 size_t lsdb_fa_pairs_scratch_ints(int nL);
 size_t lsdb_fa_keep_scratch_ints(int nHyp);
 void lsdb_launch_fa_keep(cudaStream_t s, int nHyp, const LsdbFaHyp* hyp, double below, int* scratch, LsdbFaHyp* out, int cap);
