@@ -33,6 +33,11 @@ extern "C" {
 #define LSDB_ERR_TIMEOUT 4    /* device-side watchdog fired (ordered-commit pipeline stalled) */
 #define LSDB_ERR_NO_DEVICE 5  /* no usable CUDA device */
 
+/* Largest |angle| (radians) a caller may pass as a beam / ray angle (lsdb_feature_scan_frames, lsdb_fa_legacy,
+ * lsdb_fa_legacy_frames): 2^19.  The device's sin / cos are exact-reduction, correctly rounded functions up to 2^20 and NaN
+ * beyond; the association adds up to 3 pi to a ray's angle, so 2^19 leaves headroom.  Larger angles are LSDB_ERR_ARG. */
+#define LSDB_MAX_ANGLE 524288.0
+
 typedef struct lsdb_ctx lsdb_ctx;
 typedef struct lsdb_batch lsdb_batch;
 typedef struct lsdb_fa_map lsdb_fa_map;
@@ -209,7 +214,8 @@ int lsdb_fa_score_kept(lsdb_ctx* ctx, const lsdb_fa_map* m, int n_frames, const 
  * 13-argument call of LSD/main_on_linux.cpp:132.  `m` holds MapCache (the three-argument createMapCache: cells beyond z_occ_max_dis
  * read exactly 2.0, which the score counts apart, :239) and MaplinesInfo; its size is the size of MaplineIm.
  *   scan_lines : ScanlinesInfo (x1 y1 x2 y2 len are used)      lidar_pos : LidarPos[2], scan-image pixels
- *   ranges/angles : ScanRanges / ScanAngles, n_rays of each (Inf / NaN ranges fall outside the map, as in the reference)
+ *   ranges/angles : ScanRanges / ScanAngles, n_rays of each (Inf / NaN ranges fall outside the map, as in the reference);
+ *                   an angle with |angle| > LSDB_MAX_ANGLE (2^19, Inf included) is LSDB_ERR_ARG, found before anything launches
  * Output: pose_all = up to max_cols records of 15 doubles, the COLUMNS of the reference's 15 x T poseAll in its order (pose x y
  * angle[deg], score, map end points, scan end points, scan-line index, map-line index, pairing 0..3); *n_cols = T;
  * estimate_pose[3] (pixels, radians) / estimate_pose_realworld[3] (metres) = the first strict minimum of the score row (:117-127),
@@ -230,7 +236,7 @@ typedef struct {
  * the snapshot (no pose of one frame gates the next), so every frame gets exactly what lsdb_fa_legacy returns for it alone, however
  * the frames are grouped into calls:
  *   scan_lines : ScanlinesInfo of every frame concatenated, scan_line_off[n_frames+1]; lidar_pos : [n_frames][2]
- *   ranges / angles : concatenated, ray_off[n_frames+1] (Inf / NaN ranges fall outside the map)
+ *   ranges / angles : concatenated, ray_off[n_frames+1] (Inf / NaN ranges fall outside the map; |angle| <= LSDB_MAX_ANGLE)
  * Per frame: the length filter of :61-70 with 0.3 / map_resol in the reference's (scan line, map line) order, the four pairings,
  * RotateScanIm and the ray re-projection score.  Frame f's records are the columns [col_off[f], col_off[f+1]) of pose_all (15
  * doubles each, as lsdb_fa_legacy); column 12 is the frame-local scan-line index, so a frame's slice equals its lsdb_fa_legacy output.
@@ -240,7 +246,7 @@ typedef struct {
  * Sizes: est and col_off (nullable) are always filled first.  pose_all == NULL asks for the estimates only.  pose_all != NULL and a
  * total T > max_cols: LSDB_ERR_CAPACITY with est and col_off filled and pose_all untouched (the sizing query).  A total T above
  * 2^31-1 is LSDB_ERR_CAPACITY.  n_frames == 0 is LSDB_OK.  LSDB_ERR_ARG: offsets that do not start at 0 or decrease, null arrays
- * with non-zero counts, est or lidar_pos NULL (n_frames > 0), max_cols < 0, map_resol <= 0.
+ * with non-zero counts, est or lidar_pos NULL (n_frames > 0), max_cols < 0, map_resol <= 0, an angle beyond LSDB_MAX_ANGLE.
  * One host-to-device copy, two launches (scores, per-frame selection), one synchronise. */
 int lsdb_fa_legacy_frames(lsdb_ctx* ctx, const lsdb_fa_map* m, int n_frames,
                           const lsdb_line* scan_lines, const int* scan_line_off,
@@ -283,7 +289,8 @@ typedef struct {
     double lidar_x, lidar_y;   /* FS.lidarPos */
 } lsdb_scan_info;
 /* Inputs: ranges / angles concatenated per frame (finite values only — the callers drop Inf beams,
- * LSD/main_on_windows.cpp:110-123), beam_off[n_frames+1]; every frame needs at least one beam.
+ * LSD/main_on_windows.cpp:110-123 — and |angle| <= LSDB_MAX_ANGLE, 2^19; anything else is LSDB_ERR_ARG before any launch),
+ * beam_off[n_frames+1]; every frame needs at least one beam.
  * Outputs (host buffers):
  *   info[n_frames]; line_off / pt_off [n_frames+1] (prefix sums of n_lines / n_pts); im_off[n_frames+1] (bytes)
  *   lines  : records in the reference's order, frame f at lines[line_off[f]]  (lsdb_line; `orient` as FeatureScan sets it)

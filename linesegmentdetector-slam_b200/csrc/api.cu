@@ -958,6 +958,9 @@ static int fa_legacy_run(lsdb_ctx* ctx, const char* what, const lsdb_fa_map* m, 
                          const int* rayOff, lsdb_fa_legacy_estimate* est, double* poseAll, int maxCols, int* colOff, bool truncate) {
     static_assert(sizeof(lsdb_fa_legacy_estimate) == sizeof(LsdbFaLegacyEst) && sizeof(LsdbFaLegacyEst) == 64, "layout");
     const std::string name(what);
+    for (int i = 0; i < rayOff[nFrames]; i++)   // the kernel adds |theta| <= 3 pi; lsd_math.h's sin / cos are defined up to 2^20
+        if (fabs(angles[i]) > LSDB_MAX_ANGLE)
+            return fail(ctx, LSDB_ERR_ARG, (name + ": the angle of ray %s%lld exceeds 2^19 in magnitude").c_str(), "", i);
     std::vector<LsdbFaTask> tasks;
     std::vector<int> off((size_t)nFrames + 1, 0);
     const double lenDiff = 0.3 / mapResol;   // :61-62
@@ -1095,9 +1098,12 @@ static int fs_run(lsdb_ctx* ctx, double resol, double oriX, double oriY, const l
         maxBeams = std::max(maxBeams, n);
     }
     const int nB = beamOff[nFrames];
-    for (int i = 0; i < nB; i++)
+    for (int i = 0; i < nB; i++) {
         if (!std::isfinite(ranges[i]) || !std::isfinite(angles[i]))
             return fail(ctx, LSDB_ERR_ARG, "lsdb_feature_scan_frames: beam %s%lld is not finite (drop Inf ranges first)", "", i);
+        if (fabs(angles[i]) > LSDB_MAX_ANGLE)   // lsd_math.h's sin / cos are defined up to 2^20
+            return fail(ctx, LSDB_ERR_ARG, "lsdb_feature_scan_frames: the angle of beam %s%lld exceeds 2^19 in magnitude", "", i);
+    }
     const size_t smem = lsdb_fscan_smem(maxBeams);
     if (smem > 200 * 1024) return fail(ctx, LSDB_ERR_CAPACITY, "lsdb_feature_scan_frames: %s%lld beams in one frame exceed the shared-memory layout", "", maxBeams);
     CK(ctx, cudaSetDevice(ctx->device));

@@ -12,8 +12,11 @@
  *     < 2^-63 from a 1/64-spaced table + short polynomial and returns when hi+lo±err round to
  *     the same double; phase 2 (≈0.2 % of calls) re-evaluates in double-double (~2^-100).
  *   - exp, log, log10, sinh, pow: double-double throughout.
- * Domain notes: sin/cos are accurate for |x| <= 2^20; atan2 assumes operands that are zero or
- * within [2^-900, 2^900] (no subnormal/near-overflow scaling tricks).  NaN/Inf follow C99.
+ * Domain notes: sin/cos are accurate for |x| <= 2^20 (the range of lsdm_rem_pio2) and return NaN for any larger |x|, so no
+ * argument indexes outside the tables; callers that take angles from outside keep them within 2^19.  atan2 / atan take
+ * every double: a pair of finite non-zero operands outside [2^-900, 2^900] is first scaled by one exact power of two (which
+ * leaves the ratio and so the result alone), so the error-free products never overflow or underflow, and a result below
+ * 2^-960 is rounded once onto the subnormal grid (lsdm_atan_tiny) instead of going through phase 1.  NaN/Inf follow C99.
  */
 #ifndef LSD_MATH_H
 #define LSD_MATH_H
@@ -93,9 +96,14 @@ LSDM_FN lsdm_dd lsdm_fast_two_sum(double a, double b) { /* requires |a| >= |b| o
     return r;
 }
 LSDM_FN void lsdm_split(double a, double* hi, double* lo) {
-    double c = 134217729.0 * a; /* 2^27 + 1 */
-    double ab = c - a;
-    *hi = c - ab;
+    /* above 2^996, 134217729 * a overflows: split a * 2^-28 instead and scale back, the same halves since both scalings are exact
+     * (only a 26-bit head that rounds up to 2^1024 still overflows).  The device's error-free product has no such limit, so
+     * without this the host's pow of a result in [2^997, 2^1000) left the integer-power path the device takes. */
+    const double s = fabs(a) > 0x1p996 ? 0x1p-28 : 1.0;
+    double as = a * s;
+    double c = 134217729.0 * as; /* 2^27 + 1 */
+    double ab = c - as;
+    *hi = (c - ab) / s;
     *lo = a - *hi;
 }
 LSDM_FN lsdm_dd lsdm_two_prod(double a, double b) {
@@ -161,6 +169,14 @@ LSDM_FN int lsdm_round_ok(double h, double l, double* out) {
     return u == v;
 }
 
+/* nearest integer to 64 a for 0 <= a <= 1, halves up: the index of a's 1/64-spaced table entry.  Not (int)(a * 64 + 0.5): for
+ * a = 2^-7 - 2^-60 that sum rounds up to 1, and a - 1/64 is then not exact (phase 1 was 2^-53 off and misrounded sin and atan). */
+LSDM_FN int lsdm_tab64(double a) {
+    const double s = a * 64.0; /* exact, and so is s - j */
+    const int j = (int)s;
+    return j + (s - (double)j >= 0.5);
+}
+
 /* =====================================================================  sin / cos  */
 
 /* x - k*pi/2 as a double-double, k = nearest integer; returns k (valid for |x| <= 2^20). */
@@ -204,7 +220,7 @@ LSDM_FN lsdm_dd lsdm_sincos_fast(double rh, double rl, int which) {
     int neg = rh < 0.0;
     double a = neg ? -rh : rh;
     double al = neg ? -rl : rl;
-    int j = (int)(a * 64.0 + 0.5);
+    int j = lsdm_tab64(a);
     double d = a - (double)j * 0.015625; /* exact */
     lsdm_dd dd = lsdm_two_sum(d, al);
     double dh = dd.h, dl = dd.l;
@@ -242,9 +258,11 @@ LSDM_SLOW double lsdm_sincos_slow(lsdm_dd r, int n) {
     }
 }
 
+#define LSDM_SINCOS_MAX 0x1p20 /* |x| beyond which lsdm_rem_pio2 is not exact: sin / cos return NaN */
+
 /* n = quadrant offset: 0 for sin, 1 for cos */
 LSDM_FN double lsdm_sincos_eval(double x, int want_cos) {
-    if (lsdm_isnan(x) || lsdm_isinf(x)) return x - x; /* NaN */
+    if (!(fabs(x) <= LSDM_SINCOS_MAX)) return (x - x) / 0.0; /* NaN, also for NaN / Inf */
     if (fabs(x) < 0x1p-27) return want_cos ? 1.0 : x;
     lsdm_dd r;
     int n = (lsdm_rem_pio2(x, &r) + want_cos) & 3;
@@ -259,10 +277,10 @@ LSDM_FN double lsdm_cos(double x) { return lsdm_sincos_eval(x, 1); }
 
 /* Phase 1 of lsdm_sin AND lsdm_cos of the same argument, sharing the reduction.  Returns 1 with *s == lsdm_sin(x) and
  * *c == lsdm_cos(x) (the same operations in the same order as lsdm_sincos_eval, hence the same bits) when both rounding
- * tests pass; returns 0 — outputs unspecified — when either needs phase 2 or x is not finite: the caller then calls
- * lsdm_sin / lsdm_cos.  Lets a kernel keep its warps on the short path and collect the rare phase-2 arguments elsewhere. */
+ * tests pass; returns 0 — outputs unspecified — when either needs phase 2 or |x| is not <= LSDM_SINCOS_MAX: the caller then
+ * calls lsdm_sin / lsdm_cos.  Lets a kernel keep its warps on the short path and collect the rare phase-2 arguments elsewhere. */
 LSDM_FN int lsdm_sincos_try(double x, double* s, double* c) {
-    if (lsdm_isnan(x) || lsdm_isinf(x)) return 0;
+    if (!(fabs(x) <= LSDM_SINCOS_MAX)) return 0;
     if (fabs(x) < 0x1p-27) { *s = x; *c = 1.0; return 1; }
     lsdm_dd r;
     const int n = lsdm_rem_pio2(x, &r);
@@ -309,7 +327,7 @@ LSDM_FN lsdm_dd lsdm_atan_ratio_fast(double a, double b) {
     lsdm_dd p = lsdm_two_prod(th, b);
     double rem = (a - p.h) - p.l; /* exact remainder of the division */
     double tl = lsdm_div_pos(rem, b);
-    int j = (int)(th * 64.0 + 0.5);
+    int j = lsdm_tab64(th);
     double uh, ul, Ah = 0.0, Al = 0.0;
     if (j == 0) {
         uh = th; ul = tl;
@@ -346,6 +364,34 @@ LSDM_SLOW double lsdm_atan2_slow(double ay, double ax, int swap, int xneg) {
     return r.h;
 }
 
+/* Finite non-zero |y|, |x| with one outside [2^-900, 2^900]: both times one power of two that puts the larger in [2^899, 2^900).
+ * Exact, unless the smaller then underflows — its ratio to the larger is below 2^-1900 and rounds to 0 either way.  Inside the
+ * range nothing changes, so those results keep their bits. */
+LSDM_FN void lsdm_atan2_prescale(double* ay, double* ax) {
+    if (*ay >= 0x1p-900 && *ay <= 0x1p900 && *ax >= 0x1p-900 && *ax <= 0x1p900) return;
+    const double s = (*ay > *ax ? *ay : *ax) < 0x1p-100 ? 0x1p1000 : 1.0;
+    double y = *ay * s, x = *ax * s;
+    const int e = (int)((lsdm_bits(y > x ? y : x) >> 52) & 0x7ff) - 1023; /* the larger is normal: e in [-100, 1023] */
+    const double t = lsdm_pow2i(899 - e);
+    *ay = y * t; *ax = x * t;
+}
+
+LSDM_FN double lsdm_dd_ldexp_round(lsdm_dd m, int e);
+
+/* atan(a/b) for 0 <= a/b < 2^-960 (a, b finite, b > 0): a result near or below the smallest normal, where phase 1's tail and
+ * error bound are subnormal and round too coarsely.  atan t = t - t^3/3 lies within t * 2^-1900 of t, so the result is t rounded
+ * once onto the 2^-1074 grid, except that an exact midpoint goes down: the quotient of the frexp mantissas as a double-double,
+ * nudged down by far less than any non-zero remainder, through the subnormal-aware rounding of exp. */
+LSDM_SLOW double lsdm_atan_tiny(double a, double b) {
+    if (a == 0.0) return 0.0; /* the prescale's underflow: a/b < 2^-1900 */
+    int ea, eb;
+    const double ma = frexp(a, &ea), mb = frexp(b, &eb); /* [0.5, 1) */
+    const double q = ma / mb;                               /* (0.5, 2) */
+    const lsdm_dd p = lsdm_two_prod(q, mb);
+    const double ql = ((ma - p.h) - p.l) / mb - q * 0x1p-150;
+    return lsdm_dd_ldexp_round(lsdm_dd_make(q, ql), ea - eb);
+}
+
 LSDM_FN double lsdm_atan2(double y, double x) {
     if (lsdm_isnan(x) || lsdm_isnan(y)) return x + y;
     int yneg = lsdm_signbit(y), xneg = lsdm_signbit(x);
@@ -360,25 +406,32 @@ LSDM_FN double lsdm_atan2(double y, double x) {
         else if (lsdm_isinf(ay)) r = LSDM_PIO2_H;
         else r = xneg ? LSDM_PI_H : 0.0;
     } else {
+        lsdm_atan2_prescale(&ay, &ax);
         int swap = ay > ax;
-        lsdm_dd f = swap ? lsdm_atan_ratio_fast(ax, ay) : lsdm_atan_ratio_fast(ay, ax);
-        if (swap) f = lsdm_const_minus(LSDM_PIO2_H, LSDM_PIO2_L, f);
-        if (xneg) f = lsdm_const_minus(LSDM_PI_H, LSDM_PI_L, f);
-        if (!lsdm_round_ok(f.h, f.l, &r)) r = lsdm_atan2_slow(ay, ax, swap, xneg);
+        if (!swap && !xneg && ay * 0x1p960 < ax) { /* |y/x| < 2^-960 exactly; pi/2 - t and pi - t take the general path */
+            r = lsdm_atan_tiny(ay, ax);
+        } else {
+            lsdm_dd f = swap ? lsdm_atan_ratio_fast(ax, ay) : lsdm_atan_ratio_fast(ay, ax);
+            if (swap) f = lsdm_const_minus(LSDM_PIO2_H, LSDM_PIO2_L, f);
+            if (xneg) f = lsdm_const_minus(LSDM_PI_H, LSDM_PI_L, f);
+            if (!lsdm_round_ok(f.h, f.l, &r)) r = lsdm_atan2_slow(ay, ax, swap, xneg);
+        }
     }
     return yneg ? -r : r;
 }
 LSDM_FN double lsdm_atan(double x) { return lsdm_atan2(x, 1.0); }
 
 /* Phase 1 of lsdm_atan2 for finite non-zero operands: returns 1 with *out == lsdm_atan2(y, x) when the rounding test
- * passes, 0 (output unspecified) when phase 2 is needed or an operand is zero / infinite / NaN — the caller then calls
- * lsdm_atan2.  Same operations as lsdm_atan2's general branch; the operands of the ratio are selected instead of the
+ * passes, 0 (output unspecified) when phase 2 is needed, the result is below 2^-960 or an operand is zero / infinite / NaN —
+ * the caller then calls lsdm_atan2.  Same operations as lsdm_atan2's general branch; the operands of the ratio are selected instead of the
  * call being duplicated, so a warp whose lanes disagree on |y| > |x| runs the ratio code once. */
 LSDM_FN int lsdm_atan2_try(double y, double x, double* out) {
-    const double ay = fabs(y), ax = fabs(x);
+    double ay = fabs(y), ax = fabs(x);
     if (!(ay > 0.0) || !(ax > 0.0) || lsdm_isinf(ax) || lsdm_isinf(ay)) return 0;   /* zero, NaN or infinite */
+    lsdm_atan2_prescale(&ay, &ax);
     const int yneg = lsdm_signbit(y), xneg = lsdm_signbit(x);
     const int swap = ay > ax;
+    if (!swap && !xneg && ay * 0x1p960 < ax) return 0;   /* lsdm_atan_tiny */
     const double lo = swap ? ax : ay, hi = swap ? ay : ax;
     lsdm_dd f = lsdm_atan_ratio_fast(lo, hi);
     if (swap) f = lsdm_const_minus(LSDM_PIO2_H, LSDM_PIO2_L, f);

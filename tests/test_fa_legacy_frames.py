@@ -301,6 +301,37 @@ def test_modes_capacity_and_argument_errors(lsdb, ctx, fm, gold):
 
 
 @pytest.mark.gpu
+def test_angles_beyond_2_19_are_rejected_before_any_launch(lsdb, ctx, fm, gold):
+    """A ray angle the device's sin / cos cannot reduce (|a| > LSDB_MAX_ANGLE = 2^19; the kernel adds up to 3 pi) is LSDB_ERR_ARG
+    in both entry points, found before any launch: the estimates stay untouched.  +-2^19 itself is accepted, NaN angles keep
+    their meaning (the ray falls outside the map), and the context keeps working."""
+    frames = make_frames(40, 17, gold["map_lines"])
+    res, ori = 0.05, (1.5, -2.0)
+    est, pose, coff = fm.legacy_frames(frames, res, ori, want_pose_all=True)
+    L = lsdb.lib()
+    p = lsdb._p
+    nf, lines, loff, lp, r, a, roff = fm.pack_legacy(frames)
+    k = int(roff[nf // 2]) + 1                                            # a ray of a frame in the middle of the batch
+    fr = next(f for f in frames if len(f["angles"]) > 1 and len(f["scan_lines"]) > 0)
+    for bad in (1e22, -1e22, np.nextafter(2.0 ** 19, np.inf), np.inf, -1.7976931348623157e308):
+        a2 = a.copy(); a2[k] = bad
+        e = np.frombuffer(b"\xab" * est.nbytes, lsdb.LEGACY_EST_DTYPE).copy(); c = np.full(nf + 1, -7, np.int32)
+        assert L.lsdb_fa_legacy_frames(ctx.h, fm.h, nf, p(lines), p(loff), res, ori[0], ori[1], p(lp), p(r), p(a2), p(roff), p(e),
+                                       None, 0, p(c)) == 2
+        assert "lsdb_fa_legacy_frames: the angle of ray %d" % k in L.lsdb_last_error(ctx.h).decode()
+        assert (e.view(np.uint8) == 0xAB).all() and (c == -7).all()
+        one = np.asarray(fr["angles"], np.float64).copy(); one[1] = bad
+        with pytest.raises(lsdb.LsdbError, match="ARG"):
+            fm.legacy(fr["scan_lines"], res, ori, fr["lidar_pos"], fr["ranges"], one)
+        assert "lsdb_fa_legacy: the angle of ray 1" in L.lsdb_last_error(ctx.h).decode()
+    for edge in (2.0 ** 19, -(2.0 ** 19), np.nan):
+        one = np.asarray(fr["angles"], np.float64).copy(); one[1] = edge
+        fm.legacy(fr["scan_lines"], res, ori, fr["lidar_pos"], fr["ranges"], one)
+    est2, pose2, coff2 = fm.legacy_frames(frames, res, ori, want_pose_all=True)
+    assert est2.tobytes() == est.tobytes() and _same(pose2, pose) and np.array_equal(coff2, coff)
+
+
+@pytest.mark.gpu
 def test_ten_thousand_frames_in_one_call(fm, gold):
     frames = make_frames(10000, 19, gold["map_lines"])
     res, ori = 0.05, (1.5, -2.0)

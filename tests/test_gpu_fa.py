@@ -158,3 +158,59 @@ def test_kept_hypotheses_equal_the_filtered_full_table(lsdb, ctx):
     none, nh0 = fm.score_kept([frames[5]])
     assert len(none) == 0 and nh0 == 0
     fm.close()
+
+
+def _bits_equal(a, b):
+    """same shape and the same bits, a NaN on both sides counting as equal (so -0 differs from +0)"""
+    a = np.asarray(a, np.float64); b = np.asarray(b, np.float64)
+    return a.shape == b.shape and np.array_equal(np.isnan(a), np.isnan(b)) and \
+        np.array_equal(a[~np.isnan(a)].view(np.int64), b[~np.isnan(b)].view(np.int64))
+
+
+def _degenerate(lines):
+    """copies of line records (the lengths kept, so the length filters still pair them) with degenerate end points: vertical with
+    dx = +-0, dx = +-5e-324 / 1e-310 / 1e-300 under dy = 1 (|dy/dx| overflows or reaches 1e300, where atan used to overflow on the
+    host), horizontal (dy = 0), zero length"""
+    out = []
+    for ln in lines:
+        for x1, x2, dy in [(0.0, 0.0, 1.0), (0.0, -0.0, 1.0), (-0.0, 0.0, -1.0), (3.0, 3.0, -2.0)] + \
+                          [(0.0, s * d, 1.0) for d in (5e-324, 1e-310, 1e-300) for s in (1.0, -1.0)] + \
+                          [(12.0, 15.0, 0.0), (15.0, 12.0, 0.0), (7.0, 7.0, 0.0)]:
+            r = np.array(ln, np.float64)
+            r[4], r[6], r[7] = x1, x2, r[5] + dy
+            out.append(r)
+    return np.array(out)
+
+
+def test_degenerate_line_geometry(lsdb, ctx):
+    """Vertical, horizontal, nearly vertical (|dy/dx| up to 2^1074) and zero-length scan and map lines through both association
+    paths: lsdb_fa_score's poses and lsdb_fa_legacy_frames' records have the oracle's bits."""
+    m = synth.occupancy_grid(500, 400, seed=31)
+    o = oraclebind.lsd(m)
+    mc = oraclebind.map_cache(m, 0.05)
+    fr = synth.fake_scan_frame(m, o["lines"], seed=4)
+    ml = np.concatenate([o["lines"], _degenerate(o["lines"][:3])])
+    sl = np.concatenate([fr["scan_lines"][:2], _degenerate(fr["scan_lines"][:3])])
+    fm = lsdb.FaMap(ctx, mc, ml)
+    frames = [dict(fr, scan_lines=sl), dict(fr, scan_lines=sl, last_pose=np.array([-1.0, -1.0, 0.0]))]
+    hyp = fm.score(frames)
+    n_deg = 0
+    for f, frame in enumerate(frames):
+        h = hyp[hyp["frame"] == f]
+        oi, ov = oraclebind.fa_scores(frame["scan_lines"], ml, frame["pts"], mc, frame["lidar_pose"], frame["last_pose"])
+        assert np.array_equal(np.stack([h["i_scan"], h["i_map"], h["i_pair"]], 1), oi)
+        for j, k in enumerate(("x", "y", "ang")):
+            assert _bits_equal(h[k], ov[:, j]), k
+        fin = np.isfinite(ov[:, 3])
+        assert np.array_equal(np.isfinite(h["score"]), fin)
+        assert np.allclose(h["score"][fin], ov[fin, 3], rtol=1e-9)
+        n_deg += int(((oi[:, 0] >= 2) | (oi[:, 1] >= len(o["lines"]))).sum())
+    assert n_deg > 100                                                   # the degenerate lines do get paired
+    r, a = synth.lidar_frame(5)
+    lp = np.rint(np.asarray(fr["lidar_pose"], np.float64)).astype(np.int32)
+    res, ori = 0.05, (1.5, -2.0)
+    est, pose, coff = fm.legacy_frames([dict(scan_lines=sl, lidar_pos=lp, ranges=r, angles=a)], res, ori, want_pose_all=True)
+    want, we, wr = oraclebind.fa_legacy(sl, ml, res, ori, lp, mc, r, a)
+    assert len(pose) > 100 and _bits_equal(pose, want)
+    assert _bits_equal(est[0]["estimate_pose"], we) and _bits_equal(est[0]["estimate_pose_realworld"], wr)
+    fm.close()

@@ -142,6 +142,33 @@ def test_error_paths(lsdb, ctx):
     assert b"max_lines" in L.lsdb_last_error(ctx.h)
 
 
+def test_angles_beyond_2_19_are_rejected_before_any_launch(lsdb, ctx):
+    """A finite angle the device's sin / cos cannot reduce (|a| > LSDB_MAX_ANGLE = 2^19) is LSDB_ERR_ARG, found on the host
+    before anything is launched or written; +-2^19 itself is accepted, and the context keeps working."""
+    import ctypes as C
+    L = lsdb.lib()
+    r, a = synth.lidar_frame(1)
+    base = ctx.feature_scan(MP[2], MP[3], MP[4], [(r, a)])
+    boff = np.array([0, len(r)], np.int32); prm = lsdb._RdpParams(3, 0.08, 0.5)
+    p = lambda x: x.ctypes.data_as(C.c_void_p)  # noqa: E731
+    for bad in (1e22, -1e22, 2.0 ** 19 + 2.0 ** -33, 1.7976931348623157e308):
+        a2 = a.copy(); a2[7] = bad
+        info = np.frombuffer(b"\xab" * lsdb.SCAN_INFO_DTYPE.itemsize, lsdb.SCAN_INFO_DTYPE).copy()
+        loff = np.zeros(2, np.int32); poff = np.zeros(2, np.int32); ioff = np.zeros(2, np.int64)
+        assert L.lsdb_feature_scan_frames(ctx.h, MP[2], MP[3], MP[4], C.byref(prm), 1, p(r), p(a2), p(boff), p(info),
+                                          None, 0, p(loff), None, 0, p(poff), None, 0, p(ioff)) == 2
+        assert b"angle of beam 7" in L.lsdb_last_error(ctx.h)
+        assert (info.view(np.uint8) == 0xAB).all()                        # nothing ran: the sizing query's output is untouched
+        with pytest.raises(lsdb.LsdbError, match="ARG"):
+            ctx.feature_scan(MP[2], MP[3], MP[4], [(r, a2)])
+    for edge in (2.0 ** 19, -(2.0 ** 19)):
+        a3 = a.copy(); a3[7] = edge
+        assert len(ctx.feature_scan(MP[2], MP[3], MP[4], [(r, a3)])) == 1
+    again = ctx.feature_scan(MP[2], MP[3], MP[4], [(r, a)])
+    assert np.array_equal(lsdb.lines_to_array(again[0]["lines"]), lsdb.lines_to_array(base[0]["lines"]), equal_nan=True)
+    assert np.array_equal(again[0]["pts"], base[0]["pts"])
+
+
 def test_scan_to_estimate_chain(lsdb, ctx):
     """lidar frames -> device FeatureScan -> device scoring + reduction: the same estimates as from the reference's
     scan lines / points of the golden association fixture"""

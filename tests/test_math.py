@@ -3,6 +3,7 @@ import ctypes as C
 import math
 import os
 import subprocess
+import sys
 
 import mpmath as mp
 import numpy as np
@@ -127,6 +128,8 @@ def test_pow(L):
     cases += [(float(x), 6.0) for x in list(range(16, 2000, 13)) + [9741, 9742, 20000, 65536, 100000]]  # Windschitl, :909
     cases += [(float(a), float(b)) for a, b in zip(rng.uniform(0, 2, 1200), rng.integers(1, 4000, 1200))]  # tail bound, :1052
     cases += [(float(a), float(b)) for a, b in zip(10 ** rng.uniform(-5, 5, 600), rng.uniform(-50, 50, 600))]
+    # small integer powers whose operands reach [2^996, 2^1000), where Dekker's split used to overflow on the host only
+    cases += [(float(2.0 ** ((996 + 4 * u) / n)), float(n)) for n in (3, 4, 7, 8, 16, 31, 32, 33, 63, 64) for u in rng.random(12)]
     for x, y in cases:
         assert L.t_pow(x, y) == _cr(mp.power(mp.mpf(x), mp.mpf(y))), (x, y)
     assert L.t_pow(3.7, 2.0) == 3.7 * 3.7 and L.t_pow(5.0, 0.0) == 1.0
@@ -138,3 +141,100 @@ def test_close_to_glibc(L):
     xs = rng.uniform(-np.pi, np.pi, 20000)
     d = [abs(L.t_sin(float(x)) - math.sin(x)) / max(abs(math.sin(x)), 1e-300) for x in xs]
     assert max(d) < 3e-16 and sum(1 for v in d if v > 0) < 200
+
+
+_OUT_OF_DOMAIN = r"""
+import ctypes as C, sys
+lib = C.CDLL(sys.argv[1])
+lib.t_sin.restype = lib.t_cos.restype = C.c_double
+lib.t_sin.argtypes = lib.t_cos.argtypes = [C.c_double]
+n = 0
+for line in sys.stdin:
+    x = float.fromhex(line)
+    s, c, ok = C.c_double(7.0), C.c_double(7.0), C.c_ubyte(7)
+    k = lib.v_sincos_try(C.byref(C.c_double(x)), C.byref(s), C.byref(c), C.byref(ok), 1)
+    assert lib.t_sin(x) != lib.t_sin(x) and lib.t_cos(x) != lib.t_cos(x) and k == 0 and ok.value == 0, x.hex()
+    n += 1
+print(n)
+"""
+
+
+def test_sin_cos_beyond_the_reduction_range_are_nan():
+    """lsdm_rem_pio2 is exact for |x| <= 2^20 only; beyond it sin / cos return NaN and lsdm_sincos_try fails, before any table
+    lookup (an index past the tables once read far outside them: sin(1e22) crashed, sin(2^63) was 7e211).  Run in a child
+    process, so that an out-of-bounds read fails this test instead of ending the session."""
+    subprocess.check_call(["make", "-s", "-C", HERE, "all"])
+    rng = np.random.default_rng(9)
+    mags = [math.nextafter(2.0 ** 20, math.inf), 2.0 ** 20 + 1, 2.0 ** 21, 2.0 ** 30, 1e22, 2.0 ** 63, 1e300, 2.0 ** 1023,
+            1.7976931348623157e308] + list(2.0 ** rng.uniform(20.0001, 1024, 3000))
+    xs = [s * float(m) for m in mags for s in (1.0, -1.0) if math.isfinite(m)]
+    p = subprocess.run([sys.executable, "-c", _OUT_OF_DOMAIN, os.path.join(HERE, "_mathlib.so")], input="\n".join(x.hex() for x in xs),
+                       capture_output=True, text=True, timeout=120)
+    assert p.returncode == 0, (p.returncode, p.stderr[-2000:])
+    assert int(p.stdout) == len(xs)
+
+
+def test_sin_cos_at_the_edge_of_the_reduction_range(L):
+    """2^20 itself and the doubles just below it are still in the domain and correctly rounded"""
+    xs = [2.0 ** 20, math.nextafter(2.0 ** 20, 0), 2.0 ** 20 - 1, 2.0 ** 19 + 0.5, 1048575.9999999999]
+    xs += [-x for x in xs]
+    _check(L.t_sin, mp.sin, xs); _check(L.t_cos, mp.cos, xs)
+
+
+def _any_double(rng, n):
+    """n doubles of every magnitude, subnormals included: a random 52-bit mantissa and a uniform biased exponent 0..2046"""
+    bits = (rng.integers(0, 2047, n, dtype=np.int64) << 52) | rng.integers(0, 1 << 52, n, dtype=np.int64)
+    return bits.view(np.float64) * rng.choice([-1.0, 1.0], n)
+
+
+def test_atan2_atan_across_the_exponent_range(L):
+    """Any finite operands — subnormal, near DBL_MAX, ratios that overflow or underflow — give the correctly rounded atan2 / atan.
+    Operands at or above 2^997 used to overflow the error-free product and return NaN on the host."""
+    rng = np.random.default_rng(10)
+    ys, xs = _any_double(rng, 3000), _any_double(rng, 3000)
+    with np.errstate(over="ignore"):
+        near = xs[:500] * 2.0 ** rng.integers(-60, 60, 500)                          # ratios 2^-60..2^60 at every scale
+    ys[:500] = np.where(np.isfinite(near) & (near != 0), near, ys[:500])
+    pairs = list(zip(ys.tolist(), xs.tolist()))
+    pairs += [(2.0 ** 997, 1.0), (1e305, 1.0), (1.0, 1e305), (-1.0, -1e305), (1e308, 5e-324), (5e-324, 1e308), (5e-324, 5e-324),
+              (-5e-324, 3 * 5e-324), (1e-310, -1e-300), (2.0 ** -900, 2.0 ** 900), (math.nextafter(2.0 ** -900, 0), 1.0),
+              (1.7976931348623157e308, -1.7976931348623157e308), (1.7976931348623157e308, 1.0), (2.0 ** 900, math.nextafter(2.0 ** 900, math.inf))]
+    P = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+    y = np.array([p[0] for p in pairs]); x = np.array([p[1] for p in pairs])
+    o = np.empty(len(y)); ok = np.empty(len(y), np.uint8)
+    L.v_atan2_try(P(y), P(x), P(o), P(ok), len(y))
+    for i, (yy, xx) in enumerate(pairs):
+        want = math.copysign(_cr(mp.atan2(abs(mp.mpf(yy)), mp.mpf(xx))), yy)       # odd in y, the sign of a zero result too
+        got = L.t_atan2(yy, xx)
+        assert got == want and math.copysign(1, got) == math.copysign(1, want), (yy.hex(), xx.hex())
+        assert L.t_atan2_slow(yy, xx) == want, (yy.hex(), xx.hex())
+        assert not ok[i] or o[i] == want, (yy.hex(), xx.hex())
+    with np.errstate(all="ignore"):
+        tiny = (x > 0) & (np.abs(y) * 2.0 ** 960 < x)                                # results below 2^-960 skip phase 1
+    assert not ok[tiny].any() and ok[~tiny].mean() > 0.99
+    _check(L.t_atan, mp.atan, np.concatenate([_any_double(rng, 2000), [2.0 ** 997, -2.0 ** 1000, 1.7976931348623157e308, 5e-324, -1e-310]]))
+    assert L.t_atan(1.7976931348623157e308) == math.pi / 2 and L.t_atan2(5e-324, 1.0) == 5e-324
+
+
+def test_device_math_is_built_with_the_product_device_flags():
+    """tests/devmath.cu (the device build test_gpu_math.py checks) must compile lsd_math.h as the product does: same target,
+    same optimisation, and above all no contraction of a*b+c into an FMA, which would change the device's bits."""
+    import re
+
+    def flags(path, var):
+        with open(path) as f:
+            text = f.read()
+        defs = dict(re.findall(r"^(\w+)\s*:?=(.*)$", text, re.M))
+        v = defs[var]
+        for name, val in defs.items():
+            v = v.replace("$(%s)" % name, val)
+        return v.split()
+
+    prod = flags(os.path.join(HERE, "..", "linesegmentdetector-slam_b200", "Makefile"), "NVFLAGS")
+    test = flags(os.path.join(HERE, "Makefile"), "DEVFLAGS")
+    for f in prod + test:
+        if f.startswith("-fmad") or f.startswith("--fmad"):
+            assert f in ("-fmad=false", "--fmad=false"), f
+    assert "-fmad=false" in prod and "-fmad=false" in test
+    pick = lambda fl: [f for f in fl if f.startswith(("-O", "arch=", "-gencode", "-arch", "--use_fast_math", "-ftz", "-prec"))]  # noqa: E731
+    assert pick(prod) == pick(test), (prod, test)
