@@ -12,6 +12,7 @@
  *                                 (thread_ScanToMapMatch), :274-305, :307-355, :357-396
  *   lsdb_hypothesis           <- structScore                            LSD/myFA.h:49-54
  *   lsdb_map_cache            <- mylsd::createMapCache                  LSD/myLSD.h:131, LSD/myLSD.cpp:11-127
+ *   lsdb_batch_map_caches     <- the same for every map of a batch, on the device
  *
  * There is no CPU fallback: every compute entry point fails with LSDB_ERR_NO_DEVICE / LSDB_ERR_CUDA
  * when no sm_100 device is usable.  All functions return LSDB_OK (0) or an error code; the text of
@@ -155,6 +156,18 @@ int lsdb_map_cache(lsdb_ctx* ctx, const uint8_t* map, int cols, int rows, double
  * defined behaviour and the one implemented. */
 int lsdb_map_cache_fill(lsdb_ctx* ctx, const uint8_t* map, int cols, int rows, double res, double max_dist, double unreached,
                         double* out);
+/* createMapCache (LSD/myLSD.cpp:11-127; the snapshot's 3-argument flavour via `unreached`) for every map of the batch, on the device,
+ * from the source planes lsdb_batch_upload / lsdb_batch_upload_scan_rasters left (value 1 = occupied).  res[n_maps] (> 0, finite);
+ * max_dist >= 0; unreached = value of cells the fire never reaches (max_dist for the current source, 2 for the snapshot).
+ * out: NULL (keep on the device only) or n_maps host pointers (rows*cols f64 each; NULL entries skipped).  Independent of
+ * lsdb_batch_run: before or after it, the result is the same.  Cell for cell what lsdb_map_cache_fill returns for each map alone.
+ * The caches stay in a plane the batch owns (8 bytes per source pixel, allocated on the first call, overwritten by the next).
+ * LSDB_ERR_ARG: res NULL, a res not finite and > 0, max_dist < 0 or NaN, a map with more than 65535 columns or rows. */
+int lsdb_batch_map_caches(lsdb_batch* b, const double* res, double max_dist, double unreached, double* const* out);
+/* An association map from map i of the batch: its cache (lsdb_batch_map_caches must have run) copied device to device, and its
+ * segment table exactly as lsdb_batch_download returns it (the batch must have run).  The lsdb_fa_map owns its copies.
+ * LSDB_ERR_ARG: out NULL, i out of range, before lsdb_batch_run or before lsdb_batch_map_caches. */
+int lsdb_fa_map_create_from_batch(lsdb_batch* b, int i, lsdb_fa_map** out);
 
 /* ---- one process, several GPUs ---- */
 /* A batch of independent maps split contiguously over the listed devices (the first n % k devices get one map more), one host

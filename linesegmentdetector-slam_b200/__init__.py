@@ -84,6 +84,8 @@ def lib():
         L.lsdb_lsd.argtypes = [vp, vp, ci, ci, C.POINTER(_Params), vp, ci, vp, vp, vp]
         L.lsdb_map_cache.argtypes = [vp, vp, ci, ci, cd, cd, vp]
         L.lsdb_map_cache_fill.argtypes = [vp, vp, ci, ci, cd, cd, cd, vp]
+        L.lsdb_batch_map_caches.argtypes = [vp, vp, cd, cd, vp]
+        L.lsdb_fa_map_create_from_batch.argtypes = [vp, ci, C.POINTER(vp)]
         L.lsdb_multi_create.argtypes = [C.POINTER(vp), vp, ci]
         L.lsdb_multi_destroy.argtypes = [vp]; L.lsdb_multi_destroy.restype = None
         L.lsdb_multi_last_error.argtypes = [vp]; L.lsdb_multi_last_error.restype = C.c_char_p
@@ -379,6 +381,18 @@ class Batch:
         self.ctx.check(lib().lsdb_batch_line_images(self.h, ptrs), "lsdb_batch_line_images")
         return outs
 
+    def map_caches(self, res, max_dist=1.0, unreached=None, download=True):
+        """mylsd::createMapCache of every map of the batch, on the device, from the uploaded source planes
+        (lsdb_batch_map_caches).  `res`: one resolution for all maps or one per map; `unreached` = the value of the cells
+        the brush fire never reaches (default max_dist; the catkin snapshot stores 2).  The caches stay on the device for
+        FaMap.from_batch; with download=True they also come back as a list of rows x cols f64 arrays, else None."""
+        r = np.ascontiguousarray(np.broadcast_to(np.asarray(res, np.float64), (self.n,)))
+        outs = [np.empty((rows, cols)) for cols, rows in self.sizes] if download else None
+        ptrs = (C.c_void_p * self.n)(*[o.ctypes.data for o in outs]) if download else None
+        self.ctx.check(lib().lsdb_batch_map_caches(self.h, _p(r), float(max_dist), float(max_dist if unreached is None else unreached), ptrs),
+                       "lsdb_batch_map_caches")
+        return outs
+
     def planes(self, i):
         W, H = self.scaled(i)
         mag = np.zeros((H, W)); deg = np.zeros((H, W)); used = np.zeros((H, W), np.uint8)
@@ -441,6 +455,17 @@ class FaMap:
         rows, cols = mc.shape
         ctx.check(lib().lsdb_fa_map_create(ctx.h, _p(mc), cols, rows, _p(ml), len(ml), C.byref(self.h)), "lsdb_fa_map_create")
         self.n_lines = len(ml)
+
+    @classmethod
+    def from_batch(cls, batch, i):
+        """lsdb_fa_map_create_from_batch: map i of `batch` — its cache from Batch.map_caches, copied on the device, and its
+        segment table as Batch.download returns it.  The FaMap owns its copies and outlives the batch."""
+        self = cls.__new__(cls)
+        self.ctx = batch.ctx
+        self.h = C.c_void_p()
+        batch.ctx.check(lib().lsdb_fa_map_create_from_batch(batch.h, int(i), C.byref(self.h)), "lsdb_fa_map_create_from_batch")
+        self.n_lines = int(batch.counts()[i])
+        return self
 
     def _marshal(self, frames):
         nf = len(frames)

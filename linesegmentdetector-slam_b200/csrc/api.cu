@@ -54,11 +54,12 @@ struct lsdb_batch {
     int* labels; LsdbRect* rects; LsdbImgDyn* dyn; LsdbImg* imgsD; int* tileImg; unsigned int* lists;
     int* imgCounter; LsdbLsdConst* kcD; double* gaussDbg; unsigned char* recBuf; unsigned int* banBits;
     uint8_t* lineImD;   // lineIm planes of all maps (allocated on first use by lsdb_batch_line_images; geometry of src)
+    double* mcCache;    // mapCache planes of all maps, rows*cols f64 each, packed in batch order (allocated on first use by lsdb_batch_map_caches)
     unsigned int* nzBits; int2* bandOf; int2* bandsOfImg; unsigned int* orderTabs; int nBands;   // ordering stage: "mag != 0" bits, row bands, count tables
     // host (pinned)
     LsdbImgDyn* dynH; LsdbRect* rectsH;
     cudaEvent_t ev[4];
-    bool ran, downloaded;
+    bool ran, downloaded, mcReady;
     int launches;
 };
 
@@ -171,7 +172,7 @@ extern "C" void lsdb_batch_destroy(lsdb_batch* b) {
     cudaFree(b->src); cudaFree(b->mag); cudaFree(b->deg); cudaFree(b->cosm); cudaFree(b->state); cudaFree(b->bins); cudaFree(b->cells);
     cudaFree(b->labels); cudaFree(b->rects); cudaFree(b->dyn); cudaFree(b->imgsD); cudaFree(b->tileImg); cudaFree(b->lists);
     cudaFree(b->imgCounter); cudaFree(b->kcD); cudaFree(b->gaussDbg); cudaFree(b->recBuf); cudaFree(b->banBits);
-    cudaFree(b->lineImD); cudaFree(b->nzBits); cudaFree(b->bandOf); cudaFree(b->bandsOfImg); cudaFree(b->orderTabs);
+    cudaFree(b->lineImD); cudaFree(b->mcCache); cudaFree(b->nzBits); cudaFree(b->bandOf); cudaFree(b->bandsOfImg); cudaFree(b->orderTabs);
     cudaFreeHost(b->dynH); cudaFreeHost(b->rectsH);
     for (int i = 0; i < 4; i++) cudaEventDestroy(b->ev[i]);
     if (b->ctx->cached == b) b->ctx->cached = 0;
@@ -189,7 +190,7 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
     memset(&b->kc, 0, sizeof b->kc);
     b->ctx = ctx; b->n = n; b->params = *prm; b->ran = false; b->downloaded = false; b->launches = 0;
     b->src = 0; b->mag = 0; b->deg = 0; b->cosm = 0; b->sinm = 0; b->state = 0; b->bins = 0; b->cells = 0; b->labels = 0; b->rects = 0; b->dyn = 0;
-    b->imgsD = 0; b->tileImg = 0; b->lists = 0; b->imgCounter = 0; b->kcD = 0; b->gaussDbg = 0; b->recBuf = 0; b->banBits = 0; b->dynH = 0; b->rectsH = 0; b->lineImD = 0; b->nzBits = 0; b->bandOf = 0; b->bandsOfImg = 0; b->orderTabs = 0; b->nBands = 0;
+    b->imgsD = 0; b->tileImg = 0; b->lists = 0; b->imgCounter = 0; b->kcD = 0; b->gaussDbg = 0; b->recBuf = 0; b->banBits = 0; b->dynH = 0; b->rectsH = 0; b->lineImD = 0; b->mcCache = 0; b->mcReady = false; b->nzBits = 0; b->bandOf = 0; b->bandsOfImg = 0; b->orderTabs = 0; b->nBands = 0;
     for (int i = 0; i < 4; i++) cudaEventCreate(&b->ev[i]);
     b->maxSeg = maxLines > 0 ? maxLines : 4096;
 
@@ -664,6 +665,42 @@ extern "C" int lsdb_map_cache(lsdb_ctx* ctx, const uint8_t* map, int cols, int r
     return lsdb_map_cache_fill(ctx, map, cols, rows, res, maxDist, maxDist, out);   // LSD/myLSD.cpp:37
 }
 
+// element offset of map i in the batch's mapCache plane (the maps' rows*cols cells packed in batch order)
+static size_t cache_off(const lsdb_batch* b, int i) {
+    size_t off = 0;
+    for (int k = 0; k < i; k++) off += (size_t)b->imgs[k].cols * b->imgs[k].rows;
+    return off;
+}
+
+extern "C" int lsdb_batch_map_caches(lsdb_batch* b, const double* res, double maxDist, double unreached, double* const* out) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!res || !(maxDist >= 0)) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_map_caches: res must be given and max_dist >= 0%s");
+    for (int i = 0; i < b->n; i++) {
+        if (!(res[i] > 0) || !std::isfinite(res[i])) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_map_caches: res of map %s%lld is not finite and > 0", "", i);
+        if (b->imgs[i].cols > 65535 || b->imgs[i].rows > 65535)
+            return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_map_caches: map %s%lld has more than 65535 columns or rows", "", i);
+    }
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t total = cache_off(b, b->n);
+    if (!b->mcCache) CK(ctx, cudaMalloc((void**)&b->mcCache, total * 8));
+    std::vector<LsdbMcMap> maps(b->n);
+    for (int i = 0; i < b->n; i++) {
+        const LsdbImg& im = b->imgs[i];
+        maps[i] = LsdbMcMap{im.srcOff, i ? maps[i - 1].cacheOff + (size_t)maps[i - 1].cols * maps[i - 1].rows : 0, 0, im.cols, im.rows, im.srcPitch,
+                            lsdb_mc_cell_radius(maxDist, res[i]), res[i]};
+    }
+    b->mcReady = false;
+    const cudaError_t e = lsdb_map_caches_run(ctx->stream, b->n, maps.data(), b->src, unreached, b->mcCache);
+    if (e != cudaSuccess) return fail(ctx, LSDB_ERR_CUDA, "lsdb_batch_map_caches: %s", cudaGetErrorString(e));
+    b->mcReady = true;
+    if (!out) return LSDB_OK;
+    for (int i = 0; i < b->n; i++)
+        if (out[i]) CK(ctx, cudaMemcpyAsync(out[i], b->mcCache + maps[i].cacheOff, (size_t)b->imgs[i].cols * b->imgs[i].rows * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return LSDB_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ association
 struct lsdb_fa_map {
     lsdb_ctx* ctx;
@@ -673,21 +710,42 @@ struct lsdb_fa_map {
     std::vector<lsdb_line> lines;
 };
 
-extern "C" int lsdb_fa_map_create(lsdb_ctx* ctx, const double* mapCache, int cols, int rows, const lsdb_line* mapLines,
-                                  int nLines, lsdb_fa_map** out) {
-    if (!ctx || !mapCache || !out || cols <= 0 || rows <= 0 || nLines < 0 || (nLines > 0 && !mapLines)) return fail(ctx, LSDB_ERR_ARG, "lsdb_fa_map_create: bad argument%s");
+// a new lsdb_fa_map with its own copies of the cache (from host or device memory, `kind`) and of the lines (host)
+static int fa_map_new(lsdb_ctx* ctx, const char* what, const double* mapCache, cudaMemcpyKind kind, int cols, int rows, const lsdb_line* mapLines,
+                      int nLines, lsdb_fa_map** out) {
     CK(ctx, cudaSetDevice(ctx->device));
     lsdb_fa_map* m = new lsdb_fa_map();
     m->ctx = ctx; m->cols = cols; m->rows = rows; m->nLines = nLines; m->cacheD = 0; m->linesD = 0;
     m->lines.assign(mapLines, mapLines + nLines);
     cudaError_t e = cudaMalloc((void**)&m->cacheD, (size_t)cols * rows * 8);
     if (e == cudaSuccess) e = cudaMalloc((void**)&m->linesD, sizeof(LsdbFaLine) * (size_t)(nLines > 0 ? nLines : 1));
-    if (e == cudaSuccess) e = cudaMemcpyAsync(m->cacheD, mapCache, (size_t)cols * rows * 8, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(m->cacheD, mapCache, (size_t)cols * rows * 8, kind, ctx->stream);
     if (e == cudaSuccess && nLines) e = cudaMemcpyAsync(m->linesD, mapLines, sizeof(LsdbFaLine) * (size_t)nLines, cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { cudaFree(m->cacheD); cudaFree(m->linesD); delete m; return fail(ctx, LSDB_ERR_CUDA, "lsdb_fa_map_create: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { cudaFree(m->cacheD); cudaFree(m->linesD); delete m; return fail(ctx, LSDB_ERR_CUDA, what, cudaGetErrorString(e)); }
     *out = m;
     return LSDB_OK;
+}
+
+extern "C" int lsdb_fa_map_create(lsdb_ctx* ctx, const double* mapCache, int cols, int rows, const lsdb_line* mapLines,
+                                  int nLines, lsdb_fa_map** out) {
+    if (!ctx || !mapCache || !out || cols <= 0 || rows <= 0 || nLines < 0 || (nLines > 0 && !mapLines)) return fail(ctx, LSDB_ERR_ARG, "lsdb_fa_map_create: bad argument%s");
+    return fa_map_new(ctx, "lsdb_fa_map_create: %s", mapCache, cudaMemcpyHostToDevice, cols, rows, mapLines, nLines, out);
+}
+
+extern "C" int lsdb_fa_map_create_from_batch(lsdb_batch* b, int i, lsdb_fa_map** out) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!out || i < 0 || i >= b->n) return fail(ctx, LSDB_ERR_ARG, "lsdb_fa_map_create_from_batch: bad argument%s");
+    if (!b->ran) return fail(ctx, LSDB_ERR_ARG, "lsdb_fa_map_create_from_batch before lsdb_batch_run%s");
+    if (!b->mcReady) return fail(ctx, LSDB_ERR_ARG, "lsdb_fa_map_create_from_batch before lsdb_batch_map_caches%s");
+    if (!b->downloaded) { const int rc = lsdb_batch_download(b, 0, 0, 0); if (rc) return rc; }
+    const int ns = b->dynH[i].nSeg;
+    std::vector<lsdb_line> lines(ns > 0 ? ns : 1);
+    for (int j = 0; j < ns; j++) line_from_rect(b->rectsH[(size_t)i * b->maxSeg + j], b->kc.pi, &lines[j]);
+    const LsdbImg& im = b->imgs[i];
+    return fa_map_new(ctx, "lsdb_fa_map_create_from_batch: %s", b->mcCache + cache_off(b, i), cudaMemcpyDeviceToDevice, im.cols, im.rows,
+                      lines.data(), ns, out);
 }
 
 extern "C" void lsdb_fa_map_destroy(lsdb_fa_map* m) {

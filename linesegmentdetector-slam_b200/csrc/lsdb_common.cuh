@@ -134,6 +134,13 @@ void lsdb_launch_fa_pairs_count(cudaStream_t s, int nL, const LsdbFaLine* scanLi
 void lsdb_launch_fa_pairs_write(cudaStream_t s, int nL, int nFrames, const LsdbFaLine* scanLines, const int* lineOff, const LsdbFaLine* mapLines,
                                 int nMap, const int* scratch, LsdbFaTask* tasks, int* hypOff);
 
+// createMapCache of several maps (mapcache.cu).  Map i: cols x rows cells (<= 65535 each) at src + srcOff, srcPitch bytes per
+// row; its rows*cols f64 result at cache + cacheOff.  loc is set by lsdb_map_caches_run (the map's first cell in its group).
+struct LsdbMcMap { unsigned long long srcOff, cacheOff, loc; int cols, rows, srcPitch, cellRadius; double res; };
+int lsdb_mc_cell_radius(double maxDist, double res);
+// every map's cache, cell for cell what the map alone gives; synchronises the stream (it reads one count per BFS level)
+cudaError_t lsdb_map_caches_run(cudaStream_t s, int nMaps, const LsdbMcMap* maps, const uint8_t* src, double unreached, double* cache);
+
 // scan front-end (fscan.cu)
 struct LsdbFsInfo { int nLines, nPts, W, H; double lidarX, lidarY; };  // == lsdb_scan_info; nLines < 0: internal list overflow
 struct LsdbFsPiece { double x1, y1, x2, y2; int off, pad; };            // a kept line piece: end points, offset of its samples in the frame
