@@ -43,7 +43,11 @@ typedef struct lsdb_ctx lsdb_ctx;
 typedef struct lsdb_batch lsdb_batch;
 typedef struct lsdb_fa_map lsdb_fa_map;
 
-/* arguments 4-8 of myLineSegmentDetector (LSD/myLSD.h:132); defaults LSD/baseFunc.h:64-68 */
+/* arguments 4-8 of myLineSegmentDetector (LSD/myLSD.h:132); defaults LSD/baseFunc.h:64-68.
+ * Domain (lsdb_batch_create and lsdb_lsd return LSDB_ERR_ARG outside it, before anything is allocated):
+ * sca in (0,1], angThre in the open interval (0,180) degrees, denThre finite, pseBin in [1,1024].  Inside it the result is
+ * the reference's for any value (tests/test_gpu_lsd_params.py sweeps angThre from 1 to 179, denThre from 0 to 1.5, pseBin
+ * from 1 to 1023). */
 typedef struct {
     double sca;      /* 0.3  (the 3-phase Gaussian is only defined for 0.3, LSD/baseFunc.h:64) */
     double sig;      /* 0.6  */

@@ -185,6 +185,10 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
     *out = 0;
     if (prm->pseBin < 1 || prm->pseBin > 1024) return fail(ctx, LSDB_ERR_ARG, "pseBin must be in [1,1024]%s");
     if (!(prm->sca > 0 && prm->sca <= 1)) return fail(ctx, LSDB_ERR_ARG, "sca must be in (0,1]%s");
+    // outside (0,180) the thresholds derived from angThre mean nothing: regThre divides by log10(angThre/180), which is then
+    // >= 0 or NaN, and aliPro = angThre/180 >= 1 makes the NFA's log(1-p) NaN
+    if (!(prm->angThre > 0 && prm->angThre < 180)) return fail(ctx, LSDB_ERR_ARG, "angThre must be in (0,180) degrees%s");
+    if (!std::isfinite(prm->denThre)) return fail(ctx, LSDB_ERR_ARG, "denThre must be finite%s");
     CK(ctx, cudaSetDevice(ctx->device));
     lsdb_batch* b = new lsdb_batch();
     memset(&b->kc, 0, sizeof b->kc);

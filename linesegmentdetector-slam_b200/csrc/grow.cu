@@ -519,6 +519,7 @@ __device__ __forceinline__ int grow_region(WarpCtx& c, int sx, int sy, double& r
 // path then grows it in full).  Later passes only re-test the neighbours that failed the ANGLE test before:
 // out-of-image, banned and own pixels stay so (bans only grow; a pixel that gets banned meanwhile invalidates
 // the evaluation at retire time anyway).
+// The angle test is grow_region_t<true>'s, on the squares: only valid for a tolerance <= pi/2, which speculate_super checks.
 // Returns the region size (T when large).  lst[] holds the accepted pixels (packed y<<16|x), pnd[0..npnd) the pixels
 // skipped because an earlier seed's parked accept covers them (npnd = -1: more than SG_PND of them).
 // The 32 lanes run their seeds as ONE instruction stream: every trip of the loop below, each running lane first opens its
@@ -1307,7 +1308,9 @@ __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned
         bool large = act;
         const int L0 = sh.nSeg;
         __threadfence_block();
-        if (T <= SG_CAP) {   // warp-uniform: all 32 lanes enter, the ones without a seed idle
+        // small_grow decides the angle on the squares, which is the literal test only for a tolerance <= pi/2 (grow_region's
+        // predicate); above that every live seed takes the warp path, like every seed when T > SG_CAP
+        if (T <= SG_CAP && c.kc->degThre <= c.kc->pi / 2.0) {   // warp-uniform: all 32 lanes enter, the ones without a seed idle
             num = small_grow(c, act, myp, T, lst, myChunk, pnd, npnd);
             large = act && num >= T;
         }

@@ -17,6 +17,7 @@
 //   * no error channel: failures abort with the library's message.
 #include <myLSD.h>
 
+#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 #include <vector>
@@ -40,6 +41,15 @@ namespace mylsd {
 
 structLSD myLineSegmentDetector(Mat MapGray, int oriMapCol, int oriMapRow, double sca, double sig, double angThre,
                                 double denThre, LSDB_PSEBIN_T pseBin) {
+#ifdef LSDB_ROS_FLAVOUR
+    // The snapshot bins with zoom = 1.0*pseBin/maxGrad on the double (as LSD/myLSD.cpp:179 does on the int): a fractional
+    // pseBin gives another seed order than any integer the library takes, so it is refused instead of truncated.
+    if (!(pseBin >= 1 && pseBin <= 1024 && pseBin == (double)(int)pseBin)) {
+        fprintf(stderr, "lsdb200: myLineSegmentDetector: pseBin %.17g is not an integer in [1,1024]; the library bins with an integer pseBin\n",
+                (double)pseBin);
+        abort();
+    }
+#endif
     lsdb_ctx* ctx = lsdb_host::context();
     const size_t npx = (size_t)oriMapCol * oriMapRow;
     std::vector<uint8_t> in(npx), remapped(npx), lineIm(npx);

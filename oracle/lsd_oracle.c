@@ -32,6 +32,11 @@ static int* lsdo_grow_size_log = 0;
 static int lsdo_grow_size_cap = 0, lsdo_grow_size_n = 0;
 void lsdo_set_grow_size_log(int* buf, int cap) { lsdo_grow_size_log = buf; lsdo_grow_size_cap = cap; lsdo_grow_size_n = 0; }
 int lsdo_grow_size_count(void) { return lsdo_grow_size_n; }
+/* optional debug tap: the tolerance of every Refiner re-grow (set by lsdo_set_regrow_tol_log) */
+static double* lsdo_regrow_tol_log = 0;
+static int lsdo_regrow_tol_cap = 0, lsdo_regrow_tol_n = 0;
+void lsdo_set_regrow_tol_log(double* buf, int cap) { lsdo_regrow_tol_log = buf; lsdo_regrow_tol_cap = cap; lsdo_regrow_tol_n = 0; }
+int lsdo_regrow_tol_count(void) { return lsdo_regrow_tol_n; }
 
 typedef struct {
     int W, H;
@@ -284,6 +289,7 @@ static int refiner(ctx_t* c, reg_t* reg, rec_t* rec, double denThre) {
     }
     double meanDif = difSum / (ptNum * 1.0);
     double degThre = 2.0 * sqrt((squSum - 2 * meanDif * difSum) / (ptNum * 1.0) + meanDif * meanDif);
+    if (lsdo_regrow_tol_log && lsdo_regrow_tol_n < lsdo_regrow_tol_cap) lsdo_regrow_tol_log[lsdo_regrow_tol_n++] = degThre;
     region_grower(c, oriX, oriY, cenDeg, degThre, reg);
     if (c->st) c->st->regrows++;
     if (reg->num < 2) return 0;

@@ -42,6 +42,13 @@ int lsdo_lsd(const uint8_t* map, int cols, int rows, double sca, double sig, dou
  * returns h */
 int lsdo_gauss_taps(double sca, double sig, double* out, int cap);
 
+/* debug taps of the next lsdo_lsd calls: the size of every region grown, and the tolerance of every Refiner
+ * re-grow (LSD/myLSD.cpp:857), up to cap entries; a NULL buffer turns the tap off */
+void lsdo_set_grow_size_log(int* buf, int cap);
+int lsdo_grow_size_count(void);
+void lsdo_set_regrow_tol_log(double* buf, int cap);
+int lsdo_regrow_tol_count(void);
+
 /* mylsd::createMapCache restated (LSD/myLSD.cpp:11-127) */
 void lsdo_map_cache(const uint8_t* map, int cols, int rows, double res, double* out);
 

@@ -95,6 +95,23 @@ def lsd(map_u8, want_maps=True, want_line_im=True, max_lines=65536, **kw):
     return out
 
 
+def lsd_regrow_tols(map_u8, cap=1 << 20, **kw):
+    """lsd() with the oracle's re-grow tap on: adds regrow_tols, the tolerance of every Refiner re-grow (:857) in call order"""
+    L = lib()
+    L.lsdo_set_regrow_tol_log.argtypes = [C.c_void_p, C.c_int]
+    L.lsdo_regrow_tol_count.restype = C.c_int
+    tols = np.zeros(cap)
+    L.lsdo_set_regrow_tol_log(_p(tols), cap)
+    try:
+        out = lsd(map_u8, **kw)
+        n = L.lsdo_regrow_tol_count()
+    finally:
+        L.lsdo_set_regrow_tol_log(None, 0)
+    assert n < cap, "re-grow tap full"
+    out["regrow_tols"] = tols[:n].copy()
+    return out
+
+
 def gauss_taps(sca=0.3, sig=0.6):
     buf = np.zeros(3 * 64)
     h = lib().lsdo_gauss_taps(sca, sig, _p(buf), len(buf))

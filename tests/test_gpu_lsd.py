@@ -1,5 +1,6 @@
 """Parity of the CUDA LSD path (through the C ABI) with the oracle and with the reference's golden outputs.
 Bit-exact: mag, deg (vs the oracle on the same arithmetic), seed order, used-map, labels, segment table, lineIm."""
+import contextlib
 import os
 
 import numpy as np
@@ -13,8 +14,9 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 NAMES = ["mapValue", "mapValue_aisle1", "mapValue_aisle2", "mapValue_aisle3", "mapValue_map1", "mapValue_map2"]
 
 
-def _compare_with_oracle(lsdb, b, i, m, got, check_planes=True):
-    o = oraclebind.lsd(m)
+def _compare_with_oracle(lsdb, b, i, m, got, check_planes=True, **params):
+    """map i of batch b against the oracle at the batch's LSD parameters `params` (default: the reference's constants)"""
+    o = oraclebind.lsd(m, **params)
     W = o["used"].shape[1]
     assert got["counts"][i] == o["n"]
     pl = b.planes(i)
@@ -28,6 +30,23 @@ def _compare_with_oracle(lsdb, b, i, m, got, check_planes=True):
     assert np.array_equal(got["rects"][i], o["rects"], equal_nan=True)      # rectangles and log-NFA, bit for bit
     assert np.array_equal(b.line_image(i), o["line_im"])
     return o
+
+
+@contextlib.contextmanager
+def lsdb_env(env):
+    """`env` set in os.environ for the block, the previous values back afterwards.  The library reads its switches when a
+    batch is created (team size, ban plane, stencil cut) and when it runs (LSDB_GROW_WIDE picks the grower's build at
+    launch), so the block covers both."""
+    old = {k: os.environ.get(k) for k in env}
+    os.environ.update(env)
+    try:
+        yield
+    finally:
+        for k, v in old.items():
+            if v is None:
+                os.environ.pop(k, None)
+            else:
+                os.environ[k] = v
 
 
 @pytest.fixture(scope="module")
@@ -234,17 +253,9 @@ def test_result_is_independent_of_team_shape(lsdb, ctx, gold, env):
     """The ordered-commit pipeline must give the sequential result whatever the speculation looks like: team size,
     run-ahead window, team-wide queue for large seeds, ban plane in shared memory or not."""
     maps = [gold["mapValue_aisle2/map"], synth.occupancy_grid(1500, 1100, seed=77), synth.occupancy_grid(900, 1300, seed=78, border_walls=True)]
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
+    with lsdb_env(env):
         b = lsdb.Batch(ctx, [(m.shape[1], m.shape[0]) for m in maps])
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-    b.upload(maps); b.run()
+        b.upload(maps); b.run()
     got = b.download(want_rects=True)
     for i, m in enumerate(maps):
         _compare_with_oracle(lsdb, b, i, m, got, check_planes=False)
@@ -262,17 +273,9 @@ def test_result_is_independent_of_the_stencil_cut(lsdb, ctx, gold, env):
     walls included."""
     maps = [gold["mapValue/map"], synth.occupancy_grid(1057, 771, seed=91), synth.occupancy_grid(400, 1300, seed=92, border_walls=True),
             synth.occupancy_grid(97, 45, seed=12), synth.occupancy_grid(2048, 2048, seed=93)]
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
+    with lsdb_env(env):
         b = lsdb.Batch(ctx, [(m.shape[1], m.shape[0]) for m in maps])
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-    b.upload(maps); b.run()
+        b.upload(maps); b.run()
     got = b.download(want_rects=True)
     assert b.launches() == (5 if env.get("LSDB_STENCIL") == "1" or env.get("LSDB_STENCIL_DEFER") == "0" else 6)
     for i, m in enumerate(maps):

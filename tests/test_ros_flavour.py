@@ -82,3 +82,34 @@ def test_ros_flavour_dropin(lsdb, ctx, gold):
                 assert np.array_equal(std, refbind.ref_map_cache(m, res))
             unreached = ctx.map_cache(m, res, zmax, unreached=7.0) == 7.0
             assert unreached.any() and np.array_equal(out, np.where(unreached, 2.0, std))
+
+
+@pytest.mark.gpu
+@pytest.mark.skipif(not os.path.exists(DROPIN_ROS), reason="oracle/_ref/libdropin_ros.so not built")
+@pytest.mark.parametrize("pse_bin", [512.0, 1.0])
+def test_ros_flavour_dropin_other_pse_bins(lsdb, gold, pse_bin):
+    """the snapshot takes pseBin as a double and bins with 1.0*pseBin/maxGrad: every integral value must give its segments"""
+    L, R = _bind(DROPIN_ROS), _bind(REF_ROS)
+    for name in NAMES:
+        m = gold[name + "/map"]
+        lines, im, mo = _ros_lsd(L, m, pse_bin=pse_bin)
+        rl, rim, rmo = _ros_lsd(R, m, pse_bin=pse_bin)
+        assert np.array_equal(lines, rl, equal_nan=True), name
+        assert np.array_equal(im, rim) and np.array_equal(mo, rmo), name
+
+
+@pytest.mark.gpu
+@pytest.mark.skipif(not os.path.exists(DROPIN_ROS), reason="oracle/_ref/libdropin_ros.so not built")
+@pytest.mark.parametrize("pse_bin", [512.5, 0.0, 1025.0, float("nan")])
+def test_ros_flavour_dropin_refuses_a_pse_bin_it_cannot_honour(pse_bin):
+    """a pseBin the library cannot take as it is (not an integer in [1,1024]) aborts with a message instead of being
+    truncated to another seed order; the wrapper has no error channel, so the call runs in a child process"""
+    import subprocess
+    import sys
+    code = ("import sys; sys.path.insert(0, %r); import numpy as np, test_ros_flavour as t\n"
+            "g = np.load(%r)\n"
+            "t._ros_lsd(t._bind(t.DROPIN_ROS), g['mapValue/map'], pse_bin=float('%s'))\n"
+            "print('returned')\n") % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tests", "golden", "bundled_maps.npz"), pse_bin)
+    p = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert p.returncode != 0 and "returned" not in p.stdout
+    assert "pseBin" in p.stderr and "not an integer in [1,1024]" in p.stderr
