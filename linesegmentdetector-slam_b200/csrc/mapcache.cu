@@ -25,10 +25,8 @@
 // go into groups under a cell budget that bounds the transient buffers (claims 8 B, flag 1 B, two frontiers of 3 x 4 B
 // per cell of the group); a map larger than the budget is a group of its own.  One propose / flag+reduce / scan / scatter
 // round per level (<= ~1.5 * cell_radius levels); the host reads back the size of the next level.
-#include "../../include/lsdb200.h"
 #include "lsdb_common.cuh"
 #include <math.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <vector>
 
@@ -320,24 +318,4 @@ done:
     for (int k = 0; k < 2; k++) cudaFree(fm[k]);
     cudaFree(tileSum); cudaFree(count);
     return e;
-}
-
-// one map from host memory: a group of one in a device copy of the map
-extern "C" int lsdb_map_cache_device(int device, void* streamV, const uint8_t* map, int cols, int rows, double res, double maxDist, double unreached,
-                                     double* out, char* err, int errLen) {
-    cudaStream_t s = (cudaStream_t)streamV;
-    const size_t n = (size_t)cols * rows;
-    uint8_t* mapD = 0;
-    double* cache = 0;
-    LsdbMcMap m = {0, 0, 0, cols, rows, cols, lsdb_mc_cell_radius(maxDist, res), res};
-    cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&mapD, n);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&cache, n * 8);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(mapD, map, n, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess) e = lsdb_map_caches_run(s, 1, &m, mapD, unreached, cache);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, cache, n * 8, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    cudaFree(mapD); cudaFree(cache);
-    if (e != cudaSuccess) { snprintf(err, errLen, "lsdb_map_cache: %s", cudaGetErrorString(e)); return LSDB_ERR_CUDA; }
-    return LSDB_OK;
 }
