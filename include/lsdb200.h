@@ -129,6 +129,44 @@ int lsdb_batch_map_stats(lsdb_batch* b, int i, lsdb_stats* out);
 /* number of kernel launches issued by the last lsdb_batch_run */
 int lsdb_batch_launches(const lsdb_batch* b);
 
+/* ---- LSD: device memory in, device memory out ---- */
+/* For grids that already live on the GPU (a torch tensor from a GPU mapper, a learned occupancy model) and for consumers that
+ * stay there.  Rules shared by the calls below:
+ *   - Asynchronous: they only enqueue work on the context stream (per-map cudaMemcpy2DAsync / cudaMemcpyAsync device to device
+ *     and kernels); they never synchronise the stream or wait on the host.  The caller orders the producers of its inputs
+ *     before the call and the consumers of its outputs after it against the context stream (lsdb_stream gives it), and keeps
+ *     its buffers alive until the stream has passed them.  lsdb_batch_sync / lsdb_batch_download work after them as always.
+ *   - Every non-NULL pointer argument must be device or managed memory of the context's device (cudaPointerGetAttributes);
+ *     host memory, pinned host memory and another GPU's memory are LSDB_ERR_ARG, found before anything is enqueued: the batch
+ *     and the context stay usable.
+ *   - Packed per-map buffers (line images, map caches): map i starts at element sum_{k<i} rows_k*cols_k, rows cols_i apart,
+ *     the layout of the batch's own mapCache plane. */
+/* the context's cudaStream_t */
+int lsdb_stream(const lsdb_ctx* ctx, void** stream);
+/* device -> device copy of the occupancy grids: dev_maps[i] = rows[i] rows of cols[i] u8, pitches[i] bytes apart (pitches NULL:
+ * cols[i]; any byte offset).  Replaces lsdb_batch_upload for the batch, as lsdb_batch_upload_scan_rasters does;
+ * lsdb_batch_map_caches reads the same planes afterwards.  LSDB_ERR_ARG: dev_maps or a map NULL, a pitch below cols, a map
+ * that is not memory of the context's device. */
+int lsdb_batch_upload_device(lsdb_batch* b, const uint8_t* const* dev_maps, const long long* pitches);
+/* The segment tables of the last lsdb_batch_run, built on the device (the epilogue of LSD/myLSD.cpp:282-368, the same body
+ * lsdb_batch_download runs on the host), packed map after map:
+ *   dev_counts[n_maps]      : segments of map i; 0 for a map whose run failed
+ *   dev_offsets[n_maps + 1] : exclusive prefix of the counts; map i's records are [offsets[i], offsets[i] + counts[i])
+ *   dev_status[n_maps]      : (nullable) 0, or LSDB_ERR_CAPACITY / LSDB_ERR_TIMEOUT as lsdb_batch_sync would report map i;
+ *                             LSDB_ERR_CAPACITY also for a map whose records would end past max_total
+ *   dev_lines / dev_rects   : (nullable) max_total records each, byte for byte what lsdb_batch_download writes for the map
+ * Counts and offsets are always complete, so a call with dev_lines == dev_rects == NULL is a sizing query on the device.  A map
+ * flagged in status gets none of its records written, and nothing is written at or past max_total; n_maps * max_lines_per_map
+ * always suffices.  LSDB_ERR_ARG: counts or offsets NULL, max_total < 0, before lsdb_batch_run. */
+int lsdb_batch_lines_device(lsdb_batch* b, int* dev_counts, int* dev_offsets, int* dev_status,
+                            lsdb_line* dev_lines, lsdb_rect* dev_rects, long long max_total);
+/* lineIm of every map rasterised on the device into one packed u8 buffer (sum of rows*cols bytes, zeroed first), equal to what
+ * lsdb_batch_line_images writes.  LSDB_ERR_ARG: dev_out NULL, before lsdb_batch_run. */
+int lsdb_batch_line_images_device(lsdb_batch* b, uint8_t* dev_out);
+/* the caches the last lsdb_batch_map_caches left, copied into one packed f64 buffer (sum of rows*cols doubles).
+ * LSDB_ERR_ARG: dev_out NULL, before lsdb_batch_map_caches. */
+int lsdb_batch_map_caches_device(lsdb_batch* b, double* dev_out);
+
 /* ---- LSD: one map tiled over several GPUs (the stages apart) ---- */
 /* For a single-map batch.  Every GPU uploads the whole source map and runs the stencil stage (LSD/myLSD.cpp:135-174,378-484) on
  * the tile rows [tile_row0, tile_row1) only (a tile row = 32 scaled rows); the Gaussian's halo rows (floor(y/0.3+0.5) +- 8,

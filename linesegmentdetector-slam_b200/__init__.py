@@ -86,6 +86,11 @@ def lib():
         L.lsdb_map_cache_fill.argtypes = [vp, vp, ci, ci, cd, cd, cd, vp]
         L.lsdb_batch_map_caches.argtypes = [vp, vp, cd, cd, vp]
         L.lsdb_fa_map_create_from_batch.argtypes = [vp, ci, C.POINTER(vp)]
+        L.lsdb_stream.argtypes = [vp, C.POINTER(vp)]
+        L.lsdb_batch_upload_device.argtypes = [vp, vp, vp]
+        L.lsdb_batch_lines_device.argtypes = [vp, vp, vp, vp, vp, vp, C.c_longlong]
+        L.lsdb_batch_line_images_device.argtypes = [vp, vp]
+        L.lsdb_batch_map_caches_device.argtypes = [vp, vp]
         L.lsdb_multi_create.argtypes = [C.POINTER(vp), vp, ci]
         L.lsdb_multi_destroy.argtypes = [vp]; L.lsdb_multi_destroy.restype = None
         L.lsdb_multi_last_error.argtypes = [vp]; L.lsdb_multi_last_error.restype = C.c_char_p
@@ -126,6 +131,7 @@ class Context:
 
     def __init__(self, device=0, stream=None):
         self.h = C.c_void_p()
+        self.device = int(device)
         rc = lib().lsdb_create(C.byref(self.h), int(device), C.c_void_p(stream) if stream else None)
         if rc:
             raise LsdbError(f"lsdb_create(device={device}) failed: {ERR_NAMES.get(rc, rc)} — an sm_100 (B200) GPU is "
@@ -172,6 +178,23 @@ def _ctx_map_cache(self, map_u8, res, max_dist=1.0, unreached=None):
 
 
 Context.map_cache = _ctx_map_cache
+
+
+def _ctx_stream(self):
+    """lsdb_stream: the context's cudaStream_t handle (int); the device-memory calls of Batch enqueue their work there."""
+    s = C.c_void_p()
+    self.check(lib().lsdb_stream(self.h, C.byref(s)), "lsdb_stream")
+    return s.value or 0
+
+
+def _ctx_torch_stream(self):
+    """the context's stream as a torch.cuda.ExternalStream"""
+    import torch
+    return torch.cuda.ExternalStream(self.stream, device=torch.device("cuda", self.device))
+
+
+Context.stream = property(_ctx_stream)
+Context.torch_stream = _ctx_torch_stream
 
 
 class MultiContext:
@@ -343,6 +366,97 @@ class Batch:
                                                             _p(rng), _p(ang), _p(boff), _p(info)), "lsdb_batch_upload_scan_rasters")
         return info
 
+    def upload_device(self, maps):
+        """lsdb_batch_upload_device: the grids from device memory, copied device to device on the context stream.  maps: 2-D
+        uint8 CUDA tensors (rows x cols; row-pitched views such as a column slice of a wider tensor work) or 2-D objects with a
+        __cuda_array_interface__ of u1 whose last stride is 1.  The context stream first waits for torch's current stream, so
+        grids produced there are ready (other producers must be ordered against Context.stream by the caller), and torch's
+        current stream then waits for the copies, so that whatever it does next with the grids' memory comes after them.  The
+        call returns without waiting for the copies."""
+        import torch
+        if len(maps) != self.n:
+            raise ValueError(f"{len(maps)} maps for a batch of {self.n}")
+        ptrs = (C.c_void_p * self.n)(); pitches = np.zeros(self.n, np.int64)
+        for i, m in enumerate(maps):
+            ptr, shape, pitch = _dev_grid(m)
+            if shape != (self.sizes[i][1], self.sizes[i][0]):
+                raise ValueError(f"map {i}: shape {shape}, batch expects {(self.sizes[i][1], self.sizes[i][0])}")
+            ptrs[i] = ptr; pitches[i] = pitch
+        ext = self.ctx.torch_stream()
+        cur = torch.cuda.current_stream(ext.device)
+        ext.wait_stream(cur)
+        self.ctx.check(lib().lsdb_batch_upload_device(self.h, C.cast(ptrs, C.c_void_p), _p(pitches)), "lsdb_batch_upload_device")
+        cur.wait_stream(ext)
+        self._keep_dev = list(maps)   # memory that torch does not own must outlive the copies
+
+    def _device_out(self, what, call):
+        """call(), which writes torch allocations of the current stream on the context stream, between two stream waits: the
+        context stream first waits for torch's current stream, where the outputs were allocated; torch's current stream then
+        waits for the context stream, so that its consumers see the results, and a later reuse of the outputs' memory (torch
+        reuses a freed block on the stream that allocated it) comes after the writes.  That wait stands in for record_stream,
+        which would tie the tensors to the context's stream: a tensor freed after Context.close() would then make torch record
+        an event on a destroyed stream.  Nothing is synchronised."""
+        import torch
+        ext = self.ctx.torch_stream()
+        cur = torch.cuda.current_stream(ext.device)
+        ext.wait_stream(cur)
+        self.ctx.check(call(), what)
+        cur.wait_stream(ext)
+
+    def lines_device(self, max_total=None, want_rects=False):
+        """lsdb_batch_lines_device: the segment tables of the last run, built on the device, as CUDA tensors: counts (n,) int32,
+        offsets (n+1,) int32, status (n,) int32 (0, or LSDB_ERR_CAPACITY = 3 / LSDB_ERR_TIMEOUT = 4), lines (max_total, 80) uint8
+        lsdb_line records (line_fields() views them) and with want_rects rects (max_total, 13) float64.  Map i's records are rows
+        offsets[i] .. offsets[i] + counts[i] - 1.  max_total defaults to n * max_lines, which always suffices.  Nothing is
+        synchronised: torch's current stream waits for the results."""
+        import torch
+        max_total = self.n * self.max_lines if max_total is None else int(max_total)
+        if max_total < 0:
+            raise ValueError("max_total must be >= 0")
+        dev = torch.device("cuda", self.ctx.device)
+        counts = torch.empty(self.n, dtype=torch.int32, device=dev)
+        offsets = torch.empty(self.n + 1, dtype=torch.int32, device=dev)
+        status = torch.empty(self.n, dtype=torch.int32, device=dev)
+        lines = torch.empty((max_total, LINE_DTYPE.itemsize), dtype=torch.uint8, device=dev)
+        rects = torch.empty((max_total, 13), dtype=torch.float64, device=dev) if want_rects else None
+        ptr = lambda t: (t.data_ptr() or None) if t is not None else None  # noqa: E731  (an empty tensor has no storage)
+        self._device_out("lsdb_batch_lines_device",
+                         lambda: lib().lsdb_batch_lines_device(self.h, ptr(counts), ptr(offsets), ptr(status), ptr(lines), ptr(rects), max_total))
+        out = dict(counts=counts, offsets=offsets, status=status, lines=lines)
+        if want_rects:
+            out["rects"] = rects
+        return out
+
+    def _packed(self, out, dtype, what):
+        """a packed per-map CUDA buffer (map i after the rows*cols elements of the maps before it) and its per-map views"""
+        import torch
+        total = sum(c * r for c, r in self.sizes)
+        if out is None:
+            out = torch.empty(total, dtype=dtype, device=torch.device("cuda", self.ctx.device))
+        elif not (isinstance(out, torch.Tensor) and out.is_cuda and out.dtype == dtype and out.is_contiguous() and out.numel() >= total):
+            raise ValueError(f"{what}: out must be a contiguous CUDA {dtype} tensor of at least {total} elements")
+        flat, views, o = out.view(-1), [], 0
+        for c, r in self.sizes:
+            views.append(flat[o:o + r * c].view(r, c))
+            o += r * c
+        return out, views
+
+    def line_images_device(self, out=None):
+        """lsdb_batch_line_images_device: lineIm of every map rasterised on the device into one packed uint8 CUDA tensor (`out`
+        or a new one).  Returns (packed tensor, [rows x cols view per map]); nothing is synchronised."""
+        import torch
+        out, views = self._packed(out, torch.uint8, "line_images_device")
+        self._device_out("lsdb_batch_line_images_device", lambda: lib().lsdb_batch_line_images_device(self.h, out.data_ptr()))
+        return out, views
+
+    def map_caches_device(self, out=None):
+        """lsdb_batch_map_caches_device: the caches the last map_caches() left, copied into one packed float64 CUDA tensor (`out`
+        or a new one).  Returns (packed tensor, [rows x cols view per map]); nothing is synchronised."""
+        import torch
+        out, views = self._packed(out, torch.float64, "map_caches_device")
+        self._device_out("lsdb_batch_map_caches_device", lambda: lib().lsdb_batch_map_caches_device(self.h, out.data_ptr()))
+        return out, views
+
     def run(self):
         self.ctx.check(lib().lsdb_batch_run(self.h), "lsdb_batch_run")
 
@@ -423,6 +537,34 @@ class Batch:
         if self.h:
             lib().lsdb_batch_destroy(self.h)
             self.h = C.c_void_p()
+
+
+def _dev_grid(m):
+    """(device pointer, (rows, cols), row pitch in bytes) of a 2-D uint8 CUDA tensor or __cuda_array_interface__ object whose
+    last stride is 1"""
+    import torch
+    if isinstance(m, torch.Tensor):
+        if not m.is_cuda or m.dtype != torch.uint8 or m.dim() != 2:
+            raise ValueError(f"a 2-D uint8 CUDA tensor is required, got {m.dtype} {tuple(m.shape)} on {m.device}")
+        shape, strides, ptr = tuple(m.shape), tuple(m.stride()), m.data_ptr()
+    else:
+        cai = getattr(m, "__cuda_array_interface__", None)
+        if cai is None or len(cai["shape"]) != 2 or cai["typestr"] not in ("|u1", "<u1", ">u1"):
+            raise ValueError("a 2-D uint8 CUDA tensor or __cuda_array_interface__ object is required")
+        shape = tuple(int(v) for v in cai["shape"])
+        strides = tuple(cai["strides"]) if cai.get("strides") else (shape[1], 1)
+        ptr = int(cai["data"][0])
+    rows, cols = shape
+    if cols > 1 and strides[1] != 1:
+        raise ValueError(f"the last stride must be 1, got {strides}")
+    return ptr, (rows, cols), (int(strides[0]) if rows > 1 else cols)
+
+
+def line_fields(lines):
+    """zero-copy views of an (N, 80) uint8 tensor of lsdb_line records: ((N, 9) float64 k, b, dx, dy, x1, y1, x2, y2, len;
+    (N,) int32 orient)"""
+    import torch
+    return lines.view(torch.float64)[:, :9], lines.view(torch.int32)[:, 18]
 
 
 def lines_to_array(lines):

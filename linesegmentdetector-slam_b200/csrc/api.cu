@@ -10,6 +10,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <initializer_list>
 #include <math.h>
 #include <string>
 #include <vector>
@@ -82,6 +83,9 @@ struct lsdb_batch {
     unsigned char* recBuf = nullptr; unsigned int* banBits = nullptr;
     uint8_t* lineImD = nullptr;   // lineIm planes of all maps (allocated on first use by lsdb_batch_line_images; geometry of src)
     double* mcCache = nullptr;    // mapCache planes of all maps, rows*cols f64 each, packed in batch order (allocated on first use by lsdb_batch_map_caches)
+    // the packed layout of per-map images and caches: map i at packOff[i] = sum of rows*cols of the maps before it (n + 1 entries)
+    std::vector<unsigned long long> packOff;
+    unsigned long long* packOffD = nullptr;
     // ordering stage: "mag != 0" bits, row bands, count tables
     unsigned int* nzBits = nullptr; int2* bandOf = nullptr; int2* bandsOfImg = nullptr; unsigned int* orderTabs = nullptr; int nBands = 0;
     // host (pinned)
@@ -186,7 +190,7 @@ extern "C" void lsdb_batch_destroy(lsdb_batch* b) {
     cudaFree(b->src); cudaFree(b->mag); cudaFree(b->deg); cudaFree(b->cosm); cudaFree(b->state); cudaFree(b->bins); cudaFree(b->cells);
     cudaFree(b->labels); cudaFree(b->rects); cudaFree(b->dyn); cudaFree(b->imgsD); cudaFree(b->tileImg); cudaFree(b->lists);
     cudaFree(b->imgCounter); cudaFree(b->kcD); cudaFree(b->gaussDbg); cudaFree(b->recBuf); cudaFree(b->banBits);
-    cudaFree(b->lineImD); cudaFree(b->mcCache); cudaFree(b->nzBits); cudaFree(b->bandOf); cudaFree(b->bandsOfImg); cudaFree(b->orderTabs);
+    cudaFree(b->lineImD); cudaFree(b->mcCache); cudaFree(b->packOffD); cudaFree(b->nzBits); cudaFree(b->bandOf); cudaFree(b->bandsOfImg); cudaFree(b->orderTabs);
     cudaFreeHost(b->dynH); cudaFreeHost(b->rectsH);
     for (int i = 0; i < 4; i++) cudaEventDestroy(b->ev[i]);
     if (b->ctx->cached == b) b->ctx->cached = 0;
@@ -264,6 +268,8 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
         if (im.n > maxN) maxN = im.n;
     }
     b->nTiles = tile0; b->totalN = nOff; b->totalSrc = srcOff; b->totalBan = banOff;
+    b->packOff.assign((size_t)n + 1, 0);
+    for (int i = 0; i < n; i++) b->packOff[i + 1] = b->packOff[i] + (unsigned long long)cols[i] * rows[i];
     b->listCap = maxN + 2 < (1 << 16) ? ((maxN + 2 + 1) & ~1) : (1 << 16);  // even: the arena behind it holds doubles
     if (b->listCap < 32 * LSDB_SUPER) b->listCap = 32 * LSDB_SUPER;          // the scratch behind it also holds a super-chunk's seed queue
     {   // team size: spread the device's warp slots over the maps of the batch (16 warps for a lone map,
@@ -340,6 +346,7 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
     }
     AL(b->bandOf, bandOfH.size() * sizeof(int2)); AL(b->bandsOfImg, (size_t)n * sizeof(int2));
     AL(b->orderTabs, (size_t)b->nBands * lsdb_order_tab_words_per_band() * 4);
+    AL(b->packOffD, ((size_t)n + 1) * sizeof(unsigned long long));
 #undef AL
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->bandOf, bandOfH.data(), bandOfH.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->bandsOfImg, bandsOfImgH.data(), (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream);
@@ -350,6 +357,7 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->imgsD, b->imgs.data(), (size_t)n * sizeof(LsdbImg), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->tileImg, tileImgH.data(), tileImgH.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(b->kcD, &b->kc, sizeof(LsdbLsdConst), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(b->packOffD, b->packOff.data(), ((size_t)n + 1) * sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) {
         lsdb_batch_destroy(b);
@@ -476,21 +484,10 @@ extern "C" int lsdb_batch_sync(lsdb_batch* b) {
     return fetch_dyn(b);
 }
 
-// epilogue of one segment, LSD/myLSD.cpp:282-368 (host; identical operation order to the reference)
+// epilogue of one segment, LSD/myLSD.cpp:282-368: the body lsdb_launch_seg_table runs on the device (lsdb_common.cuh)
 static void line_from_rect(const LsdbRect& R, double pi, lsdb_line* L) {
-    const double x1 = R.v[0], y1 = R.v[1], x2 = R.v[2], y2 = R.v[3];
-    const double k = (y2 - y1) / (x2 - x1);
-    double ang = lsdm_atan(k) * 180.0 / pi;  // atand
-    int orient = 1;
-    if (ang < 0) { ang += 180; orient = -1; }
-    L->k = k;
-    L->b = (y1 + y2) / 2.0 - k * (x1 + x2) / 2.0;
-    L->dx = lsdm_cos(ang / 180.0 * pi);      // cosd
-    L->dy = lsdm_sin(ang / 180.0 * pi);      // sind
-    L->x1 = x1; L->y1 = y1; L->x2 = x2; L->y2 = y2;
-    const double ddy = y2 - y1, ddx = x2 - x1;
-    L->len = sqrt(ddy * ddy + ddx * ddx);
-    L->orient = orient; L->_pad = 0;
+    static_assert(sizeof(lsdb_line) == sizeof(LsdbFaLine), "layout");
+    lsdb_line_from_rect(R, pi, (LsdbFaLine*)L);
 }
 
 static void raster_line(const LsdbRect& R, int oriMapCol, int oriMapRow, uint8_t* lineIm) {  // :296-355
@@ -560,7 +557,7 @@ extern "C" int lsdb_batch_line_images(lsdb_batch* b, uint8_t* const* lineIms) {
     CK(ctx, cudaSetDevice(ctx->device));
     if (!b->lineImD) CK(ctx, cudaMalloc((void**)&b->lineImD, b->totalSrc + 64));
     CK(ctx, cudaMemsetAsync(b->lineImD, 0, b->totalSrc + 64, s));
-    lsdb_launch_line_images(s, b->n, b->maxSeg, b->imgsD, b->dyn, b->rects, b->lineImD);
+    lsdb_launch_line_images(s, b->n, b->maxSeg, b->imgsD, b->dyn, b->rects, b->lineImD, nullptr);
     CK(ctx, cudaGetLastError());
     for (int i = 0; i < b->n; i++) {
         if (!lineIms[i]) continue;
@@ -685,11 +682,7 @@ extern "C" int lsdb_map_cache(lsdb_ctx* ctx, const uint8_t* map, int cols, int r
 }
 
 // element offset of map i in the batch's mapCache plane (the maps' rows*cols cells packed in batch order)
-static size_t cache_off(const lsdb_batch* b, int i) {
-    size_t off = 0;
-    for (int k = 0; k < i; k++) off += (size_t)b->imgs[k].cols * b->imgs[k].rows;
-    return off;
-}
+static size_t cache_off(const lsdb_batch* b, int i) { return (size_t)b->packOff[i]; }
 
 extern "C" int lsdb_batch_map_caches(lsdb_batch* b, const double* res, double maxDist, double unreached, double* const* out) {
     if (!b) return LSDB_ERR_ARG;
@@ -717,6 +710,100 @@ extern "C" int lsdb_batch_map_caches(lsdb_batch* b, const double* res, double ma
     for (int i = 0; i < b->n; i++)
         if (out[i]) CK(ctx, cudaMemcpyAsync(out[i], b->mcCache + maps[i].cacheOff, (size_t)b->imgs[i].cols * b->imgs[i].rows * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return LSDB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ device-memory in / out
+// Every call below only enqueues work on the context stream: no synchronise, no host wait.  The caller orders the producers of
+// its inputs and the consumers of its outputs against that stream (lsdb_stream).  Pointers are checked before anything is
+// enqueued, so a refused call leaves the batch and the context as they were.
+
+extern "C" int lsdb_stream(const lsdb_ctx* ctx, void** stream) {
+    if (!ctx || !stream) return LSDB_ERR_ARG;
+    *stream = (void*)ctx->stream;
+    return LSDB_OK;
+}
+
+// device or managed memory of the context's device (not host, pinned host or another GPU's memory)
+static bool on_ctx_device(const lsdb_ctx* ctx, const void* p) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == ctx->device;
+}
+
+// the nullable pointer arguments of entry point fn: each one given must be memory of the context's device
+static int check_dev_ptrs(lsdb_ctx* ctx, const char* fn, std::initializer_list<const void*> ptrs) {
+    long long k = 0;
+    for (const void* p : ptrs) {
+        if (p && !on_ctx_device(ctx, p)) return fail(ctx, LSDB_ERR_ARG, "%s: pointer argument %lld is not device memory of the context's device", fn, k);
+        k++;
+    }
+    return LSDB_OK;
+}
+
+extern "C" int lsdb_batch_upload_device(lsdb_batch* b, const uint8_t* const* maps, const long long* pitches) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!maps) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_upload_device: maps must be given%s");
+    CK(ctx, cudaSetDevice(ctx->device));
+    for (int i = 0; i < b->n; i++) {
+        const LsdbImg& im = b->imgs[i];
+        const long long pitch = pitches ? pitches[i] : im.cols;
+        if (!maps[i]) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_upload_device: map %s%lld is NULL", "", i);
+        if (pitch < im.cols) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_upload_device: the pitch of map %s%lld is below its cols", "", i);
+        const uint8_t* last = maps[i] + pitch * (im.rows - 1) + (im.cols - 1);
+        if (!on_ctx_device(ctx, maps[i]) || !on_ctx_device(ctx, last))
+            return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_upload_device: map %s%lld is not device memory of the context's device", "", i);
+    }
+    for (int i = 0; i < b->n; i++) {
+        const LsdbImg& im = b->imgs[i];
+        CK(ctx, cudaMemcpy2DAsync(b->src + im.srcOff, im.srcPitch, maps[i], pitches ? (size_t)pitches[i] : (size_t)im.cols, im.cols, im.rows,
+                                  cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    return LSDB_OK;
+}
+
+extern "C" int lsdb_batch_lines_device(lsdb_batch* b, int* counts, int* offsets, int* status, lsdb_line* lines, lsdb_rect* rects,
+                                       long long maxTotal) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!counts || !offsets || maxTotal < 0) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_lines_device: counts and offsets must be given, max_total >= 0%s");
+    if (!b->ran) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_lines_device before lsdb_batch_run%s");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int rc = check_dev_ptrs(ctx, "lsdb_batch_lines_device", {counts, offsets, status, lines, rects});
+    if (rc) return rc;
+    static_assert(sizeof(lsdb_rect) == sizeof(LsdbRect), "layout");
+    // offsets are int: their total is at most n * max_lines_per_map records, whose rectangles the batch holds on the device
+    lsdb_launch_seg_table(ctx->stream, b->n, b->maxSeg, b->dyn, b->rects, b->kc.pi, maxTotal, counts, offsets, status, (LsdbFaLine*)lines,
+                          (double*)rects);
+    CK(ctx, cudaGetLastError());
+    return LSDB_OK;
+}
+
+extern "C" int lsdb_batch_line_images_device(lsdb_batch* b, uint8_t* out) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!out) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_line_images_device: out must be given%s");
+    if (!b->ran) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_line_images_device before lsdb_batch_run%s");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int rc = check_dev_ptrs(ctx, "lsdb_batch_line_images_device", {out});
+    if (rc) return rc;
+    CK(ctx, cudaMemsetAsync(out, 0, b->packOff[b->n], ctx->stream));
+    lsdb_launch_line_images(ctx->stream, b->n, b->maxSeg, b->imgsD, b->dyn, b->rects, out, b->packOffD);
+    CK(ctx, cudaGetLastError());
+    return LSDB_OK;
+}
+
+extern "C" int lsdb_batch_map_caches_device(lsdb_batch* b, double* out) {
+    if (!b) return LSDB_ERR_ARG;
+    lsdb_ctx* ctx = b->ctx;
+    if (!out) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_map_caches_device: out must be given%s");
+    if (!b->mcReady) return fail(ctx, LSDB_ERR_ARG, "lsdb_batch_map_caches_device before lsdb_batch_map_caches%s");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int rc = check_dev_ptrs(ctx, "lsdb_batch_map_caches_device", {out});
+    if (rc) return rc;
+    // the cache plane is already packed the way the caller's buffer is: one copy
+    CK(ctx, cudaMemcpyAsync(out, b->mcCache, b->packOff[b->n] * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     return LSDB_OK;
 }
 

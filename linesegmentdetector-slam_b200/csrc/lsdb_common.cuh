@@ -98,8 +98,10 @@ void lsdb_launch_order(cudaStream_t s, int nImgs, int nBands, const LsdbImg* img
                        const double* mag, const unsigned int* nzBits, const int2* bandOf, const int2* bandsOfImg, unsigned int* tabs,
                        unsigned short* bins, unsigned int* cells);
 size_t lsdb_order_tab_words_per_band(void);
+// lineIm of every map (lineim.cu) into `plane`: at each map's srcOff with srcPitch rows (packOff == NULL) or at packOff[i] with
+// rows of cols bytes (a packed caller buffer); the plane must be zeroed first
 void lsdb_launch_line_images(cudaStream_t s, int nImgs, int maxSeg, const LsdbImg* imgs, const LsdbImgDyn* dyn, const LsdbRect* rects,
-                             uint8_t* plane);
+                             uint8_t* plane, const unsigned long long* packOff);
 void lsdb_launch_grow(cudaStream_t s, int nImgs, int nCtas, int warpsPerCta, const LsdbImg* imgs, LsdbImgDyn* dyn,
                       const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm, const double* sinm,
                       unsigned int* state, const unsigned int* cells, int* labels, LsdbRect* rects, int maxSeg,
@@ -115,6 +117,34 @@ int lsdb_grow_max_bitmap_words(int device);
 struct LsdbFaTask { int frame, iScan, iMap, pad; };
 struct LsdbFaHyp { int frame, iScan, iMap, iPair; double x, y, ang, score; };  // == lsdb_hypothesis
 struct LsdbFaLine { double k, b, dx, dy, x1, y1, x2, y2, len; int orient, pad; };  // == lsdb_line
+
+// The segment-table epilogue of one accepted rectangle, LSD/myLSD.cpp:282-295,356-368, in the reference's operation order.
+// One body for the host (lsdb_batch_download) and the device (lsdb_launch_seg_table): lsdm_atan / lsdm_cos / lsdm_sin give
+// the same bits in both builds, and sqrt and / are IEEE on both sides.
+LSDM_FN void lsdb_line_from_rect(const LsdbRect& R, double pi, LsdbFaLine* L) {
+    const double x1 = R.v[0], y1 = R.v[1], x2 = R.v[2], y2 = R.v[3];
+    const double k = (y2 - y1) / (x2 - x1);
+    double ang = lsdm_atan(k) * 180.0 / pi;  // atand
+    int orient = 1;
+    if (ang < 0) { ang += 180; orient = -1; }
+    L->k = k;
+    L->b = (y1 + y2) / 2.0 - k * (x1 + x2) / 2.0;
+    L->dx = lsdm_cos(ang / 180.0 * pi);      // cosd
+    L->dy = lsdm_sin(ang / 180.0 * pi);      // sind
+    L->x1 = x1; L->y1 = y1; L->x2 = x2; L->y2 = y2;
+    const double ddy = y2 - y1, ddx = x2 - x1;
+    L->len = sqrt(ddy * ddy + ddx * ddx);
+    L->orient = orient; L->pad = 0;
+}
+
+// The segment tables of a batch on the device (segtab.cu), two launches:
+//   one CTA reads every map's nSeg / err and writes counts[n] (0 for a map with err != 0: nSeg keeps counting past maxSeg when
+//   the grower aborts), offsets[n+1] (exclusive prefix of counts) and, when status != NULL, status[n] (0, LSDB_ERR_CAPACITY or
+//   LSDB_ERR_TIMEOUT as lsdb_batch_sync reports the map; LSDB_ERR_CAPACITY too when offsets[i] + counts[i] > maxTotal);
+//   a grid-stride kernel over (map, slot) writes the records of every map that fits into lines[offsets[i] + j] and / or
+//   rects[offsets[i] + j] (13 doubles each); nothing at or past maxTotal is written.
+void lsdb_launch_seg_table(cudaStream_t s, int nImgs, int maxSeg, const LsdbImgDyn* dyn, const LsdbRect* rects, double pi,
+                           long long maxTotal, int* counts, int* offsets, int* status, LsdbFaLine* lines, double* rectsOut);
 void lsdb_launch_fa(cudaStream_t s, int nTasks, const LsdbFaTask* tasks, const LsdbFaLine* scanLines, const int* scanLineOff,
                     const double* pts, const int* ptOff, const double* lidarPose, const double* lastPose,
                     const LsdbFaLine* mapLines, const double* mapCache, int cols, int rows, double pi, LsdbFaHyp* out, void* poseBuf);
