@@ -37,6 +37,7 @@
 // (lane-parallel operands, serial adds); counts and min/max are order-free and reduced in parallel.
 // The stage is latency-bound (dependent gathers, serial accept chains), not bandwidth-bound.
 #include "lsdb_common.cuh"
+#include "nfa.cuh"
 #include "../../include/lsdb200.h"
 #include <stdlib.h>
 
@@ -150,10 +151,6 @@ __device__ __forceinline__ void bbox_add(const WarpCtx& c, BBox& b, int x, int y
 __device__ __noinline__ double d_sin(double x) { return lsdm_sin(x); }
 __device__ __noinline__ double d_cos(double x) { return lsdm_cos(x); }
 __device__ __noinline__ double d_atan2(double y, double x) { return lsdm_atan2(y, x); }
-__device__ __noinline__ double d_log(double x) { return lsdm_log(x); }
-__device__ __noinline__ double d_log10(double x) { return lsdm_log10(x); }
-__device__ __noinline__ double d_exp(double x) { return lsdm_exp(x); }
-__device__ __noinline__ double d_pow(double x, double y) { return lsdm_pow(x, y); }
 
 __device__ __forceinline__ unsigned int pack_xy(int x, int y) { return ((unsigned int)y << 16) | (unsigned int)x; }
 __device__ __forceinline__ int px_of(unsigned int v) { return (int)(v & 0xffffu); }
@@ -715,36 +712,6 @@ __device__ __forceinline__ double dist_xy(int ox, int oy, double x, double y) {
     return sqrt(a * a + b * b);
 }
 
-// ------------------------------------------------------------------ LogGammaCalculator (:882-924)
-__device__ double log_gamma_calc(int x) {
-    double val;
-    if (x > 15) {
-        const double xd = x;
-        val = 0.918938533204673 + (xd - 0.5) * d_log(xd) - xd +
-              0.5 * xd * d_log(xd * lsdm_sinh(1.0 / xd) + 1.0 / (810 * d_pow(xd, 6)));
-    } else {
-        const double q[7] = {75122.6331530, 80916.6278952, 36308.2951477, 8687.24529705,
-                             1168.92649479, 83.8676043424, 2.50662827511};
-        double a = (x + 0.5) * d_log(x + 5.5) - (x + 5.5);
-        double b = 0;
-        for (int i = 0; i < 7; i++) {
-            a -= d_log(x + i);
-            b += q[i] * d_pow(x, i);
-        }
-        val = a + d_log(b);
-    }
-    return val;
-}
-__device__ __forceinline__ double log_gamma(const WarpCtx& c, int x) {
-    if (x >= 0 && x < c.lgammaN) return c.lgammaTab[x];
-    return log_gamma_calc(x);
-}
-
-__global__ void lsdb_lgamma_table_kernel(double* tab, int n) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) tab[i] = i >= 1 ? log_gamma_calc(i) : 0.0;
-}
-
 // ------------------------------------------------------------------ RectangleNFACalculator (:926-1059)
 __device__ __noinline__ double rect_nfa_impl(WarpCtx& c, const Rect& rec, double logNT) {
     const int xLim = c.W, yLim = c.H;
@@ -803,53 +770,7 @@ __device__ __noinline__ double rect_nfa_impl(WarpCtx& c, const Rect& rec, double
     }
     STAT(c, ST_NFACALLS, 1); STAT(c, ST_NFAPX, allPixNum);
 
-    if (allPixNum == 0 || aliPixNum == 0) return -logNT;
-    // log(p), log(1-p), log10(p): p only takes the values aliPro/2^k (:1085,:1149) — host-made table
-    double logP, log1mP, log10P;
-    {
-        int k = -1;
-#pragma unroll
-        for (int i = 0; i < LSDB_NP; i++) if (rec.p == c.kc->pTab[i]) k = i;
-        if (k >= 0) { logP = c.kc->logP[k]; log1mP = c.kc->log1mP[k]; log10P = c.kc->log10P[k]; }
-        else { logP = d_log(rec.p); log1mP = d_log(1 - rec.p); log10P = d_log10(rec.p); }
-    }
-    if (allPixNum == aliPixNum) return -logNT - allPixNum * log10P;
-    const double proTerm = rec.p / (1.0 - rec.p);
-    const double log1Coef = log_gamma(c, allPixNum + 1) - log_gamma(c, aliPixNum + 1) - log_gamma(c, allPixNum - aliPixNum + 1);
-    const double log1Term = log1Coef + aliPixNum * logP + (allPixNum - aliPixNum) * log1mP;
-    double term = d_exp(log1Term);
-    const double eps = 2.2204e-16;
-    if (fabs(term) < 100 * eps) {
-        if (aliPixNum > allPixNum * rec.p) return -d_log10(term) - logNT;
-        return -logNT;
-    }
-    double binTail = term;
-    const double tole = 0.1;
-    for (int i = aliPixNum + 1; i <= allPixNum; i++) {
-        const double binTerm = (allPixNum - i + 1) / (i * 1.0);
-        const double multTerm = binTerm * proTerm;
-        term *= multTerm;
-        binTail += term;
-        if (binTerm < 1) {
-            // break test of :1052-1054.  It is a comparison, so it is first decided with the hardware
-            // pow/log10 (<= 2 ulp) and a 1e-9 safety margin; only a knife-edge falls back to the
-            // correctly-rounded pow/log10 the reference's arithmetic is defined by.
-            const double nn = (double)(allPixNum - i + 1);
-            const double X = (1 - pow(multTerm, nn)) / (1.0 - multTerm);
-            const double errA = term * (X - 1);
-            const double l10 = log10(binTail);
-            const double rhsA = tole * fabs(-l10 - logNT) * binTail;
-            const double scale = fabs(term) * (fabs(X) + 1) + tole * fabs(binTail) * (fabs(l10) + fabs(logNT));
-            bool brk;
-            if (fabs(errA - rhsA) > 1e-9 * scale) brk = errA < rhsA;
-            else {
-                const double err = term * ((1 - d_pow(multTerm, nn)) / (1.0 - multTerm) - 1);
-                brk = err < tole * fabs(-d_log10(binTail) - logNT) * binTail;
-            }
-            if (brk) break;
-        }
-    }
-    return -d_log10(binTail) - logNT;
+    return nfa_tail(allPixNum, aliPixNum, rec.p, logNT, c.kc, c.lgammaTab, c.lgammaN);
 }
 
 __device__ double rect_nfa(WarpCtx& c, const Rect& rec, double logNT) {

@@ -37,6 +37,11 @@ static double* lsdo_regrow_tol_log = 0;
 static int lsdo_regrow_tol_cap = 0, lsdo_regrow_tol_n = 0;
 void lsdo_set_regrow_tol_log(double* buf, int cap) { lsdo_regrow_tol_log = buf; lsdo_regrow_tol_cap = cap; lsdo_regrow_tol_n = 0; }
 int lsdo_regrow_tol_count(void) { return lsdo_regrow_tol_n; }
+/* optional debug tap: every RectangleNFACalculator call as (allPix, aliPix, p, logNT, result) (set by lsdo_set_nfa_log) */
+static double* lsdo_nfa_log = 0;
+static int lsdo_nfa_cap = 0, lsdo_nfa_n = 0;
+void lsdo_set_nfa_log(double* buf, int cap) { lsdo_nfa_log = buf; lsdo_nfa_cap = cap; lsdo_nfa_n = 0; }
+int lsdo_nfa_log_count(void) { return lsdo_nfa_n; }
 
 typedef struct {
     int W, H;
@@ -300,7 +305,7 @@ static int refiner(ctx_t* c, reg_t* reg, rec_t* rec, double denThre) {
 }
 
 /* LogGammaCalculator :882-924 */
-static double log_gamma(int x) {
+double lsdo_log_gamma(int x) {
     double val;
     if (x > 15) {
         double xd = x;
@@ -318,6 +323,71 @@ static double log_gamma(int x) {
         val = a + lsdm_log(b);
     }
     return val;
+}
+
+/* RectangleNFACalculator :1006-1059, the part after the pixel count; probe (test instrumentation, may be NULL) watches the
+ * break tests without touching the arithmetic */
+typedef struct { double few, near, margin; int* out; } nfa_probe_t;
+
+static double nfa_tail(int allPixNum, int aliPixNum, double p, double logNT, int* exit_idx, const nfa_probe_t* pr) {
+    int ex_;
+    int* ex = exit_idx ? exit_idx : &ex_;
+    if (allPixNum == 0 || aliPixNum == 0) { *ex = LSDO_NFA_EXIT_EMPTY; return -logNT; }
+    if (allPixNum == aliPixNum) { *ex = LSDO_NFA_EXIT_ALL_ALIGNED; return -logNT - allPixNum * lsdm_log10(p); }
+    double proTerm = p / (1.0 - p);
+    double log1Coef = lsdo_log_gamma(allPixNum + 1) - lsdo_log_gamma(aliPixNum + 1) - lsdo_log_gamma(allPixNum - aliPixNum + 1);
+    double log1Term = log1Coef + aliPixNum * lsdm_log(p) + (allPixNum - aliPixNum) * lsdm_log(1 - p);
+    double term = lsdm_exp(log1Term);
+    double eps = 2.2204e-16;
+    if (fabs(term) < 100 * eps) {
+        if (aliPixNum > allPixNum * p) { *ex = LSDO_NFA_EXIT_TINY_TERM_HIGH; return -lsdm_log10(term) - logNT; }
+        *ex = LSDO_NFA_EXIT_TINY_TERM_LOW;
+        return -logNT;
+    }
+    double binTail = term, tole = 0.1;
+    int i = aliPixNum + 1;
+    for (; i <= allPixNum; i++) {
+        double binTerm = (allPixNum - i + 1) / (i * 1.0);
+        double multTerm = binTerm * proTerm;
+        term *= multTerm;
+        binTail += term;
+        if (binTerm < 1) {
+            double pw = lsdm_pow(multTerm, allPixNum - i + 1);
+            double err = term * ((1 - pw) / (1.0 - multTerm) - 1);
+            double l10 = lsdm_log10(binTail);
+            double rhs = tole * fabs(-l10 - logNT) * binTail;
+            if (pr) {
+                /* out: break tests, m == 1, 0 < |1 - m| <= few, tests the device decides with the correctly rounded path when
+                 * its hardware pow / log10 are correctly rounded too (|1 - m| < near, or |err - rhs| within margin * scale),
+                 * and those the margin without the |m^n| / |1 - m| term of scale would have sent there */
+                double gap = fabs(1.0 - multTerm);
+                double X = (1 - pw) / (1.0 - multTerm);
+                double scale = fabs(term) * (fabs(X) + 1 + fabs(pw) / gap) + tole * fabs(binTail) * (fabs(l10) + fabs(logNT));
+                double scaleOld = fabs(term) * (fabs(X) + 1) + tole * fabs(binTail) * (fabs(l10) + fabs(logNT));
+                pr->out[0]++;
+                if (multTerm == 1.0) pr->out[1]++;
+                else if (gap <= pr->few) pr->out[2]++;
+                if (!(gap >= pr->near && fabs(err - rhs) > pr->margin * scale)) pr->out[3]++;
+                if (!(fabs(err - rhs) > pr->margin * scaleOld)) pr->out[4]++;
+            }
+            if (err < rhs) break;
+        }
+    }
+    *ex = i;
+    return -lsdm_log10(binTail) - logNT;
+}
+
+double lsdo_nfa_tail(int allPix, int aliPix, double p, double logNT, int* exit_idx) {
+    return nfa_tail(allPix, aliPix, p, logNT, exit_idx, 0);
+}
+
+void lsdo_nfa_tail_many(int n, const int* allPix, const int* aliPix, const double* p, const double* logNT, double few, double near,
+                        double margin, double* out, int* exit_idx, int* probe) {
+    for (int k = 0; k < n; k++) {
+        nfa_probe_t pr = {few, near, margin, probe ? probe + 5 * (size_t)k : 0};
+        if (pr.out) pr.out[0] = pr.out[1] = pr.out[2] = pr.out[3] = pr.out[4] = 0;
+        out[k] = nfa_tail(allPix[k], aliPix[k], p[k], logNT[k], exit_idx ? exit_idx + k : 0, pr.out ? &pr : 0);
+    }
 }
 
 /* RectangleNFACalculator :926-1059 */
@@ -386,29 +456,12 @@ static double rect_nfa(ctx_t* c, const rec_t* rec, double logNT) {
     }
     if (c->st) { c->st->nfa_calls++; c->st->nfa_px += allPixNum; }
 
-    if (allPixNum == 0 || aliPixNum == 0) return -logNT;
-    if (allPixNum == aliPixNum) return -logNT - allPixNum * lsdm_log10(rec->p);
-    double proTerm = rec->p / (1.0 - rec->p);
-    double log1Coef = log_gamma(allPixNum + 1) - log_gamma(aliPixNum + 1) - log_gamma(allPixNum - aliPixNum + 1);
-    double log1Term = log1Coef + aliPixNum * lsdm_log(rec->p) + (allPixNum - aliPixNum) * lsdm_log(1 - rec->p);
-    double term = lsdm_exp(log1Term);
-    double eps = 2.2204e-16;
-    if (fabs(term) < 100 * eps) {
-        if (aliPixNum > allPixNum * rec->p) return -lsdm_log10(term) - logNT;
-        return -logNT;
+    double v = lsdo_nfa_tail(allPixNum, aliPixNum, rec->p, logNT, 0);
+    if (lsdo_nfa_log && lsdo_nfa_n < lsdo_nfa_cap) {
+        double* r = lsdo_nfa_log + 5 * (size_t)lsdo_nfa_n++;
+        r[0] = allPixNum; r[1] = aliPixNum; r[2] = rec->p; r[3] = logNT; r[4] = v;
     }
-    double binTail = term, tole = 0.1;
-    for (int i = aliPixNum + 1; i <= allPixNum; i++) {
-        double binTerm = (allPixNum - i + 1) / (i * 1.0);
-        double multTerm = binTerm * proTerm;
-        term *= multTerm;
-        binTail += term;
-        if (binTerm < 1) {
-            double err = term * ((1 - lsdm_pow(multTerm, allPixNum - i + 1)) / (1.0 - multTerm) - 1);
-            if (err < tole * fabs(-lsdm_log10(binTail) - logNT) * binTail) break;
-        }
-    }
-    return -lsdm_log10(binTail) - logNT;
+    return v;
 }
 
 /* RectangleImprover :1061-1158 */

@@ -48,6 +48,27 @@ void lsdo_set_grow_size_log(int* buf, int cap);
 int lsdo_grow_size_count(void);
 void lsdo_set_regrow_tol_log(double* buf, int cap);
 int lsdo_regrow_tol_count(void);
+/* debug tap of the next lsdo_lsd calls: every RectangleNFACalculator call as 5 doubles (allPix, aliPix, p, logNT, result),
+ * up to cap records; a NULL buffer turns the tap off */
+void lsdo_set_nfa_log(double* buf, int cap);
+int lsdo_nfa_log_count(void);
+
+/* RectangleNFACalculator after the pixel count (LSD/myLSD.cpp:1006-1059): -log10 NFA of allPix pixels, aliPix of them
+ * aligned at precision p.  *exit_idx (may be NULL) = the index i of the binomial-tail loop it broke at, allPix + 1 when
+ * the loop ran to the end, or one of the early returns below (csrc/nfa.cuh reports the same codes). */
+enum { LSDO_NFA_EXIT_EMPTY = -1,           /* allPix == 0 or aliPix == 0 */
+       LSDO_NFA_EXIT_ALL_ALIGNED = -2,     /* allPix == aliPix */
+       LSDO_NFA_EXIT_TINY_TERM_HIGH = -3,  /* first term below 100 eps, aliPix > allPix * p */
+       LSDO_NFA_EXIT_TINY_TERM_LOW = -4 }; /* first term below 100 eps, otherwise */
+double lsdo_nfa_tail(int allPix, int aliPix, double p, double logNT, int* exit_idx);
+/* n tails at once; probe (may be NULL) = [n][5] counts of the break tests each tail ran: all of them, m == 1,
+ * 0 < |1 - m| <= few, those the device leaves to its correctly rounded pow / log10 when its hardware ones round
+ * correctly (|1 - m| < near, or |err - rhs| <= margin * scale, csrc/nfa.cuh), and those a margin without scale's
+ * |m^n| / |1 - m| term would leave there */
+void lsdo_nfa_tail_many(int n, const int* allPix, const int* aliPix, const double* p, const double* logNT, double few, double near,
+                        double margin, double* out, int* exit_idx, int* probe);
+/* LogGammaCalculator (LSD/myLSD.cpp:882-924) */
+double lsdo_log_gamma(int x);
 
 /* mylsd::createMapCache restated (LSD/myLSD.cpp:11-127) */
 void lsdo_map_cache(const uint8_t* map, int cols, int rows, double res, double* out);

@@ -112,6 +112,46 @@ def lsd_regrow_tols(map_u8, cap=1 << 20, **kw):
     return out
 
 
+def lsd_nfa_calls(map_u8, cap=1 << 20, **kw):
+    """lsd() with the oracle's NFA tap on: adds nfa_calls, one row (allPix, aliPix, p, logNT, result) per RectangleNFACalculator
+    call in call order"""
+    L = lib()
+    L.lsdo_set_nfa_log.argtypes = [C.c_void_p, C.c_int]
+    L.lsdo_nfa_log_count.restype = C.c_int
+    buf = np.zeros((cap, 5))
+    L.lsdo_set_nfa_log(_p(buf), cap)
+    try:
+        out = lsd(map_u8, **kw)
+        n = L.lsdo_nfa_log_count()
+    finally:
+        L.lsdo_set_nfa_log(None, 0)
+    assert n < cap, "NFA tap full"
+    out["nfa_calls"] = buf[:n].copy()
+    return out
+
+
+def nfa_tail(all_pix, ali_pix, p, logNT, few=0.0, near=0.0, margin=0.0):
+    """lsdo_nfa_tail over arrays of tuples: (result, exit index, probe [n][5]); the probe counts each tail's break tests, those
+    at m == 1, those at 0 < |1 - m| <= few, those inside (near, margin) of the device's fast break test, and those inside the
+    margin without its |m^n| / |1 - m| term (lsd_oracle.h)"""
+    L = lib()
+    L.lsdo_nfa_tail_many.restype = None
+    L.lsdo_nfa_tail_many.argtypes = [C.c_int] + [C.c_void_p] * 4 + [C.c_double] * 3 + [C.c_void_p] * 3
+    a = np.ascontiguousarray(all_pix, np.int32); b = np.ascontiguousarray(ali_pix, np.int32)
+    pp = np.ascontiguousarray(p, np.float64); ln = np.ascontiguousarray(logNT, np.float64)
+    n = len(a)
+    out = np.zeros(n); ex = np.zeros(n, np.int32); probe = np.zeros((n, 5), np.int32)
+    L.lsdo_nfa_tail_many(n, _p(a), _p(b), _p(pp), _p(ln), few, near, margin, _p(out), _p(ex), _p(probe))
+    return out, ex, probe
+
+
+def log_gamma(xs):
+    L = lib()
+    L.lsdo_log_gamma.restype = C.c_double
+    L.lsdo_log_gamma.argtypes = [C.c_int]
+    return np.array([L.lsdo_log_gamma(int(x)) for x in xs])
+
+
 def gauss_taps(sca=0.3, sig=0.6):
     buf = np.zeros(3 * 64)
     h = lib().lsdo_gauss_taps(sca, sig, _p(buf), len(buf))
