@@ -404,7 +404,7 @@ static int run_regions(lsdb_batch* b) {
     CK(ctx, cudaEventRecord(b->ev[1], s));
     lsdb_launch_order(s, b->n, b->nBands, b->imgsD, b->dyn, b->kcD, b->mag, b->nzBits, b->bandOf, b->bandsOfImg, b->orderTabs, b->bins, b->cells);
     CK(ctx, cudaEventRecord(b->ev[2], s));
-    lsdb_launch_grow(s, b->n, b->nCtas, b->nWarps, b->imgsD, b->dyn, b->kcD, b->mag, b->deg, b->cosm, b->sinm, b->state, b->cells, b->labels, b->rects,
+    lsdb_launch_grow(s, b->n, b->nCtas, b->nWarps, b->imgsD, b->dyn, b->kcD, b->mag, b->deg, b->cosm, b->state, b->cells, b->labels, b->rects,
                      b->maxSeg, b->lists, b->listCap, b->arenaCap, b->runAhead, b->recBuf, ctx->lgammaTab, ctx->lgammaN, b->imgCounter, b->banBits,
                      b->bmCapWords, b->steal);
     CK(ctx, cudaEventRecord(b->ev[3], s));

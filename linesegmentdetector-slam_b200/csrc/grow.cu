@@ -80,6 +80,8 @@ struct GrowShared {
     unsigned int grid[GRID * GRID];          // per coarse cell: 1 + index of the LAST accepted region that touched the cell
     unsigned long long stats[TM_N];
 };
+// the team's state, at file scope so that every phase addresses it as shared memory (LDS / STS, not generic loads)
+__shared__ GrowShared growSh;
 
 #define LSDB_REJ_CAP (1 << 16)   // words per reject list of grow_region (two per warp)
 #define LSDB_PND_CAP (1 << 12)   // words of the pending-dependency list per warp
@@ -101,21 +103,24 @@ struct BBox { int x0, y0, x1, y1; };
 
 #if 1  /* cycle counters are cheap (one clock64 + one smem atomic per measured call) and feed bench.py */
 #define TIC long long t0_ = clock64()
-#define TOC(c, idx) do { if ((c).lane == 0) atomicAdd(&(c).sh->stats[idx], (unsigned long long)(clock64() - t0_)); } while (0)
+#define TOC(c, idx) do { if ((c).lane == 0) atomicAdd(&growSh.stats[idx], (unsigned long long)(clock64() - t0_)); } while (0)
 #else
 #define TIC
 #define TOC(c, idx)
 #endif
-#define STAT(c, idx, v) do { if ((c).lane == 0) atomicAdd(&(c).sh->stats[idx], (unsigned long long)(v)); } while (0)
+#define STAT(c, idx, v) do { if ((c).lane == 0) atomicAdd(&growSh.stats[idx], (unsigned long long)(v)); } while (0)
 
+// The context of a warp.  It is passed by reference to the __noinline__ phases, so it lives on the stack: the hot loops copy
+// the fields they use into locals first (every atomic, fence and state-word load would otherwise reload them from there).
+// The read-only planes are read through __ldg: nothing writes them while the kernel runs (the stencil stage precedes it on
+// the stream, and the giant path assembles them before the region stage).
 struct WarpCtx {
     int W, H, lane, w;
     unsigned int mybit;
     unsigned int* state;
     const double* deg;
     const double* mag;
-    const double* cosm;   // lsdm_cos(deg), lsdm_sin(deg) of every non-banned pixel (stencil stage)
-    const double* sinm;
+    const double2* cs;      // (lsdm_cos(deg), lsdm_sin(deg)) of every non-banned pixel (stencil stage: one interleaved plane)
     unsigned int* list;     // working point list (packed y<<16|x), listCap words
     unsigned int* scratch;  // 2*listCap+64 words: result of a frontier (non-speculative) evaluation
     unsigned int* arenas;   // NSLOTS record arenas of arenaCap words (parked speculative results, per super-chunk)
@@ -124,7 +129,6 @@ struct WarpCtx {
     const LsdbLsdConst* kc;
     const double* lgammaTab;
     int lgammaN;
-    GrowShared* sh;
     unsigned int* rej[2];   // reject lists of grow_region (ping-pong), rejCap words each
     int rejCap;
     unsigned int* pnd;      // pixels the current speculative evaluation skipped because a PARKED accept covers them
@@ -133,10 +137,7 @@ struct WarpCtx {
     int specChunk;          // seed-list chunk of the seed being evaluated speculatively; -1 at the frontier (parked
                             //   regions are then ignored: the state is final)
     double* stage;          // 32 x 4 doubles of shared memory: operands of the ordered sums in rect_from_region
-    volatile unsigned int* bm;   // the ban plane (usedMap==1), one bit per pixel, pw words per row: its shared-memory copy when the map
-                                 // fits (bmInSmem), else the global plane itself (48 MB for 256 maps of 4096^2: L2-resident, unlike the
-                                 // 1.5 GB of state words)
-    bool bmInSmem;
+    unsigned int* bm;       // the map's global ban plane (see BanPlane); unused by the build that keeps it in shared memory
     int pw;
     double logNT, regThre;
     int cellShift;        // accept-grid cell = 2^cellShift pixels, grid <= GRID x GRID
@@ -159,49 +160,58 @@ __device__ __forceinline__ int py_of(unsigned int v) { return (int)(v >> 16); }
 
 // clear this warp's curMap bit on list[0..num)
 __device__ void clear_bits(const WarpCtx& c, const unsigned int* lst, int num) {
+    unsigned int* const state = c.state;
+    const int W = c.W;
+    const unsigned int keep = ~c.mybit;
     for (int k = c.lane; k < num; k += 32) {
         unsigned int v = lst[k];
-        atomicAnd(&c.state[(size_t)py_of(v) * c.W + px_of(v)], ~c.mybit);
+        atomicAnd(&state[(size_t)py_of(v) * W + px_of(v)], keep);
     }
     __syncwarp();
 }
 
 // ------------------------------------------------------------------ ban plane (usedMap == 1)
-// The hot question of the grower — "is this neighbour banned?" (:537) — is answered from a one-bit-per-pixel
-// copy of the plane in shared memory when the map fits (c.bm), else from the global state words.
-__device__ __forceinline__ bool ban_at(const WarpCtx& c, int x, int y) {
-    if (c.bm) return (c.bm[(size_t)y * c.pw + (x >> 5)] >> (x & 31)) & 1u;
-    return (lsdb_ld_state(&c.state[(size_t)y * c.W + x]) & LSDB_ST_BAN) != 0;
-}
-// bits (x-1, x, x+1) of row y, bit 0 = x-1; out-of-image pixels read as banned
-__device__ __forceinline__ unsigned int ban_row3(const WarpCtx& c, int x, int y) {
-    if (y < 0 || y >= c.H) return 7u;
-    unsigned int out;
-    if (c.bm) {
-        const volatile unsigned int* r = c.bm + (size_t)y * c.pw;
-        if (x == 0) out = ((r[0] << 1) | 1u) & 7u;
+// The hot question of the grower — "is this neighbour banned?" (:537) — is answered from a one-bit-per-pixel plane,
+// pw words per row.  The kernel is built twice: BS (ban plane in shared memory) copies the plane of the map into shared memory
+// (bmShared) and reads it with LDS; the host runs that build only when every map of the batch fits bmCapWords.  The other build
+// reads the global plane that the stencil stage wrote (48 MB for 256 maps of 4096^2: L2-resident, unlike the 1.5 GB of state
+// words) with ld.global.cg, the coherence level of the state words; commits set its bits with atomics.
+extern __shared__ unsigned int bmShared[];
+template <bool BS>
+struct BanPlane {
+    unsigned int* g;   // the global plane of the map (!BS)
+    int pw, W, H;
+    __device__ __forceinline__ unsigned int word(size_t i) const {
+        if (BS) return static_cast<const volatile unsigned int*>(bmShared)[i];
+        return __ldcg(g + i);
+    }
+    __device__ __forceinline__ bool at(int x, int y) const { return (word((size_t)y * pw + (x >> 5)) >> (x & 31)) & 1u; }
+    // bits (x-1, x, x+1) of row y, bit 0 = x-1; out-of-image pixels read as banned
+    __device__ __forceinline__ unsigned int row3(int x, int y) const {
+        if (y < 0 || y >= H) return 7u;
+        const size_t r = (size_t)y * pw;
+        unsigned int out;
+        if (x == 0) out = ((word(r) << 1) | 1u) & 7u;
         else {
             const int xl = x - 1, wi = xl >> 5, sh = xl & 31;
-            const unsigned int lo = r[wi];
-            const unsigned int hi = (sh > 29 && wi + 1 < c.pw) ? r[wi + 1] : 0xffffffffu;
+            const unsigned int lo = word(r + wi);
+            const unsigned int hi = (sh > 29 && wi + 1 < pw) ? word(r + wi + 1) : 0xffffffffu;
             out = __funnelshift_r(lo, hi, sh) & 7u;
         }
-    } else {
-        const unsigned int* r = c.state + (size_t)y * c.W;
-        out = 0;
-        if (x == 0 || (lsdb_ld_state(&r[x - 1]) & LSDB_ST_BAN)) out |= 1u;
-        if (lsdb_ld_state(&r[x]) & LSDB_ST_BAN) out |= 2u;
-        if (x + 1 >= c.W || (lsdb_ld_state(&r[x + 1]) & LSDB_ST_BAN)) out |= 4u;
+        if (x + 1 >= W) out |= 4u;
+        return out;
     }
-    if (x + 1 >= c.W) out |= 4u;
-    return out;
-}
-// the 3x3 neighbourhood of (x,y) in the reference's scan order (:533-535): bit (dy+1)*3+(dx+1) set = banned / outside
-__device__ __forceinline__ unsigned int ban9(const WarpCtx& c, int x, int y) {
-    return ban_row3(c, x, y - 1) | (ban_row3(c, x, y) << 3) | (ban_row3(c, x, y + 1) << 6);
-}
-__device__ __forceinline__ void ban_set(const WarpCtx& c, int x, int y) {
-    if (c.bm) atomicOr(const_cast<unsigned int*>(c.bm) + (size_t)y * c.pw + (x >> 5), 1u << (x & 31));
+    // the 3x3 neighbourhood of (x,y) in the reference's scan order (:533-535): bit (dy+1)*3+(dx+1) set = banned / outside
+    __device__ __forceinline__ unsigned int nb9(int x, int y) const { return row3(x, y - 1) | (row3(x, y) << 3) | (row3(x, y + 1) << 6); }
+    __device__ __forceinline__ void set(int x, int y) const {
+        atomicOr((BS ? bmShared : g) + (size_t)y * pw + (x >> 5), 1u << (x & 31));
+    }
+};
+template <bool BS>
+__device__ __forceinline__ BanPlane<BS> ban_plane(const WarpCtx& c) {
+    BanPlane<BS> b;
+    b.g = c.bm; b.pw = c.pw; b.W = c.W; b.H = c.H;
+    return b;
 }
 
 // ------------------------------------------------------------------ parked regions
@@ -212,8 +222,10 @@ __device__ __forceinline__ bool pend_applies(unsigned int st, unsigned int kinds
 // mark the pixels of a parked accept / reject candidate (kind = LSDB_ST_PACC / LSDB_ST_PREJ); the earliest chunk tag wins
 __device__ void park_pixels(const WarpCtx& c, const unsigned int* px, int n, unsigned int kind, int chunk) {
     const unsigned int tag = (unsigned int)chunk & 4095u;
+    unsigned int* const state = c.state;
+    const int W = c.W;
     for (int k = c.lane; k < n; k += 32) {
-        unsigned int* w = &c.state[(size_t)py_of(px[k]) * c.W + px_of(px[k])];
+        unsigned int* w = &state[(size_t)py_of(px[k]) * W + px_of(px[k])];
         unsigned int old = lsdb_ld_state(w);
         while (true) {
             unsigned int neu;
@@ -230,8 +242,10 @@ __device__ void park_pixels(const WarpCtx& c, const unsigned int* px, int n, uns
 // a parked candidate was dropped (its seed died, or the evaluation was invalidated): take its marks back
 __device__ void unpark_pixels(const WarpCtx& c, const unsigned int* px, int n, int chunk) {
     const unsigned int tag = (unsigned int)chunk & 4095u;
+    unsigned int* const state = c.state;
+    const int W = c.W;
     for (int k = c.lane; k < n; k += 32) {
-        unsigned int* w = &c.state[(size_t)py_of(px[k]) * c.W + px_of(px[k])];
+        unsigned int* w = &state[(size_t)py_of(px[k]) * W + px_of(px[k])];
         const unsigned int old = lsdb_ld_state(w);
         if ((old & (LSDB_ST_PACC | LSDB_ST_PREJ)) && (old >> LSDB_ST_TAG_SHIFT) == tag) atomicAnd(w, ~(LSDB_ST_PACC | LSDB_ST_PREJ));
     }
@@ -285,11 +299,21 @@ __device__ __forceinline__ void sums_refresh(GrowSums& g, double c2, double cTau
 // accept loop over the (up to 32) candidates the lanes hold, in lane order.  cand: lane holds a live candidate
 // (in the image, not banned, not in the region); p/n/m its pixel; dg/cd/sd its angle data.  On return cand is
 // true exactly for the candidates that failed the angle test (the rest joined the region or dropped out).
+// the fields of WarpCtx that the grower's loop uses, held in registers
+struct GrowIO {
+    unsigned int* state;
+    unsigned int* list;
+    const double* deg;
+    int listCap, lane;
+    unsigned int mybit;
+    double pi;
+};
+
 template <bool tauSmall>
-__device__ __forceinline__ int accept_lanes(WarpCtx& c, GrowSums& g, bool& cand, size_t p, int n, int m, double dg, double cd, double sd,
+__device__ __forceinline__ int accept_lanes(const GrowIO& c, GrowSums& g, bool& cand, size_t p, int n, int m, double dg, double cd, double sd,
                                             int& num, bool& haveExact, double& regExact, double degThre, double c2, double cTau,
                                             bool tauGtPi, float tauF) {
-    const double pi = c.kc->pi;
+    const double pi = c.pi;
     const double pi32 = pi * 3 / 2.0, pi2 = 2.0 * pi;
     int start = 0;
     if (tauSmall && g.nrmOK && g.n2 >= 1.0) {
@@ -369,7 +393,7 @@ __device__ __forceinline__ int accept_lanes(WarpCtx& c, GrowSums& g, bool& cand,
         if (__any_sync(FULL, unc)) {
             if (!haveExact) { regExact = d_atan2(g.sinDeg, g.cosDeg); haveExact = true; }
             if (unc) {  // the literal test, :540-543
-                if (tauSmall) dg = c.deg[p];   // not loaded up front on this path
+                if (tauSmall) dg = __ldg(&c.deg[p]);   // not loaded up front on this path
                 double degDif = fabs(regExact - dg);
                 if (degDif > pi32) degDif = fabs(degDif - pi2);
                 pass = degDif < degThre;
@@ -397,35 +421,47 @@ __device__ __forceinline__ int accept_lanes(WarpCtx& c, GrowSums& g, bool& cand,
 
 // two builds of the grower: the common one (tolerance <= pi/2: the test on the squares only) keeps the float / sqrt / un-wrapped-band
 // code of the wide tolerances (Refiner re-grows with 2 sigma, :857) out of its loop
-template <bool tauSmall>
+template <bool tauSmall, bool BS>
 __device__ __noinline__ int grow_region_t(WarpCtx& c, int sx, int sy, double& regDeg, double degThre, BBox& bb) {
     const int W = c.W, H = c.H;
-    const double pi = c.kc->pi;
+    GrowIO io;
+    io.state = c.state; io.list = c.list; io.deg = c.deg; io.listCap = c.listCap; io.lane = c.lane; io.mybit = c.mybit; io.pi = c.kc->pi;
+    const double pi = io.pi;
+    const double2* const cs = c.cs;
+    const BanPlane<BS> bp = ban_plane<BS>(c);
+    unsigned int* const rej0 = c.rej[0];
+    unsigned int* const rej1 = c.rej[1];
+    unsigned int* const pndList = c.pnd;
+    const int rejCap = c.rejCap, specChunk = c.specChunk;
+    int npnd = c.npnd;
     TIC;
     const size_t sp = (size_t)sy * W + sx;
     const double regDeg0 = regDeg;
     GrowSums g;
-    g.sinDeg = c.sinm[2 * sp]; g.cosDeg = c.cosm[2 * sp];  // sin(regDeg), cos(regDeg)  (:515-516)
+    {
+        const double2 v = __ldg(&cs[sp]);
+        g.cosDeg = v.x; g.sinDeg = v.y;   // cos(regDeg), sin(regDeg)  (:515-516)
+    }
     const bool tauGtPi = degThre > pi;
     const double cTau = degThre == c.kc->degThre ? c.kc->cosDegThre : (tauGtPi ? -1.0 : d_cos(degThre));
     const double c2 = cTau * cTau;
     const float tauF = (float)degThre;
-    if (c.lane == 0) {
-        c.list[0] = pack_xy(sx, sy);
-        atomicOr(&c.state[sp], c.mybit);
+    if (io.lane == 0) {
+        io.list[0] = pack_xy(sx, sy);
+        atomicOr(&io.state[sp], io.mybit);
     }
     __syncwarp();
     int num = 1;
     sums_refresh<tauSmall>(g, c2, cTau);
     bool haveExact = true;
     double regExact = regDeg0;
-    const unsigned int lt = (1u << c.lane) - 1u;
+    const unsigned int lt = (1u << io.lane) - 1u;
     int startNum = 0, nPrev = 0, cur = 0;   // cur = which reject buffer is being filled
     bool literal = false;                   // reject list overflowed: literal full re-scans from now on
     while (true) {
         const int numAtStart = num;
-        unsigned int* rPrev = c.rej[cur ^ 1];
-        unsigned int* rNext = c.rej[cur];
+        unsigned int* rPrev = cur ? rej0 : rej1;
+        unsigned int* rNext = cur ? rej1 : rej0;
         int nNext = 0;
         // (i) the candidates that failed the angle test in the previous pass, in scan order, then
         // (ii) the points that have not been scanned yet (all of them while `literal`)
@@ -439,45 +475,52 @@ __device__ __noinline__ int grow_region_t(WarpCtx& c, int sx, int sy, double& re
             bool cand;
             unsigned int banMask;
             if (rescan) {
-                const int e = base + c.lane;
+                const int e = base + io.lane;
                 cand = e < nPrev;
                 const unsigned int pv = cand ? rPrev[e] : 0u;
                 n = px_of(pv); m = py_of(pv);
-                banMask = c.mybit;               // may have joined the region meanwhile
+                banMask = io.mybit;              // may have joined the region meanwhile
             } else {
-                const int myc = pos + c.lane;
+                const int myc = pos + io.lane;
                 const bool valid = myc < lim;
                 const int pt = myc / 9, nb = myc - pt * 9;
-                const unsigned int pv = valid ? c.list[pt] : 0u;
+                const unsigned int pv = valid ? io.list[pt] : 0u;
                 const int r3 = nb / 3;
                 m = py_of(pv) + r3 - 1; n = px_of(pv) + (nb - r3 * 3) - 1;
                 // banned? — from the shared-memory bit plane; only un-banned candidates touch global memory
-                cand = valid && m >= 0 && n >= 0 && m < H && n < W && !(c.bmInSmem && ban_at(c, n, m));
-                banMask = LSDB_ST_BAN | c.mybit;
+                cand = valid && m >= 0 && n >= 0 && m < H && n < W && !(BS && bp.at(n, m));
+                banMask = LSDB_ST_BAN | io.mybit;
             }
             const size_t p = cand ? (size_t)m * W + n : 0;
-            const unsigned int st = cand ? lsdb_ld_state(&c.state[p]) : 0u;
+            const unsigned int st = cand ? lsdb_ld_state(&io.state[p]) : 0u;
             double dg = 0.0, cd = 0.0, sd = 0.0;
-            if (cand) { cd = c.cosm[2 * p]; sd = c.sinm[2 * p]; if (!tauSmall) dg = c.deg[p]; }  // issued with the state load, not after it
+            if (cand) {   // issued with the state load, not after it
+                const double2 v = __ldg(&cs[p]);
+                cd = v.x; sd = v.y;
+                if (!tauSmall) dg = __ldg(&io.deg[p]);
+            }
             cand = cand && !(st & banMask);
-            if (c.specChunk >= 0) {
+            if (specChunk >= 0) {
                 // speculation: a pixel inside a region an earlier seed has parked for acceptance counts as banned;
                 // it is listed so that the guess can be checked when this evaluation retires
-                const bool pend = cand && pend_applies(st, LSDB_ST_PACC, c.specChunk);
+                const bool pend = cand && pend_applies(st, LSDB_ST_PACC, specChunk);
                 const unsigned int pb = __ballot_sync(FULL, pend);
                 if (pb) {
-                    if (c.npnd >= 0 && c.npnd + 32 <= LSDB_PND_CAP) {
-                        if (pend) c.pnd[c.npnd + __popc(pb & lt)] = pack_xy(n, m);
-                        c.npnd += __popc(pb);
-                    } else c.npnd = -1;
+                    if (npnd >= 0 && npnd + 32 <= LSDB_PND_CAP) {
+                        if (pend) pndList[npnd + __popc(pb & lt)] = pack_xy(n, m);
+                        npnd += __popc(pb);
+                    } else npnd = -1;
                     if (pend) cand = false;
                 }
             }
-            if (accept_lanes<tauSmall>(c, g, cand, p, n, m, dg, cd, sd, num, haveExact, regExact, degThre, c2, cTau, tauGtPi, tauF) < 0) return -1;
+            if (accept_lanes<tauSmall>(io, g, cand, p, n, m, dg, cd, sd, num, haveExact, regExact, degThre, c2, cTau, tauGtPi, tauF) < 0) {
+                c.npnd = npnd;
+                return -1;
+            }
             if (!literal) {
                 const unsigned int rb = __ballot_sync(FULL, cand);
                 if (rb) {
-                    if (nNext + 32 > c.rejCap) literal = true;
+                    if (nNext + 32 > rejCap) literal = true;
                     else { if (cand) rNext[nNext + __popc(rb & lt)] = pack_xy(n, m); nNext += __popc(rb); }
                 }
             }
@@ -489,9 +532,10 @@ __device__ __noinline__ int grow_region_t(WarpCtx& c, int sx, int sy, double& re
         nPrev = literal ? 0 : nNext;
         cur ^= 1;
     }
+    c.npnd = npnd;
     if (num > 1) regDeg = haveExact ? regExact : d_atan2(g.sinDeg, g.cosDeg);  // :547 after the last accept
-    for (int k = c.lane; k < num; k += 32) {   // bounding box / coarse cells of the accepted pixels
-        const unsigned int v = c.list[k];
+    for (int k = io.lane; k < num; k += 32) {   // bounding box / coarse cells of the accepted pixels
+        const unsigned int v = io.list[k];
         bbox_add(c, bb, px_of(v), py_of(v));
     }
 #pragma unroll
@@ -504,8 +548,10 @@ __device__ __noinline__ int grow_region_t(WarpCtx& c, int sx, int sy, double& re
     return num;
 }
 
+template <bool BS>
 __device__ __forceinline__ int grow_region(WarpCtx& c, int sx, int sy, double& regDeg, double degThre, BBox& bb) {
-    return degThre <= c.kc->pi / 2.0 ? grow_region_t<true>(c, sx, sy, regDeg, degThre, bb) : grow_region_t<false>(c, sx, sy, regDeg, degThre, bb);
+    return degThre <= c.kc->pi / 2.0 ? grow_region_t<true, BS>(c, sx, sy, regDeg, degThre, bb)
+                                     : grow_region_t<false, BS>(c, sx, sy, regDeg, degThre, bb);
 }
 
 // ------------------------------------------------------------------ RegionGrower, one LANE per seed
@@ -526,19 +572,26 @@ __device__ __forceinline__ int grow_region(WarpCtx& c, int sx, int sy, double& r
 // A lane's own pixels are found through a 64-bit filter on (x + 8y) first; the list is only searched on a filter hit.
 __device__ __forceinline__ unsigned long long sg_bit(int x, int y) { return 1ull << ((x + 8 * y) & 63); }
 
+// The pending list has the same kind of filter.
+template <bool BS>
 __device__ __noinline__ int small_grow(const WarpCtx& c, bool act, int p0, int T, unsigned int* lst, int myChunk, unsigned int* pnd, int& npnd) {
     const int W = c.W;
     const double pi = c.kc->pi, pi32 = pi * 3 / 2.0, pi2 = 2.0 * pi;
     const double degThre = c.kc->degThre, cTau = c.kc->cosDegThre;
+    unsigned int* const state = c.state;
+    const double* const deg = c.deg;
+    const double2* const cs = c.cs;
+    const BanPlane<BS> bp = ban_plane<BS>(c);
     unsigned short rej[SG_CAP];
     const double c2 = cTau * cTau;
     double cosS = 0.0, sinS = 0.0, n2 = 0.0, c2n2 = 0.0, m2 = 0.0;   // see grow_region: the test on the squares
     bool nrmOK = false;
-    unsigned long long mine = 0ull;
+    unsigned long long mine = 0ull, pndF = 0ull;
     int num = 0;
     if (act) {
         const int sx = p0 % W, sy = p0 / W;
-        cosS = c.cosm[2 * (size_t)p0]; sinS = c.sinm[2 * (size_t)p0];
+        const double2 v = __ldg(&cs[p0]);
+        cosS = v.x; sinS = v.y;
         n2 = cosS * cosS + sinS * sinS; c2n2 = c2 * n2; m2 = 4e-13 * n2;
         nrmOK = n2 > 1e-18;
         lst[0] = pack_xy(sx, sy);
@@ -561,7 +614,7 @@ __device__ __noinline__ int small_grow(const WarpCtx& c, bool act, int p0, int T
             if (running) {
                 const unsigned int v = lst[i];
                 x = px_of(v); y = py_of(v);
-                cm = i >= startNum ? (~ban9(c, x, y)) & 0x1efu : (unsigned int)rej[i];
+                cm = i >= startNum ? (~bp.nb9(x, y)) & 0x1efu : (unsigned int)rej[i];
                 nr = 0;
             }
         }
@@ -576,20 +629,25 @@ __device__ __noinline__ int small_grow(const WarpCtx& c, bool act, int p0, int T
                 for (int k = 0; k < num; k++) own |= lst[k] == pk;
             if (!own) {
                 const size_t p = (size_t)m * W + n;
-                const unsigned int st = lsdb_ld_state(&c.state[p]);
-                const double cd = c.cosm[2 * p], sd = c.sinm[2 * p];
+                const unsigned int st = lsdb_ld_state(&state[p]);
+                const double2 v = __ldg(&cs[p]);
+                const double cd = v.x, sd = v.y;
                 if (!(st & LSDB_ST_BAN)) {
                     if (pend_applies(st, LSDB_ST_PACC, myChunk)) {   // parked for acceptance by an earlier seed: counts as banned,
                         bool dup = false;                            // to be confirmed when this evaluation retires
-                        for (int j = 0; j < npnd; j++) dup |= pnd[j] == pk;
-                        if (!dup) { if (npnd >= 0 && npnd < SG_PND) pnd[npnd++] = pk; else npnd = -1; }
+                        if (pndF & sg_bit(n, m))
+                            for (int j = 0; j < npnd; j++) dup |= pnd[j] == pk;
+                        if (!dup) {
+                            if (npnd >= 0 && npnd < SG_PND) { pnd[npnd++] = pk; pndF |= sg_bit(n, m); }
+                            else npnd = -1;
+                        }
                     } else {
                         const double dot = cosS * cd + sinS * sd;
                         const double d2 = dot * dot - c2n2;
                         bool pass = dot > 0 && d2 > 0;
                         if ((dot > 0 && !(fabs(d2) > m2)) || !nrmOK) {  // knife edge: the literal test of :540-543
-                            const double regDeg = num == 1 ? c.deg[p0] : d_atan2(sinS, cosS);
-                            double degDif = fabs(regDeg - c.deg[p]);
+                            const double regDeg = num == 1 ? __ldg(&deg[p0]) : d_atan2(sinS, cosS);
+                            double degDif = fabs(regDeg - __ldg(&deg[p]));
                             if (degDif > pi32) degDif = fabs(degDif - pi2);
                             pass = degDif < degThre;
                         }
@@ -619,7 +677,8 @@ __device__ __noinline__ int small_grow(const WarpCtx& c, bool act, int p0, int T
 // ------------------------------------------------------------------ RectangleConverter (:592-734)
 __device__ __noinline__ Rect rect_from_region(const WarpCtx& c, const unsigned int* lst, int num, double regDeg, double aliPro,
                                  double degThre) {
-    const int W = c.W;
+    const int W = c.W, lane = c.lane;
+    const double* const mag = c.mag;
     const double pi = c.kc->pi;
     TIC;
     // Sums are accumulated in list order like the reference (:608-613, :637-643).  The lanes form the addends of 32
@@ -628,16 +687,16 @@ __device__ __noinline__ Rect rect_from_region(const WarpCtx& c, const unsigned i
     double* stg = c.stage;
     double acc = 0.0;
     for (int base = 0; base < num; base += 32) {  // CenterGetter :608-613: lane 0 cenX, lane 1 cenY, lane 2 weiSum
-        const int k = base + c.lane;
+        const int k = base + lane;
         const unsigned int v = k < num ? lst[k] : 0u;
-        const double wv = k < num ? c.mag[(size_t)py_of(v) * W + px_of(v)] : 0.0;
-        stg[c.lane * 4 + 0] = wv * px_of(v);
-        stg[c.lane * 4 + 1] = wv * py_of(v);
-        stg[c.lane * 4 + 2] = wv;
+        const double wv = k < num ? __ldg(&mag[(size_t)py_of(v) * W + px_of(v)]) : 0.0;
+        stg[lane * 4 + 0] = wv * px_of(v);
+        stg[lane * 4 + 1] = wv * py_of(v);
+        stg[lane * 4 + 2] = wv;
         __syncwarp();
         const int cnt = min(32, num - base);
-        if (c.lane < 3)
-            for (int j = 0; j < cnt; j++) acc += stg[j * 4 + c.lane];
+        if (lane < 3)
+            for (int j = 0; j < cnt; j++) acc += stg[j * 4 + lane];
         __syncwarp();
     }
     double cenX = __shfl_sync(FULL, acc, 0), cenY = __shfl_sync(FULL, acc, 1), weiSum = __shfl_sync(FULL, acc, 2);
@@ -645,18 +704,18 @@ __device__ __noinline__ Rect rect_from_region(const WarpCtx& c, const unsigned i
     cenY = cenY / weiSum;
     acc = 0.0;
     for (int base = 0; base < num; base += 32) {  // OrientationGetter :637-643: lane 0 Ixx, 1 Iyy, 2 Ixy, 3 weiSum
-        const int k = base + c.lane;
+        const int k = base + lane;
         const unsigned int v = k < num ? lst[k] : 0u;
-        const double wv = k < num ? c.mag[(size_t)py_of(v) * W + px_of(v)] : 0.0;
+        const double wv = k < num ? __ldg(&mag[(size_t)py_of(v) * W + px_of(v)]) : 0.0;
         const double ey = py_of(v) - cenY, ex = px_of(v) - cenX;
-        stg[c.lane * 4 + 0] = wv * (ey * ey);
-        stg[c.lane * 4 + 1] = wv * (ex * ex);
-        stg[c.lane * 4 + 2] = -(wv * ex * ey);   // Ixy -= t  ==  Ixy += -t
-        stg[c.lane * 4 + 3] = wv;
+        stg[lane * 4 + 0] = wv * (ey * ey);
+        stg[lane * 4 + 1] = wv * (ex * ex);
+        stg[lane * 4 + 2] = -(wv * ex * ey);   // Ixy -= t  ==  Ixy += -t
+        stg[lane * 4 + 3] = wv;
         __syncwarp();
         const int cnt = min(32, num - base);
-        if (c.lane < 4)
-            for (int j = 0; j < cnt; j++) acc += stg[j * 4 + c.lane];
+        if (lane < 4)
+            for (int j = 0; j < cnt; j++) acc += stg[j * 4 + lane];
         __syncwarp();
     }
     double Ixx = __shfl_sync(FULL, acc, 0), Iyy = __shfl_sync(FULL, acc, 1), Ixy = __shfl_sync(FULL, acc, 2);
@@ -675,7 +734,7 @@ __device__ __noinline__ Rect rect_from_region(const WarpCtx& c, const unsigned i
 
     const double dx = d_cos(inertiaDeg), dy = d_sin(inertiaDeg);
     double lenMin = 0, lenMax = 0, widMin = 0, widMax = 0;  // :701-714, order-free
-    for (int k = c.lane; k < num; k += 32) {
+    for (int k = lane; k < num; k += 32) {
         const unsigned int v = lst[k];
         const double len = (px_of(v) - cenX) * dx + (py_of(v) - cenY) * dy;
         const double wid = -(px_of(v) - cenX) * dy + (py_of(v) - cenY) * dx;
@@ -714,7 +773,8 @@ __device__ __forceinline__ double dist_xy(int ox, int oy, double x, double y) {
 
 // ------------------------------------------------------------------ RectangleNFACalculator (:926-1059)
 __device__ __noinline__ double rect_nfa_impl(WarpCtx& c, const Rect& rec, double logNT) {
-    const int xLim = c.W, yLim = c.H;
+    const int xLim = c.W, yLim = c.H, lane = c.lane;
+    const double* const deg = c.deg;
     const double pi = c.kc->pi;
     const double pi32 = pi * 3 / 2.0, pi2 = 2 * pi;
     double verX[4], verY[4];
@@ -743,7 +803,7 @@ __device__ __noinline__ double rect_nfa_impl(WarpCtx& c, const Rect& rec, double
         const double k1 = (vY2 - vY1) / (vX2 - vX1);
         const double k2 = (vY2 - vY3) / (vX2 - vX3);
         const double k3 = (vY3 - vY0) / (vX3 - vX0);
-        for (int i = c.lane; i < xRang_len; i += 32) {
+        for (int i = lane; i < xRang_len; i += 32) {
             const int xi = lsdb_x86_d2i(i + x0c);
             // the reference fills yLow/yHigh with two partition passes (:987-1004); xi is
             // increasing, so entry i takes the first branch iff xi < vertex (NaN vertex: slot stays 0)
@@ -756,7 +816,7 @@ __device__ __noinline__ double rect_nfa_impl(WarpCtx& c, const Rect& rec, double
             const int j0 = yl < 0 ? 0 : yl, j1 = yh > yLim - 1 ? yLim - 1 : yh;
             for (int j = j0; j <= j1; j++) {
                 allPixNum++;
-                double degDif = fabs(rec.deg - c.deg[(size_t)j * xLim + xi]);
+                double degDif = fabs(rec.deg - __ldg(&deg[(size_t)j * xLim + xi]));
                 if (degDif > pi32) degDif = fabs(degDif - pi2);
                 if (degDif < rec.prec) aliPixNum++;
             }
@@ -837,6 +897,7 @@ __device__ bool park_pend(WarpCtx& c, unsigned int* body, int& aw, int cap, int&
     return true;
 }
 
+template <bool BS>
 __device__ __noinline__ int eval_seed(WarpCtx& c, int p0, unsigned int* out, int cap, bool wantChk, BBox& bb, int& used, int& chk, int& pndOff, int& pndN) {
     c.npnd = 0; pndOff = 0; pndN = 0;
     const LsdbLsdConst* kc = c.kc;
@@ -846,8 +907,8 @@ __device__ __noinline__ int eval_seed(WarpCtx& c, int p0, unsigned int* out, int
     used = 0;
     chk = -1;
     double regDeg = c.deg[p0];
-    int num = grow_region(c, sx, sy, regDeg, kc->degThre, bb);
-    if (num < 0) { c.sh->abortFlag = LSDB_ERR_CAPACITY; return OC_NOCHANGE; }
+    int num = grow_region<BS>(c, sx, sy, regDeg, kc->degThre, bb);
+    if (num < 0) { growSh.abortFlag = LSDB_ERR_CAPACITY; return OC_NOCHANGE; }
     unsigned int* body = out + ARENA_HDR;
     int aw = 0;  // words written after the header
     if (num < c.regThre) {  // :228
@@ -903,9 +964,9 @@ __device__ __noinline__ int eval_seed(WarpCtx& c, int p0, unsigned int* out, int
         }
         clear_bits(c, c.list, num);
         regDeg = cenDeg;
-        num = grow_region(c, sx, sy, regDeg, degThre2, bb);
+        num = grow_region<BS>(c, sx, sy, regDeg, degThre2, bb);
         STAT(c, ST_REGROWS, 1);
-        if (num < 0) { c.sh->abortFlag = LSDB_ERR_CAPACITY; return OC_NOCHANGE; }
+        if (num < 0) { growSh.abortFlag = LSDB_ERR_CAPACITY; return OC_NOCHANGE; }
         if (ARENA_HDR + aw + 2 * num + 8 > cap) { clear_bits(c, c.list, num); return OC_DEFER; }
         backup = body + aw;  // G2 in full: re-validation list and RegionRadiusReducer's "every pixel the bit was set on"
         for (int k = c.lane; k < num; k += 32) backup[k] = c.list[k];
@@ -944,7 +1005,7 @@ __device__ __noinline__ int eval_seed(WarpCtx& c, int p0, unsigned int* out, int
                             i++;
                         }
                         num = nn;
-                        atomicAdd(&c.sh->stats[ST_RRR], 1ull);
+                        atomicAdd(&growSh.stats[ST_RRR], 1ull);
                     }
                     __syncwarp();
                     num = __shfl_sync(FULL, num, 0);
@@ -1008,20 +1069,24 @@ __device__ __noinline__ int eval_seed(WarpCtx& c, int p0, unsigned int* out, int
     return oc;
 }
 
+template <bool BS>
 __device__ bool any_unbanned(const WarpCtx& c, const unsigned int* px, int n) {
+    const BanPlane<BS> bp = ban_plane<BS>(c);
     bool hit = false;
     for (int k = c.lane; k < n; k += 32) {
         const unsigned int v = px[k];
-        if (!ban_at(c, px_of(v), py_of(v))) hit = true;
+        if (!bp.at(px_of(v), py_of(v))) hit = true;
     }
     return __any_sync(FULL, hit);
 }
 
+template <bool BS>
 __device__ bool any_banned(const WarpCtx& c, const unsigned int* px, int n) {
+    const BanPlane<BS> bp = ban_plane<BS>(c);
     bool hit = false;
     for (int k = c.lane; k < n; k += 32) {
         const unsigned int v = px[k];
-        if (ban_at(c, px_of(v), py_of(v))) hit = true;
+        if (bp.at(px_of(v), py_of(v))) hit = true;
     }
     return __any_sync(FULL, hit);
 }
@@ -1033,13 +1098,14 @@ __device__ __forceinline__ bool grid_hit(const WarpCtx& c, unsigned int b0, unsi
     const int cx0 = px_of(b0) >> sh, cy0 = py_of(b0) >> sh, cx1 = px_of(b1) >> sh, cy1 = py_of(b1) >> sh;
     for (int cy = cy0; cy <= cy1; cy++)
         for (int cx = cx0; cx <= cx1; cx++)
-            if (*(volatile unsigned int*)&c.sh->grid[cy * GRID + cx] > (unsigned int)L0) return true;
+            if (*(volatile unsigned int*)&growSh.grid[cy * GRID + cx] > (unsigned int)L0) return true;
     return false;
 }
 
 // commit the result record at `recp`, at the frontier (:242-271)
+template <bool BS>
 __device__ void commit_region(WarpCtx& c, const unsigned int* recp, int* labels, LsdbRect* rects, int maxSeg) {
-    GrowShared* sh = c.sh;
+    GrowShared& sh = growSh;
     const int W = c.W;
     const int nCommit = (int)recp[26], outcome = (int)recp[27];
     const unsigned int* px = recp + recp[28];
@@ -1052,14 +1118,17 @@ __device__ void commit_region(WarpCtx& c, const unsigned int* recp, int* labels,
         __syncwarp();
         return;
     }
-    const int idx = sh->nSeg;
+    const int idx = sh.nSeg;
+    const BanPlane<BS> bp = ban_plane<BS>(c);
+    unsigned int* const state = c.state;
+    const int cellShift = c.cellShift;
     for (int k = c.lane; k < nCommit; k += 32) {
         const unsigned int v = px[k];
         const size_t p = (size_t)py_of(v) * W + px_of(v);
-        atomicOr(&c.state[p], LSDB_ST_BAN);
-        ban_set(c, px_of(v), py_of(v));
+        atomicOr(&state[p], LSDB_ST_BAN);
+        bp.set(px_of(v), py_of(v));
         labels[p] += idx + 1;  // regIdx += curMap*(regCnt+1), :261 (int32 here, u8 there)
-        atomicMax(&sh->grid[(py_of(v) >> c.cellShift) * GRID + (px_of(v) >> c.cellShift)], (unsigned int)idx + 1u);
+        atomicMax(&sh.grid[(py_of(v) >> cellShift) * GRID + (px_of(v) >> cellShift)], (unsigned int)idx + 1u);
     }
     __syncwarp();
     __threadfence_block();
@@ -1077,10 +1146,10 @@ __device__ void commit_region(WarpCtx& c, const unsigned int* recp, int* labels,
             R.v[0] = rx1; R.v[1] = ry1; R.v[2] = rx2; R.v[3] = ry2; R.v[4] = rw;
             for (int k = 5; k < 13; k++) R.v[k] = hd[k];
         } else {
-            sh->abortFlag = LSDB_ERR_CAPACITY;
+            sh.abortFlag = LSDB_ERR_CAPACITY;
         }
-        sh->nSeg = idx + 1;
-        atomicAdd(&sh->stats[ST_ACCEPTS], 1ull);
+        sh.nSeg = idx + 1;
+        atomicAdd(&sh.stats[ST_ACCEPTS], 1ull);
     }
     __syncwarp();
 }
@@ -1101,7 +1170,7 @@ struct ChunkRecs {
 // `need` words in the record arena of super-chunk slot `slot` (warp-uniform call); -1 when the arena is full
 __device__ __forceinline__ int slot_alloc(const WarpCtx& c, int slot, int need) {
     int off = 0;
-    if (c.lane == 0) off = (int)atomicAdd(&c.sh->slotHead[slot], (unsigned int)((need + 1) & ~1));
+    if (c.lane == 0) off = (int)atomicAdd(&growSh.slotHead[slot], (unsigned int)((need + 1) & ~1));
     off = __shfl_sync(FULL, off, 0);
     return off + need <= c.arenaCap ? off : -1;
 }
@@ -1114,7 +1183,7 @@ __device__ __forceinline__ bool seed_taken(unsigned int st, int chunk) {
 // the map's abort flag as ONE value for the whole warp (a per-lane read of the volatile flag could split the warp)
 __device__ __forceinline__ int aborted(const WarpCtx& c) {
     int v = 0;
-    if (c.lane == 0) v = c.sh->abortFlag;
+    if (c.lane == 0) v = growSh.abortFlag;
     return __shfl_sync(FULL, v, 0);
 }
 
@@ -1123,8 +1192,9 @@ __device__ __forceinline__ int slot_of_chunk(const GrowShared& sh, int chunk) { 
 
 // One large seed (cell ci, pixel p), speculatively, with the whole warp: grow, rectangle, refine, NFA; the result is
 // parked in the record arena of the seed's super-chunk.  Any warp of the team may run this for any queued seed.
+template <bool BS>
 __device__ void eval_large(WarpCtx& c, int p, int ci, const ChunkRecs& R) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     const int chunkJ = ci >> 5;
     {   // one read for the whole warp: the word changes under our feet (other warps park regions)
         int taken = 0;
@@ -1135,7 +1205,7 @@ __device__ void eval_large(WarpCtx& c, int p, int ci, const ChunkRecs& R) {
     const int L1 = sh.nSeg;
     __threadfence_block();
     c.specChunk = chunkJ;
-    const int oc = eval_seed(c, p, c.scratch, 2 * c.listCap + 64, true, bb, used, chk, pndOff, pndN);
+    const int oc = eval_seed<BS>(c, p, c.scratch, 2 * c.listCap + 64, true, bb, used, chk, pndOff, pndN);
     c.specChunk = -1;
     STAT(c, ST_SPEC, 1);
     if (oc == OC_DEFER) return;
@@ -1160,8 +1230,9 @@ __device__ void eval_large(WarpCtx& c, int p, int ci, const ChunkRecs& R) {
 }
 
 // take one queued large seed, if any, and evaluate it; false = queue empty
+template <bool BS>
 __device__ bool help_large(WarpCtx& c, const ChunkRecs& R) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     unsigned int p = 0, ci = 0;
     int got = 0;
     if (c.lane == 0) {
@@ -1177,7 +1248,7 @@ __device__ bool help_large(WarpCtx& c, const ChunkRecs& R) {
     got = __shfl_sync(FULL, got, 0);
     if (!got) return false;
     p = __shfl_sync(FULL, p, 0); ci = __shfl_sync(FULL, ci, 0);
-    eval_large(c, (int)p, (int)ci, R);
+    eval_large<BS>(c, (int)p, (int)ci, R);
     __threadfence();   // record visible before the super-chunk can be flagged ready
     if (c.lane == 0) atomicSub((int*)&sh.slotPending[slot_of_chunk(sh, (int)ci >> 5)], 1);
     __syncwarp();
@@ -1192,12 +1263,13 @@ __device__ bool help_large(WarpCtx& c, const ChunkRecs& R) {
 //   C  the large seeds of the group go to the team's queue, where ANY warp picks them up (this warp helps until its
 //      own are done), so that a stretch of the seed list that is rich in large regions does not serialise on one warp.
 //      Each result is parked — its pixels marked pending — before the group that follows is scouted.
+template <bool BS>
 __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned int* cl, int nCells, const ChunkRecs& R, int T) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     const int lane = c.lane;
     const unsigned int lt = (1u << lane) - 1u;
     long long tSpec = clock64();
-    const int slot = slot_of_chunk(*c.sh, chunk0);
+    const int slot = slot_of_chunk(growSh, chunk0);
     unsigned int* q = c.q;   // [2k] pixel index, [2k+1] (sub << 5 | lane)
     int qn = 0;
     for (int s = 0; s < nSub; s++) {   // ---- A
@@ -1232,7 +1304,7 @@ __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned
         // small_grow decides the angle on the squares, which is the literal test only for a tolerance <= pi/2 (grow_region's
         // predicate); above that every live seed takes the warp path, like every seed when T > SG_CAP
         if (T <= SG_CAP && c.kc->degThre <= c.kc->pi / 2.0) {   // warp-uniform: all 32 lanes enter, the ones without a seed idle
-            num = small_grow(c, act, myp, T, lst, myChunk, pnd, npnd);
+            num = small_grow<BS>(c, act, myp, T, lst, myChunk, pnd, npnd);
             large = act && num >= T;
         }
         __syncwarp();
@@ -1297,7 +1369,7 @@ __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned
                     int pend = 0;
                     if (lane == 0) pend = sh.slotPending[slot] != 0 && !sh.abortFlag;
                     if (!__shfl_sync(FULL, pend, 0)) break;
-                    if (!help_large(c, R)) __nanosleep(100);
+                    if (!help_large<BS>(c, R)) __nanosleep(100);
                 }
             } else {   // queue full: evaluate them here
                 unsigned int todo = largeMask;
@@ -1306,7 +1378,7 @@ __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned
                     todo &= todo - 1;
                     const int p = __shfl_sync(FULL, myp, j);
                     const unsigned int relJ = __shfl_sync(FULL, rel, j);
-                    eval_large(c, p, (chunk0 + (int)(relJ >> 5)) * LSDB_CHUNK + (int)(relJ & 31u), R);
+                    eval_large<BS>(c, p, (chunk0 + (int)(relJ >> 5)) * LSDB_CHUNK + (int)(relJ & 31u), R);
                 }
             }
         }
@@ -1325,20 +1397,22 @@ __device__ void speculate_super(WarpCtx& c, int chunk0, int nSub, const unsigned
 // Lane-level validation of a parked "no change" result whose pixel lists are short (the lane-per-seed evaluations):
 // every pixel it accepted must still be un-banned (looked at only when a region was accepted nearby since), and every
 // pixel it skipped because of a parked accept must be banned by now.
-__device__ __forceinline__ bool lane_valid(const WarpCtx& c, const unsigned int* earena, bool hit, int nchk, unsigned int chkOff,
+template <bool BS>
+__device__ __forceinline__ bool lane_valid(const BanPlane<BS>& bp, const unsigned int* earena, bool hit, int nchk, unsigned int chkOff,
                                            int npnd, unsigned int pndOff) {
     bool ok = true;
     if (hit) {
         const unsigned int* px = earena + chkOff;
-        for (int j = 0; j < nchk; j++) ok = ok && !ban_at(c, px_of(px[j]), py_of(px[j]));
+        for (int j = 0; j < nchk; j++) ok = ok && !bp.at(px_of(px[j]), py_of(px[j]));
     }
     const unsigned int* pp = earena + pndOff;
-    for (int j = 0; j < npnd; j++) ok = ok && ban_at(c, px_of(pp[j]), py_of(pp[j]));
+    for (int j = 0; j < npnd; j++) ok = ok && bp.at(px_of(pp[j]), py_of(pp[j]));
     return ok;
 }
 
+template <bool BS>
 __device__ void retire_chunk(WarpCtx& c, int chunk, const unsigned int* cl, int nCells, const ChunkRecs& R, int* lab, LsdbRect* rc, int maxSeg) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     const int lane = c.lane;
     const int slot = chunk & (RING - 1);
     const int ci = chunk * LSDB_CHUNK + lane;
@@ -1349,13 +1423,14 @@ __device__ void retire_chunk(WarpCtx& c, int chunk, const unsigned int* cl, int 
     const int recPnd = recOc != OC_NONE ? R.pnd[ri] : 0;
     const unsigned int recPndOff = R.pndOff[ri];
     bool committedParked = false;   // this lane's parked accept / reject was committed as parked
-    const unsigned int* earena = c.arenas + (size_t)slot_of_chunk(*c.sh, chunk) * c.arenaCap;
+    const unsigned int* earena = c.arenas + (size_t)slot_of_chunk(growSh, chunk) * c.arenaCap;
+    const BanPlane<BS> bp = ban_plane<BS>(c);
     bool live = myp >= 0 && (lsdb_ld_state(&c.state[myp]) & 3u) == 0;   // :222
     // short "no change" records are validated by their own lane, in parallel; commits, long records, failed and
     // missing evaluations are walked serially, in seed order
     const bool laneCheck = recOc == OC_NOCHANGE && recChk >= 0 && recChk + recPnd <= 64;
     bool laneOK = false;
-    if (live && laneCheck) laneOK = lane_valid(c, earena, grid_hit(c, recB0, recB1, recL0), recChk, recChkOff, recPnd, recPndOff);
+    if (live && laneCheck) laneOK = lane_valid(bp, earena, grid_hit(c, recB0, recB1, recL0), recChk, recChkOff, recPnd, recPndOff);
     unsigned int liveAtTurn = __ballot_sync(FULL, live);
     unsigned int work = __ballot_sync(FULL, live && !(laneCheck && laneOK));
     BBox bb; int used = 0, chk = -1;
@@ -1369,25 +1444,25 @@ __device__ void retire_chunk(WarpCtx& c, int chunk, const unsigned int* cl, int 
         if (valid) {
             const int nchk = __shfl_sync(FULL, recChk, k);
             const bool hit = grid_hit(c, __shfl_sync(FULL, recB0, k), __shfl_sync(FULL, recB1, k), __shfl_sync(FULL, recL0, k));
-            if (hit) valid = nchk >= 0 && !any_banned(c, earena + __shfl_sync(FULL, recChkOff, k), nchk);
+            if (hit) valid = nchk >= 0 && !any_banned<BS>(c, earena + __shfl_sync(FULL, recChkOff, k), nchk);
         }
         if (valid) {   // every pixel the evaluation took for banned because of a parked accept must be banned by now
             const int npn = __shfl_sync(FULL, recPnd, k);
-            if (npn > 0) valid = !any_unbanned(c, earena + __shfl_sync(FULL, recPndOff, k), npn);
+            if (npn > 0) valid = !any_unbanned<BS>(c, earena + __shfl_sync(FULL, recPndOff, k), npn);
         }
         bool changed = false;
         if (valid) {
-            if (oc != OC_NOCHANGE) { commit_region(c, recp, lab, rc, maxSeg); changed = true; if (lane == k) committedParked = true; }
+            if (oc != OC_NOCHANGE) { commit_region<BS>(c, recp, lab, rc, maxSeg); changed = true; if (lane == k) committedParked = true; }
         } else {
             long long t0 = clock64();
             int po_, pn_;
-            const int oc2 = eval_seed(c, p, c.scratch, 2 * c.listCap + 64, false, bb, used, chk, po_, pn_);
+            const int oc2 = eval_seed<BS>(c, p, c.scratch, 2 * c.listCap + 64, false, bb, used, chk, po_, pn_);
             STAT(c, ST_RESPEC, 1);
             STAT(c, oc == OC_NONE ? RS_NONE : RS_CONFLICT, 1);
             if (oc == OC_ACCEPT || oc == OC_REJECT) STAT(c, RS_LOST, 1);
             if (oc2 == OC_REJECT || oc2 == OC_ACCEPT) STAT(c, RS_COMMIT, 1);
             if (oc2 == OC_DEFER) { sh.abortFlag = LSDB_ERR_CAPACITY; break; }
-            if (oc2 == OC_REJECT || oc2 == OC_ACCEPT) { commit_region(c, c.scratch, lab, rc, maxSeg); changed = true; }
+            if (oc2 == OC_REJECT || oc2 == OC_ACCEPT) { commit_region<BS>(c, c.scratch, lab, rc, maxSeg); changed = true; }
             if (lane == 0) atomicAdd(&sh.stats[TM_RESPEC], (unsigned long long)(clock64() - t0));
             if (aborted(c)) break;
         }
@@ -1396,7 +1471,7 @@ __device__ void retire_chunk(WarpCtx& c, int chunk, const unsigned int* cl, int 
             __threadfence_block();
             if (lane > k && live) {
                 live = (lsdb_ld_state(&c.state[myp]) & 3u) == 0;
-                if (live && laneCheck) laneOK = lane_valid(c, earena, grid_hit(c, recB0, recB1, recL0), recChk, recChkOff, recPnd, recPndOff);
+                if (live && laneCheck) laneOK = lane_valid(bp, earena, grid_hit(c, recB0, recB1, recL0), recChk, recChkOff, recPnd, recPndOff);
             }
             const unsigned int later = ~((2u << k) - 1u);
             liveAtTurn = (liveAtTurn & ~later) | (__ballot_sync(FULL, live) & later);
@@ -1420,8 +1495,9 @@ __device__ void retire_chunk(WarpCtx& c, int chunk, const unsigned int* cl, int 
 // result has ALREADY been invalidated (a pixel it accepted is banned now — that can only stay so), take its marks back
 // and evaluate the seed again, speculatively, against today's state.  Otherwise the retire walk would have to do that
 // evaluation itself, serially, when it gets there.  The chunk is locked (flag 2) meanwhile; the retire walk waits for 1.
+template <bool BS>
 __device__ bool revalidate_ahead(WarpCtx& c, const unsigned int* cl, int nCells, int nChunks, const ChunkRecs& R) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     const int lane = c.lane;
     int target = -1;
     {   // 32 chunks after the frontier chunk, one per lane; the nearest candidate wins
@@ -1448,7 +1524,7 @@ __device__ bool revalidate_ahead(WarpCtx& c, const unsigned int* cl, int nCells,
     const int recOc = R.oc[ri], recChk = R.chk[ri], recL0 = R.L0[ri];
     const unsigned int recB0 = R.b0[ri], recB1 = R.b1[ri], recOff = R.off[ri], recChkOff = R.chkOff[ri];
     const int recPnd = recOc != OC_NONE ? R.pnd[ri] : 0;
-    const unsigned int* earena = c.arenas + (size_t)slot_of_chunk(*c.sh, target) * c.arenaCap;
+    const unsigned int* earena = c.arenas + (size_t)slot_of_chunk(growSh, target) * c.arenaCap;
     const bool heavy = myp >= 0 && (recOc == OC_ACCEPT || recOc == OC_REJECT || (recOc == OC_NOCHANGE && !(recChk >= 0 && recChk + recPnd <= 64)));
     unsigned int todo = __ballot_sync(FULL, heavy && (lsdb_ld_state(&c.state[myp]) & 3u) == 0 && grid_hit(c, recB0, recB1, recL0));
     bool did = false;
@@ -1456,7 +1532,7 @@ __device__ bool revalidate_ahead(WarpCtx& c, const unsigned int* cl, int nCells,
         const int k = __ffs(todo) - 1;
         todo &= todo - 1;
         const int nchk = __shfl_sync(FULL, recChk, k);
-        const bool stale = nchk < 0 || any_banned(c, earena + __shfl_sync(FULL, recChkOff, k), nchk);
+        const bool stale = nchk < 0 || any_banned<BS>(c, earena + __shfl_sync(FULL, recChkOff, k), nchk);
         if (!stale) continue;
         const int oc = __shfl_sync(FULL, recOc, k);
         if (oc == OC_ACCEPT || oc == OC_REJECT) {
@@ -1465,7 +1541,7 @@ __device__ bool revalidate_ahead(WarpCtx& c, const unsigned int* cl, int nCells,
         }
         if (lane == 0) R.oc[(size_t)slot * 32 + k] = OC_NONE;
         __syncwarp();
-        eval_large(c, __shfl_sync(FULL, myp, k), target * LSDB_CHUNK + k, R);
+        eval_large<BS>(c, __shfl_sync(FULL, myp, k), target * LSDB_CHUNK + k, R);
         did = true;
     }
     __threadfence();
@@ -1475,8 +1551,9 @@ __device__ bool revalidate_ahead(WarpCtx& c, const unsigned int* cl, int nCells,
 }
 
 // drain the READY prefix at the frontier if nobody else is doing it
+template <bool BS>
 __device__ void try_retire(WarpCtx& c, const unsigned int* cl, int nCells, int nChunks, const ChunkRecs& R, int* lab, LsdbRect* rc, int maxSeg) {
-    GrowShared& sh = *c.sh;
+    GrowShared& sh = growSh;
     int go = 0;
     if (c.lane == 0) {
         const int f = sh.frontier;
@@ -1493,7 +1570,7 @@ __device__ void try_retire(WarpCtx& c, const unsigned int* cl, int nCells, int n
         f = __shfl_sync(FULL, f, 0);
         if (!__shfl_sync(FULL, ready, 0)) break;
         __threadfence();
-        retire_chunk(c, f, cl, nCells, R, lab, rc, maxSeg);
+        retire_chunk<BS>(c, f, cl, nCells, R, lab, rc, maxSeg);
         __threadfence_block();
         if (c.lane == 0) {
             const int slot = f & (RING - 1);
@@ -1512,22 +1589,22 @@ __device__ void try_retire(WarpCtx& c, const unsigned int* cl, int nCells, int n
     __syncwarp();
 }
 
-template <int MAXT>
+// BS: the ban plane of every map of the batch fits bmCapWords words of shared memory (see BanPlane)
+template <int MAXT, bool BS>
 __global__ void __launch_bounds__(MAXT, 1) lsdb_grow_kernel(int nImgs, const LsdbImg* __restrict__ imgs, LsdbImgDyn* __restrict__ dyn,
                                                                    const LsdbLsdConst* __restrict__ kc, const double* __restrict__ mag,
                                                                    const double* __restrict__ deg, const double* __restrict__ cosm,
-                                                                   const double* __restrict__ sinm, unsigned int* __restrict__ state,
+                                                                   unsigned int* __restrict__ state,
                                                                    const unsigned int* __restrict__ cells, int* __restrict__ labels,
                                                                    LsdbRect* __restrict__ rects, int maxSeg, unsigned int* __restrict__ lists,
                                                                    int listCap, int arenaCap, int runAhead, unsigned char* __restrict__ recBuf,
                                                                    const double* __restrict__ lgammaTab, int lgammaN, int* __restrict__ imgCounter,
                                                                    unsigned int* banBits, int bmCapWords, int steal) {
-    __shared__ GrowShared sh;
-    extern __shared__ unsigned int bmShared[];   // the map's ban plane, one bit per pixel (bmCapWords words)
+    GrowShared& sh = growSh;
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, nw = blockDim.x >> 5;
     WarpCtx c;
     c.lane = lane; c.w = w; c.mybit = 1u << (LSDB_ST_WARP_SHIFT + w);   // bits 4..19
-    c.kc = kc; c.lgammaTab = lgammaTab; c.lgammaN = lgammaN; c.sh = &sh;
+    c.kc = kc; c.lgammaTab = lgammaTab; c.lgammaN = lgammaN;
     c.listCap = listCap; c.arenaCap = arenaCap;
     c.rejCap = LSDB_REJ_CAP;
     c.arenas = lists + (size_t)blockIdx.x * grow_words_per_cta(listCap, arenaCap, nw);
@@ -1586,17 +1663,12 @@ __global__ void __launch_bounds__(MAXT, 1) lsdb_grow_kernel(int nImgs, const Lsd
             while (((max(im.W, im.H) - 1) >> k) > GRID - 1) k++;
             c.cellShift = k;
         }
-        c.state = state + im.nOff; c.deg = deg + im.nOff; c.mag = mag + im.nOff; c.cosm = cosm + 2 * im.nOff; c.sinm = sinm + 2 * im.nOff;   // one interleaved (cos, sin) plane
+        c.state = state + im.nOff; c.deg = deg + im.nOff; c.mag = mag + im.nOff; c.cs = reinterpret_cast<const double2*>(cosm) + im.nOff;
         c.pw = im.pw;
-        {   // the ban plane written by the stencil stage moves into shared memory when it fits
+        c.bm = banBits + im.banOff;
+        if (BS) {   // the ban plane written by the stencil stage moves into shared memory (the host checked that it fits)
             const int words = im.H * im.pw;
-            if (words <= bmCapWords) {
-                const unsigned int* srcB = banBits + im.banOff;
-                for (int i = tid; i < words; i += blockDim.x) bmShared[i] = srcB[i];
-                c.bm = bmShared; c.bmInSmem = true;
-            } else {
-                c.bm = banBits + im.banOff; c.bmInSmem = false;
-            }
+            for (int i = tid; i < words; i += blockDim.x) bmShared[i] = c.bm[i];
         }
         const int T = (int)ceil(im.regThre);   // regions below regThre pixels are dropped (:228)
         __syncthreads();
@@ -1607,7 +1679,7 @@ __global__ void __launch_bounds__(MAXT, 1) lsdb_grow_kernel(int nImgs, const Lsd
         unsigned int idle = 0;
 
         while (!aborted(c)) {
-            try_retire(c, cl, nCells, nChunks, R, lab, rc, maxSeg);
+            try_retire<BS>(c, cl, nCells, nChunks, R, lab, rc, maxSeg);
             if (__shfl_sync(FULL, (int)sh.frontier, 0) >= nChunks) break;
             int chunk = -1;
             if (lane == 0) {
@@ -1620,8 +1692,8 @@ __global__ void __launch_bounds__(MAXT, 1) lsdb_grow_kernel(int nImgs, const Lsd
             }
             chunk = __shfl_sync(FULL, chunk, 0);
             if (chunk < 0) {   // nothing to claim: help with queued large seeds, else wait for the frontier to move
-                if (help_large(c, R)) { idle = 0; continue; }
-                if (revalidate_ahead(c, cl, nCells, nChunks, R)) { idle = 0; continue; }
+                if (help_large<BS>(c, R)) { idle = 0; continue; }
+                if (revalidate_ahead<BS>(c, cl, nCells, nChunks, R)) { idle = 0; continue; }
                 long long tw = clock64();
                 __nanosleep(200);
                 if (lane == 0) {
@@ -1632,7 +1704,7 @@ __global__ void __launch_bounds__(MAXT, 1) lsdb_grow_kernel(int nImgs, const Lsd
                 continue;
             }
             idle = 0;
-            speculate_super(c, chunk, min(1 << sh.supShift, nChunks - chunk), cl, nCells, R, T);
+            speculate_super<BS>(c, chunk, min(1 << sh.supShift, nChunks - chunk), cl, nCells, R, T);
         }
         __syncthreads();
         if (tid == 0) {
@@ -1662,26 +1734,40 @@ static bool lsdb_grow_wide_regs(int nCtas, int warpsPerCta) {
     return warpsPerCta <= 8 && nCtas <= 148;
 }
 
+template <int MAXT, bool BS>
+static void grow_launch(cudaStream_t s, int nImgs, int nCtas, int warpsPerCta, const LsdbImg* imgs, LsdbImgDyn* dyn,
+                        const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm,
+                        unsigned int* state, const unsigned int* cells, int* labels, LsdbRect* rects, int maxSeg,
+                        unsigned int* lists, int listCap, int arenaCap, int runAhead, unsigned char* recBuf, const double* lgammaTab, int lgammaN,
+                        int* imgCounter, unsigned int* banBits, int bmCapWords, int steal) {
+    // per device and cheap: set on every launch (a process may drive several GPUs through several contexts)
+    cudaFuncSetAttribute(lsdb_grow_kernel<MAXT, BS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)grow_dyn_smem(bmCapWords, NW_MAX));
+    if (nImgs <= 0) return;
+    lsdb_grow_kernel<MAXT, BS><<<nCtas, warpsPerCta * 32, grow_dyn_smem(bmCapWords, warpsPerCta), s>>>(
+        nImgs, imgs, dyn, kc, mag, deg, cosm, state, cells, labels, rects, maxSeg, lists, listCap, arenaCap, runAhead, recBuf,
+        lgammaTab, lgammaN, imgCounter, banBits, bmCapWords, steal);
+}
+
+// bmCapWords > 0: the ban plane of every map of the batch fits that many words (lsdb_batch_create), and the build that keeps it
+// in shared memory runs; 0: the build that reads the global plane
 void lsdb_launch_grow(cudaStream_t s, int nImgs, int nCtas, int warpsPerCta, const LsdbImg* imgs, LsdbImgDyn* dyn,
-                      const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm, const double* sinm,
+                      const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm,
                       unsigned int* state, const unsigned int* cells, int* labels, LsdbRect* rects, int maxSeg,
                       unsigned int* lists, int listCap, int arenaCap, int runAhead, unsigned char* recBuf, const double* lgammaTab, int lgammaN,
                       int* imgCounter, unsigned int* banBits, int bmCapWords, int steal) {
     if (runAhead <= 0 || runAhead > RING - (NW_MAX + 1) * LSDB_SUPER) runAhead = RING - (NW_MAX + 1) * LSDB_SUPER;
     if (runAhead < 1) runAhead = 1;
-    // per device and cheap: set on every launch (a process may drive several GPUs through several contexts)
     const bool wide = lsdb_grow_wide_regs(nCtas, warpsPerCta);
-    if (wide) cudaFuncSetAttribute(lsdb_grow_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)grow_dyn_smem(bmCapWords, NW_MAX));
-    else cudaFuncSetAttribute(lsdb_grow_kernel<NW_MAX * 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)grow_dyn_smem(bmCapWords, NW_MAX));
-    if (nImgs <= 0) return;
-    if (wide)
-        lsdb_grow_kernel<256><<<nCtas, warpsPerCta * 32, grow_dyn_smem(bmCapWords, warpsPerCta), s>>>(
-            nImgs, imgs, dyn, kc, mag, deg, cosm, sinm, state, cells, labels, rects, maxSeg, lists, listCap, arenaCap, runAhead, recBuf,
-            lgammaTab, lgammaN, imgCounter, banBits, bmCapWords, steal);
-    else
-        lsdb_grow_kernel<NW_MAX * 32><<<nCtas, warpsPerCta * 32, grow_dyn_smem(bmCapWords, warpsPerCta), s>>>(
-            nImgs, imgs, dyn, kc, mag, deg, cosm, sinm, state, cells, labels, rects, maxSeg, lists, listCap, arenaCap, runAhead, recBuf,
-            lgammaTab, lgammaN, imgCounter, banBits, bmCapWords, steal);
+#define LSDB_GROW_ARGS s, nImgs, nCtas, warpsPerCta, imgs, dyn, kc, mag, deg, cosm, state, cells, labels, rects, maxSeg, lists, listCap, arenaCap, \
+                       runAhead, recBuf, lgammaTab, lgammaN, imgCounter, banBits, bmCapWords, steal
+    if (bmCapWords > 0) {
+        if (wide) grow_launch<256, true>(LSDB_GROW_ARGS);
+        else grow_launch<NW_MAX * 32, true>(LSDB_GROW_ARGS);
+    } else {
+        if (wide) grow_launch<256, false>(LSDB_GROW_ARGS);
+        else grow_launch<NW_MAX * 32, false>(LSDB_GROW_ARGS);
+    }
+#undef LSDB_GROW_ARGS
 }
 
 size_t lsdb_grow_words_per_cta(int listCap, int arenaCap, int warpsPerCta) { return grow_words_per_cta(listCap, arenaCap, warpsPerCta); }
@@ -1700,18 +1786,23 @@ void lsdb_launch_used_plane(cudaStream_t s, const unsigned int* state, uint8_t* 
 int lsdb_grow_max_ctas(int device, int warpsPerCta, int bmCapWords) {
     int sms = 0, per = 0;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    cudaFuncSetAttribute(lsdb_grow_kernel<NW_MAX * 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)grow_dyn_smem(bmCapWords, NW_MAX));
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, lsdb_grow_kernel<NW_MAX * 32>, warpsPerCta * 32, grow_dyn_smem(bmCapWords, warpsPerCta));
+    // the build that will run (see lsdb_launch_grow)
+    if (bmCapWords > 0) {
+        cudaFuncSetAttribute(lsdb_grow_kernel<NW_MAX * 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)grow_dyn_smem(bmCapWords, NW_MAX));
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, lsdb_grow_kernel<NW_MAX * 32, true>, warpsPerCta * 32, grow_dyn_smem(bmCapWords, warpsPerCta));
+    } else {
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, lsdb_grow_kernel<NW_MAX * 32, false>, warpsPerCta * 32, grow_dyn_smem(0, warpsPerCta));
+    }
     if (per < 1) per = 1;
     return sms * per;
 }
 
-// largest ban plane (in 32-bit words) that fits in shared memory next to the kernel's static data
+// largest ban plane (in 32-bit words) that fits in shared memory next to the kernel's static data (both builds have the same)
 int lsdb_grow_max_bitmap_words(int device) {
     int optin = 0;
     cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
     cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, lsdb_grow_kernel<NW_MAX * 32>) != cudaSuccess) return 0;
+    if (cudaFuncGetAttributes(&fa, lsdb_grow_kernel<NW_MAX * 32, true>) != cudaSuccess) return 0;   // the build that holds the plane
     const long long room = (long long)optin - (long long)fa.sharedSizeBytes - 256 - NW_MAX * 1024;
     return room > 0 ? (int)(room / 4) : 0;
 }

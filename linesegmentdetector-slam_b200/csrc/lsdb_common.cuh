@@ -67,11 +67,17 @@ struct LsdbLsdConst {
 };
 
 #ifdef __CUDACC__
-__device__ __forceinline__ unsigned int lsdb_ld_state(const unsigned int* p) {
-    unsigned int v;
-    asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
+// A state word from L2 (other CTAs and warps update the words with atomics, so L1 would serve stale copies).  The load
+// is not a compiler memory barrier: the compiler may keep other loads in flight across it.  That fits every reader in
+// grow.cu, which falls in one of two classes:
+//   (a) speculative gathers whose staleness the retire-time validation tolerates (V1 / V2, DESIGN.md §4.3): the grower's
+//       and the scouts' candidate loads, the seed_taken checks of speculate_super / eval_large, park_pixels' first guess
+//       before its compare-and-swap loop;
+//   (b) reads that follow a __threadfence / __threadfence_block or the retire lock, which order them already: the live
+//       tests of retire_chunk and revalidate_ahead, unpark_pixels (its own marks were fenced when their chunk was flagged).
+// No reader polls a state word for a change (that would need a re-read the compiler cannot fold or move: a "memory"
+// clobber, as this helper had before).
+__device__ __forceinline__ unsigned int lsdb_ld_state(const unsigned int* p) { return __ldcg(p); }
 // x86-64 cvttsd2si semantics for (int)double: NaN / out of range -> INT_MIN (SURVEY.md A.9)
 __device__ __forceinline__ int lsdb_x86_d2i(double v) {
     if (!(v > -2147483649.0 && v < 2147483648.0)) return (int)0x80000000;
@@ -102,8 +108,9 @@ size_t lsdb_order_tab_words_per_band(void);
 // rows of cols bytes (a packed caller buffer); the plane must be zeroed first
 void lsdb_launch_line_images(cudaStream_t s, int nImgs, int maxSeg, const LsdbImg* imgs, const LsdbImgDyn* dyn, const LsdbRect* rects,
                              uint8_t* plane, const unsigned long long* packOff);
+// the region stage (grow.cu); cosm is the interleaved (cos, sin) plane the stencil stage writes (its sinm == cosm + 1)
 void lsdb_launch_grow(cudaStream_t s, int nImgs, int nCtas, int warpsPerCta, const LsdbImg* imgs, LsdbImgDyn* dyn,
-                      const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm, const double* sinm,
+                      const LsdbLsdConst* kc, const double* mag, const double* deg, const double* cosm,
                       unsigned int* state, const unsigned int* cells, int* labels, LsdbRect* rects, int maxSeg,
                       unsigned int* lists, int listCap, int arenaCap, int runAhead, unsigned char* recBuf, const double* lgammaTab, int lgammaN,
                       int* imgCounter, unsigned int* banBits, int bmCapWords, int steal);
