@@ -71,7 +71,7 @@ struct lsdb_batch {
     lsdb_ctx* ctx = nullptr;
     int n = 0;
     lsdb_lsd_params params = {};
-    int maxSeg = 0, listCap = 0, arenaCap = 0, nTiles = 0, nCtas = 0, nWarps = 0, runAhead = 0, bmCapWords = 0, steal = 0, stencilMode = 0;
+    int maxSeg = 0, listCap = 0, arenaCap = 0, nTiles = 0, nCtas = 0, nWarps = 0, runAhead = 0, bmCapWords = 0, steal = 0, deferCap = 0;
     size_t totalN = 0, totalSrc = 0, totalBan = 0;
     std::vector<LsdbImg> imgs;
     LsdbLsdConst kc = {};
@@ -79,7 +79,7 @@ struct lsdb_batch {
     uint8_t* src = nullptr; double* mag = nullptr; double* deg = nullptr; double* cosm = nullptr; double* sinm = nullptr;
     unsigned int* state = nullptr; unsigned short* bins = nullptr; unsigned int* cells = nullptr;
     int* labels = nullptr; LsdbRect* rects = nullptr; LsdbImgDyn* dyn = nullptr; LsdbImg* imgsD = nullptr; int* tileImg = nullptr;
-    unsigned int* lists = nullptr; int* imgCounter = nullptr; LsdbLsdConst* kcD = nullptr; double* gaussDbg = nullptr;
+    unsigned int* lists = nullptr; int* imgCounter = nullptr; LsdbLsdConst* kcD = nullptr;
     unsigned char* recBuf = nullptr; unsigned int* banBits = nullptr;
     uint8_t* lineImD = nullptr;   // lineIm planes of all maps (allocated on first use by lsdb_batch_line_images; geometry of src)
     double* mcCache = nullptr;    // mapCache planes of all maps, rows*cols f64 each, packed in batch order (allocated on first use by lsdb_batch_map_caches)
@@ -189,7 +189,7 @@ extern "C" void lsdb_batch_destroy(lsdb_batch* b) {
     cudaSetDevice(b->ctx->device);
     cudaFree(b->src); cudaFree(b->mag); cudaFree(b->deg); cudaFree(b->cosm); cudaFree(b->state); cudaFree(b->bins); cudaFree(b->cells);
     cudaFree(b->labels); cudaFree(b->rects); cudaFree(b->dyn); cudaFree(b->imgsD); cudaFree(b->tileImg); cudaFree(b->lists);
-    cudaFree(b->imgCounter); cudaFree(b->kcD); cudaFree(b->gaussDbg); cudaFree(b->recBuf); cudaFree(b->banBits);
+    cudaFree(b->imgCounter); cudaFree(b->kcD); cudaFree(b->recBuf); cudaFree(b->banBits);
     cudaFree(b->lineImD); cudaFree(b->mcCache); cudaFree(b->packOffD); cudaFree(b->nzBits); cudaFree(b->bandOf); cudaFree(b->bandsOfImg); cudaFree(b->orderTabs);
     cudaFreeHost(b->dynH); cudaFreeHost(b->rectsH);
     for (int i = 0; i < 4; i++) cudaEventDestroy(b->ev[i]);
@@ -307,7 +307,9 @@ extern "C" int lsdb_batch_create(lsdb_ctx* ctx, int n, const int* cols, const in
         if (nw == 1 && !getenv("LSDB_SMEM_BAN_KB")) b->bmCapWords = 0;
         b->runAhead = 0;   // chunks a map's team may speculate ahead of its commit frontier (0 = as far as the ring allows)
         if (getenv("LSDB_RUNAHEAD")) b->runAhead = atoi(getenv("LSDB_RUNAHEAD"));
-        b->stencilMode = lsdb_stencil_mode();
+        // records of the stencil stage's deferred list (0: what its scratch plane holds); a small cap sends tiles down the
+        // in-kernel path for a reservation that does not fit
+        if (getenv("LSDB_STENCIL_DEFER")) { int v = atoi(getenv("LSDB_STENCIL_DEFER")); if (v >= 2 && v <= (1 << 20)) b->deferCap = v; }
         b->steal = 0;   // measured: spreading large seeds over the team duplicates growth of neighbouring seeds; no net gain
         if (getenv("LSDB_STEAL")) b->steal = atoi(getenv("LSDB_STEAL")) & 0xff;
         if (getenv("LSDB_SUPER_SHIFT")) b->steal |= ((atoi(getenv("LSDB_SUPER_SHIFT")) & 3) + 1) << 8;   // chunks per claim = 1 << n (default: per map)
@@ -388,8 +390,8 @@ static int run_stencil(lsdb_batch* b, int nTiles, int tileBase) {
     CK(ctx, cudaMemsetAsync(b->labels, 0, b->totalN * 4, s));
     CK(ctx, cudaMemsetAsync(b->imgCounter, 0, 64, s));
     CK(ctx, cudaEventRecord(b->ev[0], s));
-    const int nStencil = lsdb_launch_stencil(s, nTiles, b->imgsD, b->tileImg, b->dyn, b->kcD, b->src, b->mag, b->deg, b->cosm, b->sinm, b->state, b->banBits, b->nzBits, b->gaussDbg, tileBase,
-                        b->cells, b->totalN * 4, b->imgCounter + 8, b->stencilMode);   // the seed-list plane is free until the ordering stage: scratch for the deferred pixels
+    const int nStencil = lsdb_launch_stencil(s, nTiles, b->imgsD, b->tileImg, b->dyn, b->kcD, b->src, b->mag, b->deg, b->cosm, b->sinm, b->state, b->banBits, b->nzBits, tileBase,
+                        b->cells, b->totalN * 4, b->deferCap, b->imgCounter + 8);   // the seed-list plane is free until the ordering stage: scratch for the deferred pixels
     CK(ctx, cudaEventRecord(b->ev[1], s));
     CK(ctx, cudaGetLastError());
     b->ran = false; b->downloaded = false; b->launches = nStencil;

@@ -85,21 +85,14 @@ __device__ __forceinline__ int lsdb_x86_d2i(double v) {
 }
 #endif
 
-// launchers (defined in the .cu files, called from api.cu); the stencil launchers return the number of kernels they launched.
-// mode (lsdb_stencil_mode(): LSDB_STENCIL / LSDB_STENCIL_G / LSDB_STENCIL_DEFER read when the batch is created): bits 0-1 the cut
-// (1: stencil.cu, 2: stencil2.cu), bits 2-4 tiles per CTA of stencil2.cu (1, 2, 4), bit 5 deferred pixels into a second kernel, bits 8.. a cap
-// on the records of the deferred list (0: what the scratch plane holds).
-int lsdb_stencil_mode(void);
+// launchers (defined in the .cu files, called from api.cu)
+// The stencil stage (stencil2.cu) on tiles [tileBase, tileBase + nTiles): the tile kernel and the kernel of the deferred pixels
+// (those whose angle needs the double-double phase); returns the number of kernels launched.  deferBuf (deferBytes) is scratch
+// for the deferred list, deferCap caps it in records (0: what deferBuf holds), deferCount is a zeroed counter in device memory.
 int lsdb_launch_stencil(cudaStream_t s, int nTiles, const LsdbImg* imgs, const int* tileImg, LsdbImgDyn* dyn,
-                         const LsdbLsdConst* kc, const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm,
-                         unsigned int* state, unsigned int* banBits, unsigned int* nzBits, double* gaussOut, int tileBase,
-                         void* deferBuf, size_t deferBytes, int* deferCount, int mode);
-// the second cut of the stage (stencil2.cu): what lsdb_launch_stencil runs unless the mode asks for the first.  deferBuf is
-// scratch for the launch (pixels whose angle needs the double-double phase), deferCount a zeroed counter in device memory.
-int lsdb_launch_stencil_v2(cudaStream_t s, int nTiles, const LsdbImg* imgs, const int* tileImg, LsdbImgDyn* dyn,
-                            const LsdbLsdConst* kc, const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm,
-                            unsigned int* state, unsigned int* banBits, unsigned int* nzBits, double* gaussOut, int tileBase,
-                            void* deferBuf, size_t deferBytes, int* deferCount, int groups);
+                        const LsdbLsdConst* kc, const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm,
+                        unsigned int* state, unsigned int* banBits, unsigned int* nzBits, int tileBase,
+                        void* deferBuf, size_t deferBytes, int deferCap, int* deferCount);
 void lsdb_launch_order(cudaStream_t s, int nImgs, int nBands, const LsdbImg* imgs, LsdbImgDyn* dyn, const LsdbLsdConst* kc,
                        const double* mag, const unsigned int* nzBits, const int2* bandOf, const int2* bandsOfImg, unsigned int* tabs,
                        unsigned short* bins, unsigned int* cells);

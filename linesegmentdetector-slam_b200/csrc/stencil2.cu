@@ -1,11 +1,11 @@
-// Stage A of the LSD hot path on sm_100a, second cut: the same fused remap + decimating Gaussian + gradient / level-line
-// angle / threshold mask as stencil.cu (which stays in the library as the fallback, LSDB_STENCIL=1), same results bit for bit,
-// fewer instructions.  Replaces (reference, /root/reference/LSD/myLSD.cpp) the remap loop :135-142, GaussianSampler :378-484
-// and the gradient loop :151-174 incl. maxGrad.
+// Stage A of the LSD hot path on sm_100a: the fused remap + decimating Gaussian + gradient / level-line angle / threshold
+// mask.  Replaces (reference, /root/reference/LSD/myLSD.cpp) the remap loop :135-142, GaussianSampler :378-484 and the
+// gradient loop :151-174 incl. maxGrad.
 //
-// What stencil.cu's ncu profile showed (profiles/r2_ncu_full_summary.txt: issue-bound, 17 of 32 threads active on
-// average, a third of the angle instructions in the double-double slow path taken by ~0.2 % of the calls) and what
-// this version does about it:
+// What the ncu profile of the stage's first cut showed (one pass per output with its tap loop inline, full atan2 / cos / sin
+// per pixel; retired, DESIGN.md §4.1; profiles/r2_ncu_full_summary.txt: issue-bound, 17 of 32 threads active on average,
+// a third of the angle instructions in the double-double slow path taken by ~0.2 % of the calls) and what this version
+// does about it:
 //   * X and Y pass in two phases.  Phase 1 walks (row, column) with a warp per row exactly like before but only
 //     DECIDES whether an output has a non-zero tap (one funnel shift on the bit vectors) and appends the ones that do
 //     to a work list (one shared-memory atomic per warp); phase 2 runs the tap loops over that list with full warps.
@@ -33,7 +33,7 @@
 #define SLOW_CAP 256            // deferred pixels a tile can hold
 
 struct LsdbDeferRec { unsigned long long p; double gx, gy; };   // pixel (index into the planes), gradX, gradY
-static_assert(sizeof(LsdbDeferRec) == 24, "stencil.cu caps the list in records of 24 bytes");
+static_assert(sizeof(LsdbDeferRec) == 24, "a deferred record is 24 bytes: the scratch plane (4 bytes a pixel) holds one per 6 pixels");
 
 struct __align__(16) Stencil2Smem {
     union {
@@ -161,7 +161,7 @@ __device__ __forceinline__ int st2_append(int* counter, bool has, int lane) {
     return has ? base + __popc(bal & ((1u << lane) - 1u)) : -1;
 }
 
-// the full (phase 1 + phase 2) angle triple of a pixel: what stencil.cu computes for every pixel
+// the full (phase 1 + phase 2) angle triple of a pixel, for the few whose phase-1 rounding test failed
 __device__ __noinline__ void st2_angle_full(double gradX, double gradY, double pi, bool growable, double* d_, double* c_, double* s_) {
     double d = lsdm_atan2(gradX, -gradY);
     if (fabs(d - pi) < 0.000001) d = 0.0;
@@ -169,26 +169,19 @@ __device__ __noinline__ void st2_angle_full(double gradX, double gradY, double p
     if (growable) { *c_ = lsdm_cos(d); *s_ = lsdm_sin(d); }
 }
 
-// G tiles per CTA, one group of NT threads each, all groups in step from barrier to barrier.  An experiment that stays
-// selectable (LSDB_STENCIL_G): ncu shows the GPC-level instruction cache at 85 % of its request peak with four independent
-// 8-warp CTAs per SM walking ~50 KB of code once per tile, and warps that run the same phase at the same time share what they
-// fetch — but they also wait on each other's barriers, and G = 2 / 4 measured 13 % / 33 % slower than G = 1.
-template <int G>
-__global__ void __launch_bounds__(NT * G, 4 / G) lsdb_stencil2_kernel(const LsdbImg* __restrict__ imgs, const int* __restrict__ tileImg,
+// One tile per CTA: 2 and 4 tiles per CTA were measured slower and removed (DESIGN.md §4.1).
+__global__ void __launch_bounds__(NT, 4) lsdb_stencil2_kernel(const LsdbImg* __restrict__ imgs, const int* __restrict__ tileImg,
                                                            LsdbImgDyn* __restrict__ dyn, const LsdbLsdConst* __restrict__ kc,
                                                            const uint8_t* __restrict__ src, double* __restrict__ mag,
                                                            double* __restrict__ deg, double* __restrict__ cosm,
                                                            double* __restrict__ sinm, unsigned int* __restrict__ state,
                                                            unsigned int* __restrict__ banBits, unsigned int* __restrict__ nzBits,
-                                                           double* __restrict__ gaussOut, int tileBase, int nTilesLaunch,
+                                                           double* __restrict__ gaussOut, int tileBase,
                                                            LsdbDeferRec* __restrict__ deferBuf, long long deferCap, int* __restrict__ deferCount) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int grp = G == 1 ? 0 : (int)threadIdx.x / NT;
-    Stencil2Smem& S = reinterpret_cast<Stencil2Smem*>(smem_raw)[grp];
-    const int tid = (int)threadIdx.x - grp * NT, lane = tid & 31, warp = tid >> 5;
-    int launchTile = (int)blockIdx.x * G + grp;
-    if (launchTile >= nTilesLaunch) launchTile = nTilesLaunch - 1;   // a group past the end repeats the last tile: the same values written twice
-    const int tileIdx = launchTile + tileBase;   // a launch may cover a range of tiles only (one map tiled over several GPUs)
+    Stencil2Smem& S = *reinterpret_cast<Stencil2Smem*>(smem_raw);
+    const int tid = (int)threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tileIdx = (int)blockIdx.x + tileBase;   // a launch may cover a range of tiles only (one map tiled over several GPUs)
     const int imgIdx = tileImg[tileIdx];
     const LsdbImg im = imgs[imgIdx];
     const int lt = tileIdx - im.tile0;
@@ -271,8 +264,7 @@ __global__ void __launch_bounds__(NT * G, 4 / G) lsdb_stencil2_kernel(const Lsdb
     }
     __syncthreads();
 
-    {   // (no shortcut for a tile whose window is all zero: its lists stay empty and the Y pass writes the zeros — every barrier
-        // below is reached by every thread of the CTA whatever its group's tile holds)
+    {   // (no shortcut for a tile whose window is all zero: its lists stay empty and the Y pass writes the zeros)
         // ---- X pass.  The rows that hold a non-zero pixel are listed first.
         for (int r = tid; r < nRows; r += NT) {
             const unsigned int* rb = &S.rowBits[r * ROW_WORDS];
@@ -539,34 +531,21 @@ __global__ void __launch_bounds__(128) lsdb_stencil_deferred_kernel(const LsdbDe
     }
 }
 
-template <int G>
-static void st2_launch(cudaStream_t s, int nTiles, const LsdbImg* imgs, const int* tileImg, LsdbImgDyn* dyn, const LsdbLsdConst* kc,
-                       const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm, unsigned int* state, unsigned int* banBits,
-                       unsigned int* nzBits, double* gaussOut, int tileBase, LsdbDeferRec* recs, long long cap, int* deferCount) {
-    const int smem = (int)sizeof(Stencil2Smem) * G;
-    cudaFuncSetAttribute(lsdb_stencil2_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);   // per device, cheap
-    lsdb_stencil2_kernel<G><<<(nTiles + G - 1) / G, NT * G, smem, s>>>(imgs, tileImg, dyn, kc, src, mag, deg, cosm, sinm, state, banBits, nzBits, gaussOut,
-                                                                       tileBase, nTiles, recs, cap, deferCount);
-}
-
-int lsdb_launch_stencil_v2(cudaStream_t s, int nTiles, const LsdbImg* imgs, const int* tileImg, LsdbImgDyn* dyn,
-                           const LsdbLsdConst* kc, const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm,
-                           unsigned int* state, unsigned int* banBits, unsigned int* nzBits, double* gaussOut, int tileBase,
-                           void* deferBuf, size_t deferBytes, int* deferCount, int groups) {
+int lsdb_launch_stencil(cudaStream_t s, int nTiles, const LsdbImg* imgs, const int* tileImg, LsdbImgDyn* dyn,
+                        const LsdbLsdConst* kc, const uint8_t* src, double* mag, double* deg, double* cosm, double* sinm,
+                        unsigned int* state, unsigned int* banBits, unsigned int* nzBits, int tileBase,
+                        void* deferBuf, size_t deferBytes, int deferCap, int* deferCount) {
     if (nTiles <= 0) return 0;
-    // groups = tiles per CTA (LSDB_STENCIL_G = 1, 2 or 4).  Measured on 64 maps of 4096^2: 3.66 / 4.14 / 4.87 ms — groups in step
-    // share their instruction fetches but wait on each other's barriers, and the waiting costs more: one tile per CTA is the default.
-    const long long cap = deferBuf && deferCount ? (long long)(deferBytes / sizeof(LsdbDeferRec)) : 0;
-    LsdbDeferRec* recs = cap > 0 ? (LsdbDeferRec*)deferBuf : nullptr;
-    if (groups == 1) st2_launch<1>(s, nTiles, imgs, tileImg, dyn, kc, src, mag, deg, cosm, sinm, state, banBits, nzBits, gaussOut, tileBase, recs, cap, deferCount);
-    else if (groups == 4) st2_launch<4>(s, nTiles, imgs, tileImg, dyn, kc, src, mag, deg, cosm, sinm, state, banBits, nzBits, gaussOut, tileBase, recs, cap, deferCount);
-    else st2_launch<2>(s, nTiles, imgs, tileImg, dyn, kc, src, mag, deg, cosm, sinm, state, banBits, nzBits, gaussOut, tileBase, recs, cap, deferCount);
-    if (recs) {
-        // expected: ~1 record per tile; the grid is sized for that and strides over whatever the count turns out to be
-        long long want = ((long long)nTiles + 127) / 128;
-        const int grid = (int)(want < 1 ? 1 : (want > 1184 ? 1184 : want));
-        lsdb_stencil_deferred_kernel<<<grid, 128, 0, s>>>(recs, cap, deferCount, kc, deg, cosm, sinm, state);
-        return 2;
-    }
-    return 1;
+    long long cap = (long long)(deferBytes / sizeof(LsdbDeferRec));
+    if (deferCap > 0 && deferCap < cap) cap = deferCap;
+    LsdbDeferRec* recs = (LsdbDeferRec*)deferBuf;
+    cudaFuncSetAttribute(lsdb_stencil2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Stencil2Smem));   // per device, cheap
+    // gaussOut (a debug copy of the Gaussian plane) is null, but stays a parameter: without its stores the kernel is 5 % more SASS
+    lsdb_stencil2_kernel<<<nTiles, NT, sizeof(Stencil2Smem), s>>>(imgs, tileImg, dyn, kc, src, mag, deg, cosm, sinm, state, banBits, nzBits,
+                                                                  nullptr, tileBase, recs, cap, deferCount);
+    // expected: ~1 record per tile; the grid is sized for that and strides over whatever the count turns out to be
+    long long want = ((long long)nTiles + 127) / 128;
+    const int grid = (int)(want < 1 ? 1 : (want > 1184 ? 1184 : want));
+    lsdb_stencil_deferred_kernel<<<grid, 128, 0, s>>>(recs, cap, deferCount, kc, deg, cosm, sinm, state);
+    return 2;
 }

@@ -35,7 +35,7 @@ def _compare_with_oracle(lsdb, b, i, m, got, check_planes=True, **params):
 @contextlib.contextmanager
 def lsdb_env(env):
     """`env` set in os.environ for the block, the previous values back afterwards.  The library reads its switches when a
-    batch is created (team size, ban plane, stencil cut) and when it runs (LSDB_GROW_WIDE picks the grower's build at
+    batch is created (team size, ban plane, the stencil stage's deferred-list cap) and when it runs (LSDB_GROW_WIDE picks the grower's build at
     launch), so the block covers both."""
     old = {k: os.environ.get(k) for k in env}
     os.environ.update(env)
@@ -262,22 +262,20 @@ def test_result_is_independent_of_team_shape(lsdb, ctx, gold, env):
     b.close()
 
 
-@pytest.mark.parametrize("env", [dict(LSDB_STENCIL="1"), dict(LSDB_STENCIL_DEFER="0"), dict(LSDB_STENCIL_G="2"), dict(LSDB_STENCIL_G="4", LSDB_STENCIL_DEFER="0"),
-                                 dict(LSDB_STENCIL_DEFER="5")])
-def test_result_is_independent_of_the_stencil_cut(lsdb, ctx, gold, env):
-    """The stencil stage's first cut (stencil.cu, LSDB_STENCIL=1) stays in the library as the fallback of the second
-    (stencil2.cu: work lists, phase-1-only angle math, failed rounding tests deferred to a second kernel); the second
-    also runs with the deferred pixels kept in their tiles, with a deferred list of five records (most tiles' reservations
-    then do not fit: the part inside the list becomes no-ops, the tile evaluates its own) and with 2 / 4 tiles per CTA.  Same planes, seed lists and
-    segments as the oracle from every one of them — borders with reflected taps, a ragged 33rd column and row 0 / column 0
-    walls included."""
+@pytest.mark.parametrize("cap", [0, 2, 5, 64, 512], ids=lambda c: f"{c}_records" if c else "whole_plane")
+def test_stencil_planes_with_the_deferred_list_full_and_not(lsdb, ctx, gold, cap):
+    """The stencil stage queues the pixels whose phase-1 rounding test fails in a deferred list that a second kernel
+    evaluates.  At its default size (the scratch plane) the tiles' reservations fit; capped at 2, 5, 64 and 512 records the
+    list fills after fewer or more tiles, and a tile whose reservation does not fit evaluates its own (the part inside the
+    list becomes no-ops).  Same planes, seed lists and segments as the oracle either way — borders with reflected taps, a
+    ragged 33rd column and row 0 / column 0 walls included."""
     maps = [gold["mapValue/map"], synth.occupancy_grid(1057, 771, seed=91), synth.occupancy_grid(400, 1300, seed=92, border_walls=True),
             synth.occupancy_grid(97, 45, seed=12), synth.occupancy_grid(2048, 2048, seed=93)]
-    with lsdb_env(env):
+    with lsdb_env(dict(LSDB_STENCIL_DEFER=str(cap)) if cap else {}):
         b = lsdb.Batch(ctx, [(m.shape[1], m.shape[0]) for m in maps])
         b.upload(maps); b.run()
     got = b.download(want_rects=True)
-    assert b.launches() == (5 if env.get("LSDB_STENCIL") == "1" or env.get("LSDB_STENCIL_DEFER") == "0" else 6)
+    assert b.launches() == 6
     for i, m in enumerate(maps):
         _compare_with_oracle(lsdb, b, i, m, got, check_planes=True)
     b.close()

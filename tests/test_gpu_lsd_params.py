@@ -118,10 +118,11 @@ def test_wide_tolerance_result_is_independent_of_team_shape(lsdb, ctx, angThre, 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("angThre", [1.0, 170.0])
-@pytest.mark.parametrize("env", [dict(LSDB_STENCIL="1"), dict()], ids=["first_cut", "default"])
-def test_extreme_gradient_threshold_through_both_stencil_cuts(lsdb, ctx, gold_maps_for_stencil, angThre, env):
+@pytest.mark.parametrize("env", [dict(), dict(LSDB_STENCIL_DEFER="5")], ids=["whole_plane", "5_records"])
+def test_extreme_gradient_threshold_through_the_stencil_stage(lsdb, ctx, gold_maps_for_stencil, angThre, env):
     """gradThre = 2/sin(angThre): 114.6 at 1 degree (nearly every pixel goes to the banned queue) and 11.5 at 170 degrees;
-    the planes, seed lists and segments of both stencil cuts against the oracle"""
+    the planes, seed lists and segments of the stencil stage against the oracle, with the deferred list at its default size
+    and capped at five records (the tiles that do not fit it evaluate their own, banned pixels included)"""
     with lsdb_env(env):
         _run_and_compare(lsdb, ctx, gold_maps_for_stencil, dict(angThre=angThre))
 

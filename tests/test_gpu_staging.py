@@ -177,8 +177,7 @@ def _stages_ok(b):
 def test_batch_entry_points_keep_launches_and_stage_events(lsdb, inputs, shared):
     from lsdb200 import giant
     ctx, _maps = shared
-    env = os.environ
-    n_stencil = 1 if env.get("LSDB_STENCIL") == "1" or env.get("LSDB_STENCIL_DEFER") == "0" else 2
+    n_stencil = 2
     maps = [inputs["map"], synth.occupancy_grid(700, 500, seed=5)]
     b = lsdb.Batch(ctx, [(m.shape[1], m.shape[0]) for m in maps])
     b.upload(maps)

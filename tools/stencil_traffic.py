@@ -7,7 +7,7 @@ raw = subprocess.run(["ncu", "-i", rep, "--page", "raw", "--csv"], capture_outpu
 rows = list(csv.reader(io.StringIO(raw))); hdr, units = rows[0], rows[1]
 for r in rows[2:]:
     d = dict(zip(hdr, r))
-    if "lsdb_stencil2_kernel" not in d.get("Kernel Name", "") and "lsdb_stencil_kernel" not in d.get("Kernel Name", ""):
+    if "lsdb_stencil2_kernel" not in d.get("Kernel Name", ""):
         continue
     def val(k):
         v = float(d[k].replace(",", "")); u = units[hdr.index(k)].lower()
